@@ -102,12 +102,12 @@ k_fast32x2_tiled(SrcView S, Tgt T, int nrows, int chunk_len, double *pu, double 
 
 // Whole row sums in one launch: warp-private bulk-copy pipelines, chunk partials folded through (distributed) shared
 // memory, Euler update and peer stores in the epilogue (biot_savart.cuh, "fast fused").
-template <int R, int UNROLL, int WARPS, int CL, int V, class Tgt>
-__global__ void __launch_bounds__(32 * WARPS, 16 / WARPS)
+template <int R, int CL, int V, class Tgt>
+__global__ void __launch_bounds__(32 * FW_WARPS, 2)
 k_fast_fused(SrcView S, Tgt T, int nrows, int chunk_len, int nchunks, FusedOut O)
 {
     extern __shared__ __align__(128) unsigned char fw_raw[];
-    fast_fused_block<R, UNROLL, WARPS, CL, V>(S, T, nrows, chunk_len, nchunks, O, *reinterpret_cast<FwSmem<WARPS> *>(fw_raw));
+    fast_fused_block<R, CL, V>(S, T, nrows, chunk_len, nchunks, O, *reinterpret_cast<FwSmem *>(fw_raw));
 }
 
 // Fold partials.  exact: nfold = tree depth d; fast: nfold = number of chunks.  Optional second partial set
@@ -248,20 +248,20 @@ static int prove_exact_ranges(ludvm_ctx *ctx, const SrcView &S, const Tgt &T, lo
     return LUDVM_OK;
 }
 
-template <int R, int UNROLL, int WARPS, int CL, int V, class Tgt>
+template <int R, int CL, int V, class Tgt>
 static int launch_fused_inst(ludvm_ctx *ctx, const SrcView &S, const Tgt &T, int nrows, int chunk_len, int nchunks,
                              const FusedOut &O)
 {
-    auto kern = k_fast_fused<R, UNROLL, WARPS, CL, V, Tgt>;
+    auto kern = k_fast_fused<R, CL, V, Tgt>;
     static bool configured[16] = {};                       // per device; a function attribute is per device
     if (!configured[ctx->device & 15]) {
-        CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FwSmem<WARPS>)));
+        CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FwSmem)));
         configured[ctx->device & 15] = true;
     }
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)ceil_div(nrows, 32 * R), CL, 1);
-    cfg.blockDim = dim3(32 * WARPS, 1, 1);
-    cfg.dynamicSmemBytes = sizeof(FwSmem<WARPS>);
+    cfg.blockDim = dim3(32 * FW_WARPS, 1, 1);
+    cfg.dynamicSmemBytes = sizeof(FwSmem);
     cfg.stream = ctx->stream;
     cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeClusterDimension;
@@ -272,8 +272,8 @@ static int launch_fused_inst(ludvm_ctx *ctx, const SrcView &S, const Tgt &T, int
     cfg.numAttrs = CL > 1 ? 1 : 0;
     CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, S, T, nrows, chunk_len, nchunks, O));
     ctx->launches++;
-    set_plan(ctx, LUDVM_K_FAST_FUSED, R, nchunks, 1, CL, UNROLL);
-    ctx->plan[6] = WARPS;
+    set_plan(ctx, LUDVM_K_FAST_FUSED, R, nchunks, 1, CL, fw_unroll(R));
+    ctx->plan[6] = FW_WARPS;
     ctx->plan[7] = V;
     return LUDVM_OK;
 }
@@ -286,8 +286,7 @@ static int try_launch_fused(ludvm_ctx *ctx, int mode, const SrcView &S, const Tg
                             bool *launched)
 {
     *launched = false;
-    if ((mode != LUDVM_FAST_F64 && mode != LUDVM_FAST12_F64) || getenv("LUDVM_NO_FUSED") || getenv("LUDVM_NO_TMA"))
-        return LUDVM_OK;
+    if ((mode != LUDVM_FAST_F64 && mode != LUDVM_FAST12_F64) || getenv("LUDVM_NO_FUSED")) return LUDVM_OK;
     if (S.vc4 != nullptr || S.gstride != 1 || S.n0 != S.n ||
         (((uintptr_t)S.x | (uintptr_t)S.z | (uintptr_t)S.g) & 15) != 0)
         return LUDVM_OK;
@@ -295,32 +294,23 @@ static int try_launch_fused(ludvm_ctx *ctx, int mode, const SrcView &S, const Tg
     long chunks;
     fast_chunking(S.n, &chunk_len, &chunks);
     if (chunks != 8 && chunks != 16) return LUDVM_OK;
-    // 16 chunks: one 16-warp CTA per SM (LUDVM_FUSED_WARPS=16) or a cluster of two 8-warp CTAs (default)
-    const char *we = getenv("LUDVM_FUSED_WARPS");
-    const int W = (chunks == 16 && we && atoi(we) == 16) ? 16 : 8;
-    const int CL = (int)chunks / W;
+    // 16 chunks: a cluster of two 8-warp CTAs
+    const int CL = (int)chunks / FW_WARPS;
     const long want = (long)ctx->sm_count * 2 * 6;
     int R = 4;
     while (R >= 1 && (long)ceil_div(nrows, 32 * R) * (chunks / 8) < want) R >>= 1;
     if (R < 1) return LUDVM_OK;
-    const char *ue = getenv("LUDVM_FUSED_UNROLL");
-    const int U = ue ? atoi(ue) : 4;
     int rc;
-#define FUSED_CASE(RR, UU, VV)                                                                                      \
-    rc = W == 16 ? launch_fused_inst<RR, UU, 16, 1, VV>(ctx, S, T, (int)nrows, chunk_len, (int)chunks, O)           \
-       : CL == 2 ? launch_fused_inst<RR, UU, 8, 2, VV>(ctx, S, T, (int)nrows, chunk_len, (int)chunks, O)            \
-                 : launch_fused_inst<RR, UU, 8, 1, VV>(ctx, S, T, (int)nrows, chunk_len, (int)chunks, O)
+#define FUSED_CASE(RR, VV)                                                                                          \
+    rc = CL == 2 ? launch_fused_inst<RR, 2, VV>(ctx, S, T, (int)nrows, chunk_len, (int)chunks, O)                   \
+                 : launch_fused_inst<RR, 1, VV>(ctx, S, T, (int)nrows, chunk_len, (int)chunks, O)
     if (mode == LUDVM_FAST12_F64) {   // opt-in 12-slot pair arithmetic
-        if (R == 4 && U == 4) FUSED_CASE(4, 4, 1);
-        else if (R == 4) FUSED_CASE(4, 8, 1);
-        else if (R == 2) FUSED_CASE(2, 4, 1);
-        else FUSED_CASE(1, 8, 1);
-    } else if (R == 4 && U == 1) FUSED_CASE(4, 1, 0);
-    else if (R == 4 && U == 2) FUSED_CASE(4, 2, 0);
-    else if (R == 4 && U == 8) FUSED_CASE(4, 8, 0);
-    else if (R == 4) FUSED_CASE(4, 4, 0);
-    else if (R == 2) FUSED_CASE(2, 4, 0);
-    else FUSED_CASE(1, 8, 0);
+        if (R == 4) FUSED_CASE(4, 1);
+        else if (R == 2) FUSED_CASE(2, 1);
+        else FUSED_CASE(1, 1);
+    } else if (R == 4) FUSED_CASE(4, 0);
+    else if (R == 2) FUSED_CASE(2, 0);
+    else FUSED_CASE(1, 0);
 #undef FUSED_CASE
     if (rc) return rc;
     CUDA_TRY(cudaGetLastError());
@@ -386,8 +376,7 @@ static int launch_partials(ludvm_ctx *ctx, int mode, const SrcView &S, const Tgt
         long chunks;
         fast_chunking(S.n, &chunk_len, &chunks);
         // fp32: the packed fp32x2 kernel (8 rows per thread) when the core radius is a scalar and there are enough rows
-        const bool f32x2 = f32 && S.vc4 == nullptr && (long)ceil_div(nrows, FT_THREADS * 8) * chunks >= (long)sm * 2 &&
-                           !getenv("LUDVM_NO_F32X2");
+        const bool f32x2 = f32 && S.vc4 == nullptr && (long)ceil_div(nrows, FT_THREADS * 8) * chunks >= (long)sm * 2;
         int R = f32x2 ? 8 : 4;
         if (!f32) {
             while (R > 1 && (long)ceil_div(nrows, FT_THREADS * R) * chunks < (long)sm * 2 * 6) R >>= 1;
@@ -401,7 +390,7 @@ static int launch_partials(ludvm_ctx *ctx, int mode, const SrcView &S, const Tgt
         dim3 grid(row_blocks, (unsigned)chunks);
         // one contiguous, 16-byte aligned source segment with a scalar core: TMA-staged tiles
         const bool tma = !f32 && S.vc4 == nullptr && S.gstride == 1 && S.n0 == S.n &&
-                         (((uintptr_t)S.x | (uintptr_t)S.z | (uintptr_t)S.g) & 15) == 0 && !getenv("LUDVM_NO_TMA");
+                         (((uintptr_t)S.x | (uintptr_t)S.z | (uintptr_t)S.g) & 15) == 0;
         if (f32x2) k_fast32x2_tiled<<<grid, FT_THREADS, 0, ctx->stream>>>(S, T, (int)nrows, chunk_len, (double *)a, (double *)b);
         else if (f32) k_fast32_tiled<4><<<grid, FT_THREADS, 0, ctx->stream>>>(S, T, (int)nrows, chunk_len, (double *)a, (double *)b);
         else if (tma && R == 4) k_fast_tiled_tma<4><<<grid, FT_THREADS, 0, ctx->stream>>>(S, T, (int)nrows, chunk_len, (double *)a, (double *)b);

@@ -557,79 +557,6 @@ __device__ __forceinline__ void fast_tiled_block(const SrcView &S, const Tgt &T,
     }
 }
 
-// Double-buffered form of fast_tiled_block for sources that bulk copies cannot take (the time loop's three-segment wake):
-// every thread fetches its two sources of tile k + 1 into registers BEFORE the pair loop of tile k and stores them to the
-// other buffer afterwards, so the loads are in flight during the FP64 work and one __syncthreads per tile is left
-// (fast_tiled_block: load -> barrier -> compute -> barrier, 16 % of the issue slots waiting at the barrier,
-// profiles/r01c_k_conv_old_tiled_stalls.txt).  Sources are packed (x, z) + Gamma: one LDS.128 + one LDS.64 per source
-// instead of four LDS.64.  Scalar core radius only.
-struct DbTiles {
-    double2 xz[2][FT_TILE];
-    double g[2][FT_TILE];
-};
-template <int R, class Tgt>
-__device__ __forceinline__ void fast_tiled_block_db(const SrcView &S, const Tgt &T, int nrows, int row_block, int c0, int c1,
-                                                    double *__restrict__ pu, double *__restrict__ pw_, DbTiles &sm)
-{
-    constexpr int UNROLL = R <= 2 ? 8 : FT_UNROLL;
-    constexpr int PER = FT_TILE / FT_THREADS;
-    double tx[R], tz[R], au[R], aw[R];
-    const int base = row_block * (FT_THREADS * R) + threadIdx.x;
-#pragma unroll
-    for (int r = 0; r < R; r++) {
-        T.get(min(base + r * FT_THREADS, nrows - 1), tx[r], tz[r]);
-        au[r] = 0.0;
-        aw[r] = 0.0;
-    }
-    const double vc4 = S.vc4s;
-    double lx[PER], lz[PER], lg[PER];
-    auto fetch = [&](int t0) {
-#pragma unroll
-        for (int q = 0; q < PER; q++) {
-            const int s = t0 + threadIdx.x + q * FT_THREADS;
-            const bool ok = s < c1;
-            const int p = ok ? S.phys(s) : 0;
-            lx[q] = ok ? S.x[p] : 0.0;
-            lz[q] = ok ? S.z[p] : 0.0;
-            lg[q] = ok ? S.g[p * S.gstride] * LUDVM_INV_TWO_PI : 0.0;
-        }
-    };
-    auto put = [&](int buf) {
-#pragma unroll
-        for (int q = 0; q < PER; q++) {
-            sm.xz[buf][threadIdx.x + q * FT_THREADS] = make_double2(lx[q], lz[q]);
-            sm.g[buf][threadIdx.x + q * FT_THREADS] = lg[q];
-        }
-    };
-    const int ntiles = (c1 - c0 + FT_TILE - 1) / FT_TILE;
-    if (ntiles > 0) fetch(c0);
-    __syncthreads();
-    put(0);
-    __syncthreads();
-    for (int k = 0; k < ntiles; k++) {
-        const int buf = k & 1, t0 = c0 + k * FT_TILE;
-        if (k + 1 < ntiles) fetch(t0 + FT_TILE);
-        const int cnt = min(FT_TILE, c1 - t0);
-#pragma unroll UNROLL
-        for (int j = 0; j < cnt; j++) {
-            const double2 s = sm.xz[buf][j];
-            const double g = sm.g[buf][j];
-#pragma unroll
-            for (int r = 0; r < R; r++) pair_fast(tx[r], tz[r], s.x, s.y, g, vc4, au[r], aw[r]);
-        }
-        if (k + 1 < ntiles) put(buf ^ 1);
-        __syncthreads();
-    }
-#pragma unroll
-    for (int r = 0; r < R; r++) {
-        const int row = base + r * FT_THREADS;
-        if (row < nrows) {
-            pu[row] = au[r];
-            pw_[row] = aw[r];
-        }
-    }
-}
-
 // ---------------------------------------------------------------------------------------------------
 // fast tiled, TMA-staged: for one contiguous source segment with a scalar core the x / z / Gamma tiles are brought
 // into shared memory by the copy engine (cp.async.bulk + mbarrier complete_tx, SASS UBLKCP), double-buffered so the
@@ -743,11 +670,11 @@ __device__ __forceinline__ void fast_tiled_block_tma(const SrcView &S, const Tgt
 
 // ---------------------------------------------------------------------------------------------------
 // fast fused ("warp-split"): the whole row sum inside one thread-block cluster -- no partial sums in global memory
-// and no combine kernel.  A CTA owns 32*R target rows; each of its WARPS warps holds ALL of those rows (R per lane) and
+// and no combine kernel.  A CTA owns 32*R target rows; each of its FW_WARPS warps holds ALL of those rows (R per lane) and
 // walks ONE source chunk with its own private, double-buffered bulk-copy pipeline (cp.async.bulk + mbarrier, SASS
 // UBLKCP/SYNCS), so the main loop has no block-wide barrier at all.  A cluster of CL CTAs (1 or 2: clusters of two
-// pack the 148 SMs perfectly) covers WARPS*CL source chunks: 8 chunks = one 8-warp CTA, 16 chunks = one 16-warp CTA
-// or a cluster of two 8-warp CTAs.  The chunk partials meet in shared memory and are folded IN
+// pack the 148 SMs perfectly) covers FW_WARPS*CL source chunks: 8 chunks = one 8-warp CTA, 16 chunks = a cluster of two
+// 8-warp CTAs.  The chunk partials meet in shared memory and are folded IN
 // CHUNK ORDER through distributed shared memory -- the same canonical order as fast_combine_row, so the result is
 // bitwise equal to the partial-sum path and independent of grid size and GPU count.  The epilogue applies the forward
 // Euler update (LUDVM.py:1108-1127) and the peer stores of the fused all-gather.
@@ -756,14 +683,17 @@ __device__ __forceinline__ void fast_tiled_block_tma(const SrcView &S, const Tgt
 #define FW_SUB 128       // sources per warp-private stage: three 1 KB bulk copies
 #endif
 #define FW_STAGES 2
+#define FW_WARPS 8       // warps per CTA, one source chunk each
+
+// source-loop unroll of the fused kernel: few rows per lane need a deeper unroll for independent chains
+__host__ __device__ constexpr int fw_unroll(int R) { return R == 1 ? 8 : 4; }
 
 struct FwWarpStage {
     double x[FW_SUB], z[FW_SUB], g[FW_SUB];
 };
-template <int WARPS>
 struct FwSmem {
-    FwWarpStage st[WARPS][FW_STAGES];   // 6 KB per warp; the front of each warp's region is reused for its partials
-    uint64_t full[WARPS][FW_STAGES];
+    FwWarpStage st[FW_WARPS][FW_STAGES];   // 6 KB per warp; the front of each warp's region is reused for its partials
+    uint64_t full[FW_WARPS][FW_STAGES];
 };
 
 struct FusedOut {
@@ -788,11 +718,11 @@ __device__ __forceinline__ const double *cluster_map(const double *p, unsigned r
     return (const double *)out;
 }
 
-template <int R, int UNROLL, int WARPS, int CL, int V, class Tgt>
+template <int R, int CL, int V, class Tgt>
 __device__ __forceinline__ void fast_fused_block(const SrcView &S, const Tgt &T, int nrows, int chunk_len, int nchunks,
-                                                 const FusedOut &O, FwSmem<WARPS> &sm)
+                                                 const FusedOut &O, FwSmem &sm)
 {
-    constexpr int FW_WARPS = WARPS;
+    constexpr int UNROLL = fw_unroll(R);
     constexpr int ROWS = 32 * R;
     // the warp index through a shuffle: ptxas then knows it is warp-uniform and keeps the stage addresses and the loop
     // counter on the uniform datapath (ULEA / UIADD3 + LDS [UR + imm]) instead of vector integer instructions

@@ -50,11 +50,8 @@ namespace ludvm {
 #define SIM_TILED_CHUNKS_MAX 64   // partial-sum slots per row of the tiled convection
 #define SIM_EXACT_TILED_MIN_WAKE 8192   // exact mode, graph path: wakes at least this large use k_conv_partials_exact_tiled
 #define SIM_COOP_MAX_WAKE 8192    // wakes up to this size are stepped by the persistent cooperative kernel
-#define SIM_CLUSTER_CTAS 16       // the single-cluster persistent kernel: CTAs (16 = the non-portable maximum) x threads
-#define SIM_CLUSTER_THREADS 256   // 512 threads halve the O(N^2) phases' rounds but cap the kernel at 128 registers and slow the
-                                  // solve by ~3 us: README case 30.4 / 25.7 us per step (exact / fast) against 28.7 / 24.0 with 256
-                                  // (profiles/r02s_coop_probe_1.txt; LUDVM_CLUSTER_THREADS=512 selects the other instantiation)
-#define SIM_CLUSTER_MAX_WAKE 512  // wakes up to this size are stepped by the single-cluster kernel (LUDVM_CLUSTER_MAX_WAKE).  README
+#define SIM_CLUSTER_CTAS 16       // the single-cluster persistent kernel: CTAs (16 = the non-portable maximum) x 256 threads
+#define SIM_CLUSTER_MAX_WAKE 512  // wakes up to this size are stepped by the single-cluster kernel.  README
                                   // case, us per step over the 400 steps, exact / fast: cluster up to 128: 32.2 / 26.1, 256: 31.1 / 25.3,
                                   // 384: 30.2 / 24.8, 512: 29.6 / 24.4, all 604: 31.0 / 25.0; cooperative grid alone 33.4 / 26.9
                                   // (profiles/r02l_coop_probe.txt): past ~500 vortices the O(N^2) phases want more than 16 SMs
@@ -1006,36 +1003,14 @@ __global__ void __launch_bounds__(FT_THREADS, 2) k_conv_partials_tiled(SimDev S,
 // the last wave's worth of time).  Identical in the producer and in k_finish_ov.
 struct TiledGeom {
     int chunk_len, chunks;
-    // `slots_code` = resident CTA slots, plus (opt-in, A/B runs) a wave range in bits 10-15 / 16-21 for the search below.
-    __host__ __device__ __forceinline__ TiledGeom(int nrows, int nsrc, int R, int slots_code)
+    // `slots` = resident CTA slots of the convection kernel.
+    __host__ __device__ __forceinline__ TiledGeom(int nrows, int nsrc, int R, int slots)
     {
         const int rb = (nrows + FT_THREADS * R - 1) / (FT_THREADS * R);
-        const int slots = slots_code & 1023, wmin = (slots_code >> 10) & 63, wmax = (slots_code >> 16) & 63;
-        if (wmin == 0) {
-            int want = (8 * slots + rb - 1) / rb;
-            want = want < 1 ? 1 : (want > SIM_TILED_CHUNKS_MAX ? SIM_TILED_CHUNKS_MAX : want);
-            chunk_len = (((nsrc + want - 1) / want + 63) / 64) * 64;
-            chunks = (nsrc + chunk_len - 1) / chunk_len;
-            return;
-        }
-        // Opt-in (LUDVM_TILED_WAVES=min,max): equal items run in waves over the resident slots, so the kernel should take
-        // waves x (chunk length + a fixed cost per item): try min .. max waves, for each the largest chunk count that
-        // still fits them (chunk lengths in multiples of 16), and keep the cheapest.  Measured on the dt = 2e-3 run
-        // (profiles/r02zd_hires.txt): 4..10 waves 5.86 s against 5.45 s for the rule above -- few, long CTAs free their
-        // first slot late for the solve branch.
-        long best = -1;
-        chunk_len = nsrc > 0 ? nsrc : 1;
-        chunks = 1;
-        for (int W = wmin; W <= wmax; W++) {
-            int c = (int)(((long)W * slots) / rb);
-            c = c < 1 ? 1 : (c > SIM_TILED_CHUNKS_MAX ? SIM_TILED_CHUNKS_MAX : c);
-            int len = (((nsrc + c - 1) / c + 15) / 16) * 16;
-            len = len < 16 ? 16 : len;
-            const int nch = (nsrc + len - 1) / len;
-            const long waves = ((long)rb * nch + slots - 1) / slots;
-            const long t = waves * (long)(len + 48);
-            if (best < 0 || t < best) { best = t; chunk_len = len; chunks = nch < 1 ? 1 : nch; }
-        }
+        int want = (8 * slots + rb - 1) / rb;
+        want = want < 1 ? 1 : (want > SIM_TILED_CHUNKS_MAX ? SIM_TILED_CHUNKS_MAX : want);
+        chunk_len = (((nsrc + want - 1) / want + 63) / 64) * 64;
+        chunks = (nsrc + chunk_len - 1) / chunk_len;
     }
 };
 
@@ -1047,10 +1022,10 @@ __global__ void __launch_bounds__(SOLVE_THREADS, 4) k_solve_small(SimDev S, int 
     phase_solve<LUDVM_METHOD_FAURE>(S, st, sm, sm + TABLE_SMEM_DOUBLES(S.P, S.Nc, S.sinn_smem), S.pre_sums, true);
 }
 
-template <int R, bool DB>
+template <int R>
 __global__ void __launch_bounds__(FT_THREADS, 2) k_conv_old_tiled(SimDev S, int s, int slots)
 {
-    __shared__ __align__(16) unsigned char raw[DB ? sizeof(DbTiles) : 4 * FT_TILE * sizeof(double)];
+    __shared__ __align__(16) double sx[4 * FT_TILE];
     Step st;
     if (!step_begin(S, s, st)) return;
     SrcView W = wake_view(S, st.itev, st.ilev);
@@ -1063,153 +1038,8 @@ __global__ void __launch_bounds__(FT_THREADS, 2) k_conv_old_tiled(SimDev S, int 
     place_lev(S, st.i, st.ilev, TW.xl, TW.zl);
     int c0 = blockIdx.y * G.chunk_len, c1 = min(W.n, c0 + G.chunk_len);
     size_t po = (size_t)blockIdx.y * nrows;
-    if (DB) {
-        fast_tiled_block_db<R>(W, TW, nrows, blockIdx.x, c0, c1, S.pb_u + po, S.pb_w + po, *reinterpret_cast<DbTiles *>(raw));
-    } else {
-        double *sx = reinterpret_cast<double *>(raw);
-        fast_tiled_block<R>(W, TW, nrows, blockIdx.x, c0, c1, S.pb_u + po, S.pb_w + po, sx, sx + FT_TILE, sx + 2 * FT_TILE,
-                            sx + 3 * FT_TILE);
-    }
-}
-
-// ---------------------------------------------------------------------------------------------------
-// Old-wake convection as independent WARP TASKS with warp-private bulk-copy pipelines (the shape of the fused all-pairs
-// kernel, biot_savart.cuh): task = (group of 32*R target rows, source chunk); the warp keeps its R rows per lane in
-// registers and streams the chunk's sources through its own double-buffered stages (cp.async.bulk + mbarrier), so the
-// kernel has no block-wide barrier at all -- the thread-staged tiles of k_conv_old_tiled spent 16 % of their issue
-// slots waiting at __syncthreads (profiles/r01c_k_conv_old_tiled_stalls.txt).
-// Bulk copies need 16-byte aligned, contiguous sources, and the wake is three physical segments whose ends move every
-// step.  The traversal is therefore defined on ALIGNED PHYSICAL BLOCKS of WT_SB sources: every block that overlaps a
-// segment is copied whole (the state arrays live in one arena, so a block may reach past a segment's end into
-// neighbouring storage; those entries are loaded and never used) and the source loop runs over the block's valid
-// sub-range.  Chunk = a contiguous run of blocks; partial sums [chunk][row] as before (fast mode: no order guarantee).
-// ---------------------------------------------------------------------------------------------------
-#define WT_SB 128   // sources per block / stage
-#ifndef WT_ROUNDS
-#define WT_ROUNDS 4 // rounds of warp tasks over the resident warps (more rounds: finer tail, earlier free slots for the
-                    // solve branch; fewer: less per-task pipeline fill)
-#endif
-struct BlockMap {
-    int a[3], b[3], nb[3], total;
-    __host__ __device__ __forceinline__ explicit BlockMap(const SrcView &W)
-    {
-        a[0] = 0; b[0] = W.n0;
-        a[1] = W.o1; b[1] = W.o1 + (W.n01 - W.n0);
-        a[2] = W.o2; b[2] = W.o2 + (W.n - W.n01);
-        total = 0;
-        for (int k = 0; k < 3; k++) {
-            nb[k] = b[k] > a[k] ? (b[k] - 1) / WT_SB - a[k] / WT_SB + 1 : 0;
-            total += nb[k];
-        }
-    }
-    // q-th block of the traversal -> physical block index and the valid entries [lo, hi) inside it
-    __device__ __forceinline__ void get(int q, int &pblk, int &lo, int &hi) const
-    {
-        int k = 0;
-        if (q >= nb[0]) { q -= nb[0]; k = 1; if (q >= nb[1]) { q -= nb[1]; k = 2; } }
-        pblk = a[k] / WT_SB + q;
-        lo = max(a[k] - pblk * WT_SB, 0);
-        hi = min(b[k] - pblk * WT_SB, WT_SB);
-    }
-};
-// Task geometry from the ACTUAL wake: about WT_ROUNDS rounds of warp tasks over the resident warps, whole blocks per chunk.
-// Identical in the producer and in k_finish_ov.
-struct WtGeom {
-    int nrg, chunks, bpc;
-    __host__ __device__ __forceinline__ WtGeom(int nrows, int nblocks, int R, int task_budget)
-    {
-        nrg = (nrows + 32 * R - 1) / (32 * R);
-        int want = task_budget / nrg;   // task_budget = rounds x resident warps
-        want = want < 1 ? 1 : (want > SIM_TILED_CHUNKS_MAX ? SIM_TILED_CHUNKS_MAX : want);
-        want = want > nblocks ? nblocks : want;
-        want = want < 1 ? 1 : want;
-        bpc = (nblocks + want - 1) / want;
-        bpc = bpc < 1 ? 1 : bpc;
-        chunks = (nblocks + bpc - 1) / bpc;
-        chunks = chunks < 1 ? 1 : chunks;
-    }
-};
-struct WtStage { double x[WT_SB], z[WT_SB], g[WT_SB]; };
-struct WtSmem {
-    WtStage st[8][2];
-    uint64_t full[8][2];
-};
-
-template <int R>
-__global__ void __launch_bounds__(256, 2) k_conv_old_wt(SimDev S, int s, int task_budget)
-{
-    extern __shared__ __align__(128) unsigned char wt_raw[];
-    WtSmem &sm = *reinterpret_cast<WtSmem *>(wt_raw);
-    Step st;
-    if (!step_begin(S, s, st)) return;
-    SrcView W = wake_view(S, st.itev, st.ilev);
-    const int nrows = W.n + 3;   // + the new TEV, the LEV if shed, the idle LEV slot (TgtWakePlus)
-    const BlockMap B(W);
-    const WtGeom G(nrows, B.total, R, task_budget);
-    const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;
-    const long task = (long)blockIdx.x * 8 + warp;
-    if (task >= (long)G.nrg * G.chunks) return;
-    const int c = (int)(task / G.nrg), rg = (int)(task - (long)c * G.nrg);
-    TgtWakePlus TW;
-    TW.W = W;
-    place_tev(S, st.i, st.itev, TW.xt, TW.zt);
-    place_lev(S, st.i, st.ilev, TW.xl, TW.zl);
-    double tx[R], tz[R], au[R], aw[R];
-    const int base = rg * 32 * R + lane;
-#pragma unroll
-    for (int r = 0; r < R; r++) {
-        TW.get(min(base + 32 * r, nrows - 1), tx[r], tz[r]);
-        au[r] = 0.0;
-        aw[r] = 0.0;
-    }
-    double vc4;
-    asm volatile("mov.f64 %0, %1;" : "=d"(vc4) : "d"(S.vc4));
-    const int q0 = c * G.bpc, q1 = min(B.total, q0 + G.bpc);
-    WtStage *stg = sm.st[warp];
-    uint64_t *full = sm.full[warp];
-    if (lane == 0) {
-        mbar_init(&full[0], 1);
-        mbar_init(&full[1], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-    auto issue = [&](int k) {   // lane 0: three 1 KB bulk copies of physical block pblk into stage k & 1
-        if (lane == 0) {
-            int pblk, lo, hi;
-            B.get(q0 + k, pblk, lo, hi);
-            WtStage &b = stg[k & 1];
-            const size_t off = (size_t)pblk * WT_SB;
-            mbar_expect_tx(&full[k & 1], 3 * WT_SB * sizeof(double));
-            bulk_g2s(b.x, S.wx + off, WT_SB * sizeof(double), &full[k & 1]);
-            bulk_g2s(b.z, S.wz + off, WT_SB * sizeof(double), &full[k & 1]);
-            bulk_g2s(b.g, S.wg + off, WT_SB * sizeof(double), &full[k & 1]);
-        }
-    };
-    const int nblk = q1 - q0;
-    if (nblk > 0) issue(0);
-    for (int k = 0; k < nblk; k++) {
-        __syncwarp();                               // every lane is done with stage (k + 1) & 1
-        if (k + 1 < nblk) issue(k + 1);
-        int pblk, lo, hi;
-        B.get(q0 + k, pblk, lo, hi);
-        mbar_wait(&full[k & 1], (k >> 1) & 1);
-        const WtStage &b = stg[k & 1];
-#pragma unroll 2
-        for (int j = lo; j < hi; j++) {
-            const double x = b.x[j], z = b.z[j], g = b.g[j];
-#pragma unroll
-            for (int r = 0; r < R; r++) pair_fast(tx[r], tz[r], x, z, g, vc4, au[r], aw[r]);
-        }
-    }
-    const size_t po = (size_t)c * nrows;
-#pragma unroll
-    for (int r = 0; r < R; r++) {
-        const int row = base + 32 * r;
-        if (row < nrows) {
-            S.pb_u[po + row] = au[r] * LUDVM_INV_TWO_PI;
-            S.pb_w[po + row] = aw[r] * LUDVM_INV_TWO_PI;
-        }
-    }
+    fast_tiled_block<R>(W, TW, nrows, blockIdx.x, c0, c1, S.pb_u + po, S.pb_w + po, sx, sx + FT_TILE, sx + 2 * FT_TILE,
+                        sx + 3 * FT_TILE);
 }
 
 // Row of the updated wake TEV[:itev+1] ++ LEV[:ilev+1] ++ FREE -> row of k_conv_old_tiled's partials (nold = rows of
@@ -1269,7 +1099,7 @@ __global__ void __launch_bounds__(256) k_conv_new(SimDev S, int s)
     }
 }
 
-__global__ void __launch_bounds__(256) k_finish_ov(SimDev S, int s, int R, int slots, int wt)
+__global__ void __launch_bounds__(256) k_finish_ov(SimDev S, int s, int R, int slots)
 {
     extern __shared__ double sm[];
     Step st;
@@ -1286,8 +1116,7 @@ __global__ void __launch_bounds__(256) k_finish_ov(SimDev S, int s, int R, int s
     const int i = st.i, nv = S.nv, nT = st.itev + 1, nL = st.ilev + 1;
     SrcView W = wake_view(S, nT, nL);
     const int nold = W.n - 2, npart = nold + 3;
-    const int chunks = wt ? WtGeom(npart, BlockMap(wake_view(S, st.itev, st.ilev)).total, R, slots).chunks
-                          : TiledGeom(npart, nold, R, slots).chunks;
+    const int chunks = TiledGeom(npart, nold, R, slots).chunks;
     const bool shed = S.lev_shed[i] != -1.0;
     const double dt = S.dt;
     for (long r = (long)(blockIdx.x - 2) * blockDim.x + threadIdx.x; r < W.n; r += (long)(gridDim.x - 2) * blockDim.x) {
@@ -1406,8 +1235,11 @@ __device__ __forceinline__ void persist_barrier(unsigned long long *bar, unsigne
     else grid_barrier(bar, k, counters);
 }
 
-template <bool CLUSTER, int NTH>
-__global__ void __launch_bounds__(NTH, 1) k_sim_persist(SimDev S, int nsteps, unsigned long long *bar)
+// 256 threads per CTA on both paths: 512 threads halve the O(N^2) phases' rounds but cap the kernel at 128 registers and
+// slow the solve by ~3 us: README case 30.4 / 25.7 us per step (exact / fast) against 28.7 / 24.0 with 256
+// (profiles/r02s_coop_probe_1.txt).
+template <bool CLUSTER>
+__global__ void __launch_bounds__(256, 1) k_sim_persist(SimDev S, int nsteps, unsigned long long *bar)
 {
     extern __shared__ double sm[];
     unsigned long long epoch = 0;
@@ -1823,7 +1655,7 @@ static void layout_case(SimDev &D, const ludvm_sim_params &p, const DevTables &t
     {   // one-CTA driver, fast mode: phase 1 from a shared-memory copy of the wake (cta_wof_tiled_fast)
         const long nth = cta_threads, nsl = P ? nth / (long)P : 0, nmax = (long)nstate + 2;
         D.wof_single = (compact && p.mode != LUDVM_EXACT_F64 && p.method == LUDVM_METHOD_FAURE && nsl >= 1 &&
-                        3 * nmax + 2 * (long)P * nsl <= (long)SOLVE_SCRATCH_DOUBLES(P, Nc, sum_nodes) && !getenv("LUDVM_NO_WOF_TILED")) ? 1 : 0;
+                        3 * nmax + 2 * (long)P * nsl <= (long)SOLVE_SCRATCH_DOUBLES(P, Nc, sum_nodes)) ? 1 : 0;
     }
     D.range_bad_init = (t.coords_in_window && vc4_in_safe_window(p.vc4) && !getenv("LUDVM_EXACT_FLAGS")) ? 0 : 1;
     D.range_bad = a.take<int>(1);
@@ -1892,7 +1724,6 @@ struct ludvm_sim {
     unsigned long long *d_bar = nullptr;  // grid-barrier counter of the cooperative path
     int coop_grid = 0;                    // CTAs of the cooperative kernel (0: path not available on this device)
     int cluster_ctas = 0;                 // CTAs of the single-cluster kernel (0: not available)
-    int cluster_threads = SIM_CLUSTER_THREADS;
     cudaStream_t cap_stream2 = nullptr;   // second capture stream: the overlapped step's old-wake convection branch
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     cudaStream_t cap_stream = nullptr;  // private stream used only to record graphs (the context's stream may be
@@ -1962,18 +1793,17 @@ static int bracket_of(long n)
 
 // Launch geometry of one step for every wake size up to 2^bracket.
 struct StepPlan {
-    int g1, g3, g4, g5, R, tchunks, slots, g_wt;
-    bool tiled, ov, tiled_exact, wt, db;
+    int g1, g3, g4, g5, R, tchunks, slots;
+    bool tiled, ov, tiled_exact;
     dim3 gto;
     dim3 gt;
     dim3 gte;
 };
 
 typedef void (*conv_old_fn)(SimDev, int, int);
-static conv_old_fn conv_old_kernel(int R, bool db)
+static conv_old_fn conv_old_kernel(int R)
 {
-    if (db) return R == 4 ? k_conv_old_tiled<4, true> : (R == 2 ? k_conv_old_tiled<2, true> : k_conv_old_tiled<1, true>);
-    return R == 4 ? k_conv_old_tiled<4, false> : (R == 2 ? k_conv_old_tiled<2, false> : k_conv_old_tiled<1, false>);
+    return R == 4 ? k_conv_old_tiled<4> : (R == 2 ? k_conv_old_tiled<2> : k_conv_old_tiled<1>);
 }
 
 static StepPlan plan_step(const ludvm_sim *s, int bracket)
@@ -2015,37 +1845,16 @@ static StepPlan plan_step(const ludvm_sim *s, int bracket)
                                                            ((long)sm * 2 * 6 + row_blocks - 1) / row_blocks));
         pl.gt = dim3((unsigned)row_blocks, (unsigned)pl.tchunks + 1);
         // overlapped step: old-wake convection on a second graph branch beside phase 1 + solve
-        pl.ov = D.P <= 256 && !getenv("LUDVM_NO_OVERLAP");
+        pl.ov = D.P <= 256;
         pl.gto = dim3((unsigned)((nw + 3 + FT_THREADS * pl.R - 1) / (FT_THREADS * pl.R)), (unsigned)SIM_TILED_CHUNKS_MAX);
         pl.slots = sm * (pl.R == 1 ? 3 : 2);   // resident CTAs of k_conv_old_tiled<R>: 70 registers -> 3 per SM, 112-120 -> 2
-        // double-buffered tiles (fast_tiled_block_db): opt-in, measured 5.88 s against 5.77 s on the dt = 2e-3 run
-        // (profiles/r02zd_hires.txt) -- with two or three resident CTAs per SM the barrier waits of one CTA are already
-        // covered by the others
-        pl.db = getenv("LUDVM_CONV_DB") != nullptr;
         {   // resident CTAs of the chosen instantiation, from the occupancy calculator
             int per_sm = 0;
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, conv_old_kernel(pl.R, pl.db), FT_THREADS, 0) == cudaSuccess &&
+            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, conv_old_kernel(pl.R), FT_THREADS, 0) == cudaSuccess &&
                 per_sm > 0)
                 pl.slots = sm * per_sm;
             else
                 cudaGetLastError();
-        }
-        if (const char *we = getenv("LUDVM_TILED_WAVES")) {   // "min,max": the wave search of TiledGeom (A/B)
-            int a = 0, b = 0;
-            if (sscanf(we, "%d,%d", &a, &b) == 2 && a >= 1 && b >= a && b < 64) pl.slots |= (a << 10) | (b << 16);
-        }
-        // warp-task form of the old-wake convection (k_conv_old_wt): 2 CTAs x 8 warps resident per SM
-        // (opt-in, LUDVM_CONV_WT=1: measured 5.40-5.58 s against 5.24 s for the thread-staged tiles on the 20 000-step
-        // dt = 2e-3 run -- whole-block chunks quantise the task count and a few long tasks free their slots late for
-        // the solve branch; profiles/r02f_hires.txt)
-        pl.wt = pl.ov && getenv("LUDVM_CONV_WT") != nullptr;
-        if (pl.wt) {
-            const char *re = getenv("LUDVM_WT_R");
-            pl.R = re ? atoi(re) : (rows_up >= 8192 ? 4 : (rows_up >= 4096 ? 2 : 1));
-            const char *ro = getenv("LUDVM_WT_ROUNDS");
-            pl.slots = sm * 16 * (ro ? std::max(1, atoi(ro)) : WT_ROUNDS);   // the task budget: rounds x resident warps
-            const long nrg_max = (nw + 3 + 32 * pl.R - 1) / (32 * pl.R);
-            pl.g_wt = (int)((std::max<long>(pl.slots, nrg_max) + 7) / 8);
         }
         pl.g5 = 1 + (int)std::max<long>(1, std::min<long>((nw + 255) / 256, (long)sm * 8));
     }
@@ -2066,19 +1875,14 @@ static void enqueue_step_kernel(const ludvm_sim *s, const StepPlan &pl, int whic
     case 2:
         if (pl.tiled_exact) k_conv_partials_exact_tiled<<<pl.gte, ET_THREADS, 0, cs>>>(D, k);
         else if (!pl.tiled) k_conv_partials<<<pl.g3, 256, 0, cs>>>(D, k);
-        else if (pl.wt) {
-            if (pl.R == 4) k_conv_old_wt<4><<<pl.g_wt, 256, sizeof(WtSmem), cs>>>(D, k, pl.slots);
-            else if (pl.R == 2) k_conv_old_wt<2><<<pl.g_wt, 256, sizeof(WtSmem), cs>>>(D, k, pl.slots);
-            else k_conv_old_wt<1><<<pl.g_wt, 256, sizeof(WtSmem), cs>>>(D, k, pl.slots);
-        } else if (pl.ov) {
-            conv_old_kernel(pl.R, pl.db)<<<pl.gto, FT_THREADS, 0, cs>>>(D, k, pl.slots);
-        } else if (pl.R == 4) k_conv_partials_tiled<4><<<pl.gt, FT_THREADS, 0, cs>>>(D, k, pl.tchunks);
+        else if (pl.ov) conv_old_kernel(pl.R)<<<pl.gto, FT_THREADS, 0, cs>>>(D, k, pl.slots);
+        else if (pl.R == 4) k_conv_partials_tiled<4><<<pl.gt, FT_THREADS, 0, cs>>>(D, k, pl.tchunks);
         else if (pl.R == 2) k_conv_partials_tiled<2><<<pl.gt, FT_THREADS, 0, cs>>>(D, k, pl.tchunks);
         else k_conv_partials_tiled<1><<<pl.gt, FT_THREADS, 0, cs>>>(D, k, pl.tchunks);
         break;
     case 4: k_conv_new<<<pl.g5, 256, 0, cs>>>(D, k); break;
     default:
-        if (pl.ov) k_finish_ov<<<pl.g4, 256, s->finish_smem, cs>>>(D, k, pl.R, pl.slots, pl.wt ? 1 : 0);
+        if (pl.ov) k_finish_ov<<<pl.g4, 256, s->finish_smem, cs>>>(D, k, pl.R, pl.slots);
         else k_finish<<<pl.g4, 256, s->finish_smem, cs>>>(D, k, pl.tchunks);
         break;
     }
@@ -2106,13 +1910,11 @@ static int build_graph(ludvm_sim *s, int bracket, int ksteps, cudaGraphExec_t *o
             enqueue_step_kernel(s, pl, 0, k, cs);
             enqueue_step_kernel(s, pl, 2, k, cs2);
             enqueue_step_kernel(s, pl, 1, k, cs);
-            // The new-vortex / bound-vortex terms need the solve, not the old-wake sums, so they could run beside the bulk
-            // kernel instead of after the join (LUDVM_CONV_NEW_EARLY=1): measured no better (5.88 vs 5.84 s).
-            const bool new_after_join = getenv("LUDVM_CONV_NEW_EARLY") == nullptr;
-            if (!new_after_join) enqueue_step_kernel(s, pl, 4, k, cs);
+            // The new-vortex / bound-vortex terms need the solve, not the old-wake sums; enqueueing them beside the bulk
+            // kernel instead of after the join measured no better (5.88 vs 5.84 s).
             CUDA_TRY(cudaEventRecord(s->ev_join, cs2));
             CUDA_TRY(cudaStreamWaitEvent(cs, s->ev_join, 0));
-            if (new_after_join) enqueue_step_kernel(s, pl, 4, k, cs);
+            enqueue_step_kernel(s, pl, 4, k, cs);
             enqueue_step_kernel(s, pl, 3, k, cs);
         } else {
             for (int which = 0; which < 4; which++) enqueue_step_kernel(s, pl, which, k, cs);
@@ -2140,9 +1942,6 @@ static int set_smem_limits(size_t solve_smem, size_t finish_smem)
     }
     if (finish_smem > 48 * 1024)
         CUDA_TRY(cudaFuncSetAttribute(k_finish, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)finish_smem));
-    CUDA_TRY(cudaFuncSetAttribute(k_conv_old_wt<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(WtSmem)));
-    CUDA_TRY(cudaFuncSetAttribute(k_conv_old_wt<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(WtSmem)));
-    CUDA_TRY(cudaFuncSetAttribute(k_conv_old_wt<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(WtSmem)));
     return LUDVM_OK;
 }
 
@@ -2167,7 +1966,7 @@ LUDVM_API int ludvm_sim_create(ludvm_ctx *ctx, const ludvm_sim_params *p, const 
     // exact mode splits the summation tree deeper: its large-wake convection kernel runs one 128-thread CTA per
     // (128 rows, tree node) and wants several waves of 4 CTAs/SM (the split depth never changes a result).  Measured on
     // the 20 000-step dt = 2e-3 run in exact mode: 96 x SMs 16.9 s, 192 x 15.1 s, 384 x 14.4 s.
-    const int target = cta ? 2 * (RAMESH_THREADS / 32) : ctx->sm_count * (p->mode == LUDVM_EXACT_F64 ? (getenv("LUDVM_EXACT_TARGET") ? atoi(getenv("LUDVM_EXACT_TARGET")) : 384) : 48);
+    const int target = cta ? 2 * (RAMESH_THREADS / 32) : ctx->sm_count * (p->mode == LUDVM_EXACT_F64 ? 384 : 48);
     // shared-memory staging area of the block-wide folds / integrals: all Nc Fourier integrands, or 64 partials of
     // every (row, component), in one batch
     const int sum_nodes = clamp_sum_nodes(p->P, p->Nc, std::max<long>(cta ? 1024 : 4096, std::max<long>(p->Nc * p->P, cta ? 0 : 2 * p->P * 65)));
@@ -2197,34 +1996,26 @@ LUDVM_API int ludvm_sim_create(ludvm_ctx *ctx, const ludvm_sim_params *p, const 
     {   // cooperative path: needs cooperative-launch support and one resident CTA per SM
         int coop = 0, per_sm = 0;
         cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, ctx->device);
-        if (coop && !cta && cudaFuncSetAttribute(k_sim_persist<false, 256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s->solve_smem) == cudaSuccess &&
-            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sim_persist<false, 256>, 256, s->solve_smem) == cudaSuccess && per_sm >= 1)
+        if (coop && !cta && cudaFuncSetAttribute(k_sim_persist<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s->solve_smem) == cudaSuccess &&
+            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sim_persist<false>, 256, s->solve_smem) == cudaSuccess && per_sm >= 1)
             s->coop_grid = ctx->sm_count;
-        if (const char *ge = getenv("LUDVM_COOP_GRID"))   // experiments: a smaller persistent grid (>= 4 CTAs)
-            if (s->coop_grid) s->coop_grid = std::max(4, std::min(s->coop_grid, atoi(ge)));
         cudaGetLastError();
         // cluster path: one thread-block cluster of SIM_CLUSTER_CTAS CTAs (16 needs the non-portable opt-in), if the
         // device can co-schedule it with this much shared memory per CTA
         if (!cta && !getenv("LUDVM_NO_CLUSTER")) {
-            const char *ce = getenv("LUDVM_CLUSTER_CTAS");
-            int want = ce ? atoi(ce) : SIM_CLUSTER_CTAS;
-            want = want >= 16 ? 16 : (want >= 8 ? 8 : 4);
-            const char *te = getenv("LUDVM_CLUSTER_THREADS");
-            s->cluster_threads = (te && atoi(te) == 512) ? 512 : SIM_CLUSTER_THREADS;
-            const void *kern = s->cluster_threads == 512 ? (const void *)k_sim_persist<true, 512>
-                                                         : (const void *)k_sim_persist<true, SIM_CLUSTER_THREADS>;
+            const void *kern = (const void *)k_sim_persist<true>;
             if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s->solve_smem) == cudaSuccess &&
-                (want <= 8 || cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess)) {
+                cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess) {
                 cudaLaunchConfig_t cfg = {};
-                cfg.gridDim = dim3(want);
-                cfg.blockDim = dim3(s->cluster_threads);
+                cfg.gridDim = dim3(SIM_CLUSTER_CTAS);
+                cfg.blockDim = dim3(256);
                 cfg.dynamicSmemBytes = s->solve_smem;
                 cudaLaunchAttribute at[1];
                 at[0].id = cudaLaunchAttributeClusterDimension;
-                at[0].val.clusterDim.x = want; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+                at[0].val.clusterDim.x = SIM_CLUSTER_CTAS; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
                 cfg.attrs = at; cfg.numAttrs = 1;
                 int nclusters = 0;
-                if (cudaOccupancyMaxActiveClusters(&nclusters, kern, &cfg) == cudaSuccess && nclusters >= 1) s->cluster_ctas = want;
+                if (cudaOccupancyMaxActiveClusters(&nclusters, kern, &cfg) == cudaSuccess && nclusters >= 1) s->cluster_ctas = SIM_CLUSTER_CTAS;
             }
             cudaGetLastError();
         }
@@ -2253,26 +2044,21 @@ LUDVM_API int ludvm_sim_run(ludvm_sim *s, long nsteps)
     }
     // smallest wakes: ONE thread-block cluster with the hardware cluster barrier between the phases
     if (s->cluster_ctas >= 4) {
-        const char *me = getenv("LUDVM_CLUSTER_MAX_WAKE");
-        const long cmax = me ? atol(me) : SIM_CLUSTER_MAX_WAKE;
-        const long last_small = (cmax - 2 - (long)s->p.nfree) / 2;
+        const long last_small = (SIM_CLUSTER_MAX_WAKE - 2 - (long)s->p.nfree) / 2;
         long k = std::min(todo, last_small - s->steps_enqueued);
         if (k > 0) {
             SimDev dc = s->d;
-            dc.target_warps = s->cluster_ctas * (s->cluster_threads / 32);
+            dc.target_warps = s->cluster_ctas * 8;
             cudaLaunchConfig_t cfg = {};
             cfg.gridDim = dim3(s->cluster_ctas);
-            cfg.blockDim = dim3(s->cluster_threads);
+            cfg.blockDim = dim3(256);
             cfg.dynamicSmemBytes = s->solve_smem;
             cfg.stream = s->ctx->stream;
             cudaLaunchAttribute at[1];
             at[0].id = cudaLaunchAttributeClusterDimension;
             at[0].val.clusterDim.x = s->cluster_ctas; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
             cfg.attrs = at; cfg.numAttrs = 1;
-            if (s->cluster_threads == 512)
-                CUDA_TRY(cudaLaunchKernelEx(&cfg, k_sim_persist<true, 512>, dc, (int)k, (unsigned long long *)nullptr));
-            else
-                CUDA_TRY(cudaLaunchKernelEx(&cfg, k_sim_persist<true, SIM_CLUSTER_THREADS>, dc, (int)k, (unsigned long long *)nullptr));
+            CUDA_TRY(cudaLaunchKernelEx(&cfg, k_sim_persist<true>, dc, (int)k, (unsigned long long *)nullptr));
             s->ctx->launches++;
             s->steps_enqueued += k;
             todo -= k;
@@ -2291,7 +2077,7 @@ LUDVM_API int ludvm_sim_run(ludvm_sim *s, long nsteps)
             unsigned long long *bar = s->d_bar;
             void *args[] = {&dc, &ki, &bar};
             CUDA_TRY(cudaMemsetAsync(s->d_bar, 0, COOP_BAR_WORDS * sizeof(unsigned long long), s->ctx->stream));
-            CUDA_TRY(cudaLaunchCooperativeKernel((const void *)k_sim_persist<false, 256>, dim3(s->coop_grid), dim3(256), args, s->solve_smem, s->ctx->stream));
+            CUDA_TRY(cudaLaunchCooperativeKernel((const void *)k_sim_persist<false>, dim3(s->coop_grid), dim3(256), args, s->solve_smem, s->ctx->stream));
             s->ctx->launches++;
             s->steps_enqueued += k;
             todo -= k;
@@ -2513,12 +2299,10 @@ LUDVM_API int ludvm_sweep_run(ludvm_ctx *ctx, long ncases, const ludvm_sim_param
     std::vector<SimDev> host_cases((size_t)ncases);
     std::vector<DevTables> dts((size_t)ncases);
     const bool ramesh = p0.method == LUDVM_METHOD_RAMESH;
-    const char *te = getenv("LUDVM_SWEEP_THREADS");
     // threads per case: 256 (three resident cases per SM) in fast mode; in exact mode 128 threads with the cos/sin(n theta)
     // tables read from global memory put six cases on an SM and win (4096-case sweep, 256 / 128 threads: fast 0.511 / 0.537 s,
-    // exact 0.899 / 0.832 s; profiles/r02v_sweep_threads.txt).  LUDVM_SWEEP_THREADS overrides.
-    const int want_threads = te ? atoi(te) : (p0.mode == LUDVM_EXACT_F64 ? 128 : CTA_THREADS);
-    const int cta_threads = (!ramesh && want_threads == 128) ? 128 : CTA_THREADS;
+    // exact 0.899 / 0.832 s; profiles/r02v_sweep_threads.txt).
+    const int cta_threads = (!ramesh && p0.mode == LUDVM_EXACT_F64) ? 128 : CTA_THREADS;
     const int target = 2 * (cta_threads / 32), sum_nodes = clamp_sum_nodes(p0.P, p0.Nc, std::max<long>(256, p0.Nc * p0.P));
     Arena measure;
     for (long c = 0; c < ncases; c++) {

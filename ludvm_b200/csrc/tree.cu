@@ -48,7 +48,7 @@ struct TreeGeom {
     double tdens;            // targets per unit area when they are a uniform grid (0: unknown): cells that hold more than P2
                              // grid points carry a local field even where they hold few sources
     int pth;                 // a cell with more than pth source vortices is represented by proxies (and carries a local field)
-    int L, P1, P2, generic_up;   // generic_up = 1: children's proxies go through the tile loop of k_tree_up too (A/B)
+    int L, P1, P2;
     double s[TR_MAX_P1];     // Chebyshev points of the second kind on [-1, 1], exactly antisymmetric
     double bw[TR_MAX_P1];    // barycentric weights
 };
@@ -276,7 +276,7 @@ __global__ void __launch_bounds__(TU_THREADS) k_tree_up(const __grid_constant__ 
     const int b = startS[(long)c << sh], e = startS[((long)c + 1) << sh];
     if (e - b <= G.pth) return;
     __shared__ double Lx[TU_TILE][TR_MAX_P1], Lz[TU_TILE][TR_MAX_P1], gt[TU_TILE];
-    __shared__ int seg_type[4], seg_a[4], seg_pre[5], nseg_s, prox_ch[4], prox_cell[4], nprox_s;
+    __shared__ int seg_a[4], seg_pre[5], nseg_s, prox_ch[4], prox_cell[4], nprox_s;
     __shared__ double Tq[2][TR_MAX_P1][TR_MAX_P1], Qc[TR_MAX_P1 * TR_MAX_P1], Tm[TR_MAX_P1 * TR_MAX_P1];
     const int P1 = G.P1, P2 = G.P2;
     const double h = ldexp(G.side, -(l + 1)), inv_h = 1.0 / h;
@@ -287,16 +287,14 @@ __global__ void __launch_bounds__(TU_THREADS) k_tree_up(const __grid_constant__ 
     if (tid == 0) {
         int ns = 0, run = 0, np = 0;
         if (l == G.L) {
-            seg_type[0] = 0; seg_a[0] = b; seg_pre[0] = 0; run = e - b; ns = 1;
+            seg_a[0] = b; seg_pre[0] = 0; run = e - b; ns = 1;
         } else {
             for (int ch = 0; ch < 4; ch++) {
                 const long cc = 4L * c + ch;
                 const int cb = startS[cc << (sh - 2)], ce = startS[(cc + 1) << (sh - 2)], n = ce - cb;
                 if (n == 0) continue;
-                if (n > G.pth && G.generic_up == 0) { prox_ch[np] = ch; prox_cell[np] = (int)cc; np++; continue; }
-                seg_pre[ns] = run;
-                if (n > G.pth) { seg_type[ns] = 1 + ch; seg_a[ns] = (int)cc; run += P2; }
-                else { seg_type[ns] = 0; seg_a[ns] = cb; run += n; }
+                if (n > G.pth) { prox_ch[np] = ch; prox_cell[np] = (int)cc; np++; continue; }
+                seg_pre[ns] = run; seg_a[ns] = cb; run += n;
                 ns++;
             }
         }
@@ -347,16 +345,9 @@ __global__ void __launch_bounds__(TU_THREADS) k_tree_up(const __grid_constant__ 
             if (valid) {
                 int sg = 0;
                 while (sg + 1 < nseg && seg_pre[sg + 1] <= j) sg++;
-                const int o = j - seg_pre[sg], ty = seg_type[sg];
-                if (ty == 0) {
-                    const int p = seg_a[sg] + o;
-                    xi = dim ? (zs[p] - cz) * inv_h : (xs[p] - cx) * inv_h;
-                    gval = gs[p];
-                } else {
-                    const int ch = ty - 1, k1 = o / P1, k2 = o - k1 * P1;
-                    xi = dim ? (G.s[k2] + (double)((ch >> 1) * 2 - 1)) * 0.5 : (G.s[k1] + (double)((ch & 1) * 2 - 1)) * 0.5;
-                    gval = qchild[(long)seg_a[sg] * P2 + o];
-                }
+                const int p = seg_a[sg] + j - seg_pre[sg];
+                xi = dim ? (zs[p] - cz) * inv_h : (xs[p] - cx) * inv_h;
+                gval = gs[p];
             }
             double sum = 0.0, tk[(TR_MAX_P1 + 3) / 4];
             int hit = -1;
@@ -499,8 +490,7 @@ struct TreeEval {
     double *u, *w;                         // original order
     double *uloc, *wloc;                   // local fields, laid out like qhat
     unsigned long long *pairs;             // pair evaluations (diagnostic)
-    int fmm, np;                           // 0: pure treecode (every far list evaluated at the targets)
-    int gemm;                              // 1: proxy cells of the M2L lists are applied by k_tree_m2l_gemm, not here
+    int np;
 };
 
 struct TreeSmem {
@@ -731,7 +721,7 @@ __global__ void __launch_bounds__(TE_THREADS, 4) k_tree_eval(const __grid_consta
 {
     __shared__ __align__(16) TreeSmem sm;
     const int L = G.L, P2 = G.P2;
-    const int nm2l = A.fmm ? (int)level_offset(L + 1) : 0;
+    const int nm2l = (int)level_offset(L + 1);
     if ((int)blockIdx.x < nm2l) {
         // M2L item: cell c of level l
         int l = 2;
@@ -741,7 +731,7 @@ __global__ void __launch_bounds__(TE_THREADS, 4) k_tree_eval(const __grid_consta
         if (A.startT[((long)c + 1) << sh] == A.startT[(long)c << sh]) return;           // none of this rank's targets below
         if ((int)blockIdx.y >= (((P2 + TE_THREADS - 1) / TE_THREADS + 3) >> 2)) return;
         const int cx = (int)compact16((unsigned)c), cz = (int)compact16((unsigned)c >> 1);
-        const int total = tree_build_list(G, A, cx, cz, l, false, l, l, sm, A.gemm != 0);
+        const int total = tree_build_list(G, A, cx, cz, l, false, l, l, sm, true);   // proxy cells: k_tree_m2l_dmma
         const double h = ldexp(G.side, -(l + 1));
         const long off = (level_offset(l) + c) * P2;
         TgtNodePts T{G.x0 + (2.0 * cx + 1.0) * h, G.z0 + (2.0 * cz + 1.0) * h, h, G.s, G.P1, A.uloc + off, A.wloc + off};
@@ -753,7 +743,7 @@ __global__ void __launch_bounds__(TE_THREADS, 4) k_tree_eval(const __grid_consta
     const int tb = A.startT[c], te = A.startT[c + 1];
     if (tb == te) return;
     if ((int)blockIdx.y >= (((te - tb + TE_THREADS - 1) / TE_THREADS + 3) >> 2)) return;
-    const int lstar = A.fmm ? tree_local_level(G, A.startS, c) : 1;
+    const int lstar = tree_local_level(G, A.startS, c);
     const int total = tree_build_list(G, A, (int)compact16((unsigned)c), (int)compact16((unsigned)c >> 1), L, true, lstar + 1, L, sm);
     if (threadIdx.x == 0 && blockIdx.y == 0 && A.pairs) atomicAdd(A.pairs, (unsigned long long)(te - tb) * (unsigned long long)total);
     TgtLeafPts T{A.permT, A.xt, A.zt, A.u, A.w};
@@ -764,24 +754,14 @@ __global__ void __launch_bounds__(TE_THREADS, 4) k_tree_eval(const __grid_consta
 // M2L between proxy cells as matrix products.  The proxies of a cell sit at fixed points of the cell, so the velocity
 // that the P2 proxies of cell B induce at the P2 points of cell A of the same level depends on the cells' offset
 // (dx, dz) in [-3, 3]^2 only: U_A += Mu[l][off] q_B, W_A += Mw[l][off] q_B with two P2 x P2 matrices per level and offset
-// (per level: the core radius does not scale with the cells).  An entry costs one DFMA per component instead of the 13
-// slots + MUFU of a pair evaluation, and a matrix is shared by every pair of cells with that offset: a CTA owns a
-// (TM_TI points) x (TM_TC cells) tile of the local fields of one level, walks the 40 offsets and the P2 proxies with
-// register-tiled outer products, tiles of the matrices and of the proxy strengths prefetched into registers while the
-// previous ones are consumed.  Lists entries that are plain vortices (cells with <= pth of them) stay with k_tree_eval.
-// The order of the sums is fixed (offsets, then proxies, ascending), whatever tile a cell lands in.
-// The kernel is bound by shared-memory bandwidth, not by the FP64 pipe (ncu, profiles/r03g_k_tree_m2l_gemm_*: l1tex 85 %
-// busy, FP64 45 %, top stall short scoreboard): a 2 x 4 thread tile reads 64 bytes of operands per 16 DFMA = 4 bytes
-// per DFMA, and the SM returns 128 bytes per clock for 64 FP64 lanes, i.e. 2 bytes per DFMA at full rate.  2^20 vortices:
-// 1.15e10 DFMA in 2.8 ms.  Measured and dropped (profiles/r03f_*, r03h_*, r03i_*): 4 x 4 thread tiles (3 bytes per DFMA)
-// as 64 x 32 CTA tiles with 128 threads, 64 x 64 with 256 threads at one or two CTAs per SM: 3.2 / 4.8 / 3.5 ms; a lane
-// map with fewer wavefronts per LDS: no change (the limit is bytes returned, not wavefronts).  What it wants is the FP64
-// tensor-core path (mma.sync m8n8k4.f64 with warp-level register reuse): not built.
+// (per level: the core radius does not scale with the cells).  An entry costs one FMA per component instead of the 13
+// slots + MUFU of a pair evaluation, and a matrix is shared by every pair of cells with that offset.  k_tree_m2l_mats
+// builds the matrices; k_tree_m2l_dmma applies them on the FP64 tensor cores, a CTA per (points) x (cells) tile of the
+// local fields of one level, walking the 40 offsets and the P2 proxies.  List entries that are plain vortices (cells
+// with <= pth of them) stay with k_tree_eval.  The order of the sums is fixed (offsets, then proxies, ascending),
+// whatever tile a cell lands in.  Measurements: DESIGN.md 4b.
 // ---------------------------------------------------------------------------------------------------
 #define TM_NOFF 49
-#define TM_TI 32
-#define TM_TC 64
-#define TM_JC 16
 
 // matrices [level - 2][off][j][i], i fastest
 __global__ void __launch_bounds__(128) k_tree_m2l_mats(const __grid_constant__ TreeGeom G, double *Mu, double *Mw)
@@ -820,132 +800,11 @@ __global__ void __launch_bounds__(256) k_tree_alist(const __grid_constant__ Tree
     alist[level_offset(l) + ((long)par << (2 * (l - 1))) + atomicAdd(acount + 4 * l + par, 1)] = (int)c;
 }
 
-__global__ void __launch_bounds__(256, 2) k_tree_m2l_gemm(const __grid_constant__ TreeGeom G, const int *startS, const int *alist,
-                                                          const int *acount, const double *Mu, const double *Mw,
-                                                          const double *qhat, double *uloc, double *wloc)
-{
-    // blockIdx.y -> (level, parity, cell tile): level l owns 4 x ceil(4^(l-1) / TM_TC) tiles
-    const int P2 = G.P2, tid = threadIdx.x;
-    int l = 2, tile = blockIdx.y, ntp;
-    for (;; l++) {
-        ntp = (int)(((1L << (2 * (l - 1))) + TM_TC - 1) / TM_TC);
-        if (tile < 4 * ntp) break;
-        tile -= 4 * ntp;
-    }
-    const int par = tile / ntp;
-    tile -= par * ntp;
-    const int nA = acount[4 * l + par];
-    if (tile * TM_TC >= nA) return;
-    const long abase = level_offset(l) + ((long)par << (2 * (l - 1)));
-    const int i0 = blockIdx.x * TM_TI;
-    __shared__ int Acell[TM_TC], Bcell[TM_TC];
-    __shared__ __align__(16) double sMu[TM_JC][TM_TI], sMw[TM_JC][TM_TI], sQ[TM_JC][TM_TC + 2];   // (+2: the stores of a
-                                                                        // strength tile walk down a column of sQ)
-    const int ti = tid & 15, tc = tid >> 4;              // thread tile: points i0 + 2 ti + {0, 1}, cells 4 tc + {0..3}
-    double au[2][4], aw[2][4];
-#pragma unroll
-    for (int a = 0; a < 2; a++)
-#pragma unroll
-        for (int b = 0; b < 4; b++) au[a][b] = aw[a][b] = 0.0;
-    if (tid < TM_TC) Acell[tid] = tile * TM_TC + tid < nA ? alist[abase + tile * TM_TC + tid] : -1;
-    const double *Ml_u = Mu + (size_t)(l - 2) * TM_NOFF * P2 * P2, *Ml_w = Mw + (size_t)(l - 2) * TM_NOFF * P2 * P2;
-    const double *ql = qhat + level_offset(l) * P2;
-    const int sh = 2 * (G.L - l), nc = 1 << l;
-    // loader roles: matrices -- element e = tid + 256 q (q < 2) of a TM_JC x TM_TI tile (i fastest); strengths -- element
-    // e = tid + 256 q (q < 4) of a TM_TC x TM_JC tile (j fastest inside a cell)
-    for (int off = 0; off < TM_NOFF; off++) {
-        const int dx = off % 7 - 3, dz = off / 7 - 3;
-        if (max(abs(dx), abs(dz)) <= 1) continue;
-        // B's parent must be a neighbour of A's parent: dx in [-2 - px, 3 - px] for the parity px of A, likewise dz
-        if (dx < -2 - (par & 1) || dx > 3 - (par & 1) || dz < -2 - (par >> 1) || dz > 3 - (par >> 1)) continue;
-        __syncthreads();                                   // the previous offset's tiles and Bcell are no longer read
-        if (tid < TM_TC) {
-            int bcell = -1;
-            const int a = Acell[tid];
-            if (a >= 0) {
-                const int ax = (int)compact16((unsigned)a), az = (int)compact16((unsigned)a >> 1), bx = ax + dx, bz = az + dz;
-                if (bx >= 0 && bz >= 0 && bx < nc && bz < nc && abs((bx >> 1) - (ax >> 1)) <= 1 && abs((bz >> 1) - (az >> 1)) <= 1) {
-                    const long bc = morton2(bx, bz);
-                    if (startS[(bc + 1) << sh] - startS[bc << sh] > G.pth) bcell = (int)bc;
-                }
-            }
-            Bcell[tid] = bcell;
-        }
-        const int any = __syncthreads_or(tid < TM_TC && Bcell[tid] >= 0);
-        if (!any) continue;
-        const double *Mo_u = Ml_u + (size_t)off * P2 * P2, *Mo_w = Ml_w + (size_t)off * P2 * P2;
-        double pmu[2], pmw[2], pq[4];
-        auto fetch = [&](int j0) {
-#pragma unroll
-            for (int q = 0; q < 2; q++) {
-                const int e = tid + 256 * q, jj = e / TM_TI, ii = e - jj * TM_TI, j = j0 + jj, i = i0 + ii;
-                const bool ok = j < P2 && i < P2;
-                pmu[q] = ok ? Mo_u[(size_t)j * P2 + i] : 0.0;
-                pmw[q] = ok ? Mo_w[(size_t)j * P2 + i] : 0.0;
-            }
-#pragma unroll
-            for (int q = 0; q < 4; q++) {
-                const int e = tid + 256 * q, cc = e / TM_JC, jj = e - cc * TM_JC, j = j0 + jj, bcell = Bcell[cc];
-                pq[q] = (bcell >= 0 && j < P2) ? ql[(size_t)bcell * P2 + j] : 0.0;
-            }
-        };
-        auto put = [&]() {
-#pragma unroll
-            for (int q = 0; q < 2; q++) {
-                const int e = tid + 256 * q, jj = e / TM_TI, ii = e - jj * TM_TI;
-                sMu[jj][ii] = pmu[q];
-                sMw[jj][ii] = pmw[q];
-            }
-#pragma unroll
-            for (int q = 0; q < 4; q++) {
-                const int e = tid + 256 * q, cc = e / TM_JC, jj = e - cc * TM_JC;
-                sQ[jj][cc] = pq[q];
-            }
-        };
-        fetch(0);
-        for (int j0 = 0; j0 < P2; j0 += TM_JC) {
-            __syncthreads();                               // the previous chunk has been consumed
-            put();
-            __syncthreads();
-            if (j0 + TM_JC < P2) fetch(j0 + TM_JC);        // in flight during the products
-#pragma unroll
-            for (int jj = 0; jj < TM_JC; jj++) {
-                const double2 mu = *reinterpret_cast<const double2 *>(&sMu[jj][2 * ti]);
-                const double2 mw = *reinterpret_cast<const double2 *>(&sMw[jj][2 * ti]);
-                const double2 qa = *reinterpret_cast<const double2 *>(&sQ[jj][4 * tc]);
-                const double2 qb = *reinterpret_cast<const double2 *>(&sQ[jj][4 * tc + 2]);
-                const double q4[4] = {qa.x, qa.y, qb.x, qb.y};
-#pragma unroll
-                for (int b = 0; b < 4; b++) {
-                    au[0][b] = fma(mu.x, q4[b], au[0][b]);
-                    au[1][b] = fma(mu.y, q4[b], au[1][b]);
-                    aw[0][b] = fma(mw.x, q4[b], aw[0][b]);
-                    aw[1][b] = fma(mw.y, q4[b], aw[1][b]);
-                }
-            }
-        }
-    }
-    __syncthreads();
-#pragma unroll
-    for (int b = 0; b < 4; b++) {
-        const int a = Acell[4 * tc + b];
-        if (a < 0) continue;
-        const size_t o = (size_t)(level_offset(l) + a) * P2;
-#pragma unroll
-        for (int k = 0; k < 2; k++) {
-            const int i = i0 + 2 * ti + k;
-            if (i < P2) {
-                uloc[o + i] += au[k][b];       // (k_tree_eval stored the list's plain-vortex part, or zero, before)
-                wloc[o + i] += aw[k][b];
-            }
-        }
-    }
-}
-
-// The same products on the FP64 tensor cores (mma.sync.m8n8k4.f64; Blackwell's tcgen05 has no FP64 kind, so this is the
+// The M2L products on the FP64 tensor cores (mma.sync.m8n8k4.f64; Blackwell's tcgen05 has no FP64 kind, so this is the
 // FP64 tensor path of sm_100a).  CTA tile 64 points x 64 cells, 8 warps as 4 (points) x 2 (cells), warp tile 16 x 32 =
 // 2 x 4 MMA tiles per component: per k-step of 4 proxies a thread reads 8 doubles of fragments for 16 MMAs (4096 FMA per
-// warp), 0.5 bytes of shared memory per FMA where the CUDA-core version above needs 4.  Fragment layout (PTX ISA, m8n8k4
+// warp), 0.5 bytes of shared memory per FMA where a register-tiled CUDA-core loop needs 4 and is bound by shared-memory
+// bandwidth.  Fragment layout (PTX ISA, m8n8k4
 // .f64): A[row = lane >> 2][k = lane & 3], B[k = lane & 3][col = lane >> 2], C[row = lane >> 2][col = 2 (lane & 3) + {0, 1}].
 // Row strides of 68 doubles make the fragment loads conflict-free (stride = 4 mod 16 bank pairs).
 #define TD_TI 64
@@ -1276,7 +1135,7 @@ struct TreeBufs {
     unsigned long long *pairs;
     int *maxcnt;   // [2]: largest leaf population, sources / targets
 };
-static size_t tree_layout(Arena &a, TreeBufs &b, long nw, long np, int L, int P2, bool fmm, bool gemm)
+static size_t tree_layout(Arena &a, TreeBufs &b, long nw, long np, int L, int P2)
 {
     const size_t ncell = (size_t)1 << (2 * L);
     b.keyS = a.take<int>(nw); b.slotS = a.take<int>(nw); b.keyT = a.take<int>(np); b.slotT = a.take<int>(np);
@@ -1285,11 +1144,11 @@ static size_t tree_layout(Arena &a, TreeBufs &b, long nw, long np, int L, int P2
     b.tmpS = a.take<int>(nw); b.permS = a.take<int>(nw); b.tmpT = a.take<int>(np); b.permT = a.take<int>(np);
     b.xs = a.take<double>(nw); b.zs = a.take<double>(nw); b.gs = a.take<double>(nw);
     b.qhat = a.take<double>((size_t)level_offset(L + 1) * P2);
-    b.uloc = a.take<double>(fmm ? (size_t)level_offset(L + 1) * P2 : 1);
-    b.wloc = a.take<double>(fmm ? (size_t)level_offset(L + 1) * P2 : 1);
-    b.Mu = a.take<double>(gemm ? (size_t)(L - 1) * TM_NOFF * P2 * P2 : 1);
-    b.Mw = a.take<double>(gemm ? (size_t)(L - 1) * TM_NOFF * P2 * P2 : 1);
-    b.alist = a.take<int>(gemm ? (size_t)level_offset(L + 1) : 1);
+    b.uloc = a.take<double>((size_t)level_offset(L + 1) * P2);
+    b.wloc = a.take<double>((size_t)level_offset(L + 1) * P2);
+    b.Mu = a.take<double>((size_t)(L - 1) * TM_NOFF * P2 * P2);
+    b.Mw = a.take<double>((size_t)(L - 1) * TM_NOFF * P2 * P2);
+    b.alist = a.take<int>((size_t)level_offset(L + 1));
     b.acount = a.take<int>(64);
     b.pairs = a.take<unsigned long long>(1);
     b.maxcnt = a.take<int>(2);
@@ -1348,8 +1207,7 @@ static int tree_velocity_device(ludvm_ctx *ctx, const double *g, const double *x
         // interaction is ~10x cheaper than a pair evaluation, so a cell is worth representing by more proxies than it
         // has vortices (order 14, 2^20 vortices: 7.7 -> 5.7 ms with leaves of 160; profiles/r03q_tree_probe_pth.txt)
         G.pth = std::max(1, P2 / 4);
-        if (const char *pe = getenv("LUDVM_TREE_PROXY_MIN")) G.pth = std::max(1, std::min(P2, (int)(atof(pe) * P2)));   // fraction of P2 (A/B)
-        G.L = L; G.P1 = P1; G.P2 = P2; G.generic_up = getenv("LUDVM_TREE_GENERIC_UP") ? 1 : 0;
+        G.L = L; G.P1 = P1; G.P2 = P2;
         for (int k = 0; k < P1; k++) {
             G.s[k] = std::sin(M_PI * (double)(order - 2 * k) / (double)(2 * order));
             G.bw[k] = ((k & 1) ? -1.0 : 1.0) * ((k == 0 || k == order) ? 0.5 : 1.0);
@@ -1359,12 +1217,10 @@ static int tree_velocity_device(ludvm_ctx *ctx, const double *g, const double *x
 
         Arena sizer{nullptr};
         TreeBufs B;
-        const bool fmm = !getenv("LUDVM_TREE_NO_FMM");
-        const bool gemm = fmm && !getenv("LUDVM_TREE_NO_GEMM");
-        const size_t bytes = tree_layout(sizer, B, nw, np_, L, P2, fmm, gemm);
+        const size_t bytes = tree_layout(sizer, B, nw, np_, L, P2);
         if ((rc = scratch_reserve(ctx, 8, bytes, &p))) return rc;
         Arena ar{(char *)p};
-        tree_layout(ar, B, nw, np_, L, P2, fmm, gemm);
+        tree_layout(ar, B, nw, np_, L, P2);
         const int ncell = 1 << (2 * L);
         CUDA_TRY(cudaMemsetAsync(B.cntS, 0, (size_t)(ncell + 1) * sizeof(int), st));
         CUDA_TRY(cudaMemsetAsync(B.cntT, 0, (size_t)(ncell + 1) * sizeof(int), st));
@@ -1408,53 +1264,42 @@ static int tree_velocity_device(ludvm_ctx *ctx, const double *g, const double *x
             ctx->launches++;
         }
         for (int l = L; l >= 2; l--) {
-            if (l == L && P1 <= 24 && !getenv("LUDVM_TREE_UP_SCALAR")) k_tree_up_leaf_mma<<<ncell, 128, 0, st>>>(G, B.startS, B.xs, B.zs, B.gs, B.qhat);
+            if (l == L && P1 <= 24) k_tree_up_leaf_mma<<<ncell, 128, 0, st>>>(G, B.startS, B.xs, B.zs, B.gs, B.qhat);
             else k_tree_up<<<1 << (2 * l), TU_THREADS, 0, st>>>(G, l, B.startS, B.xs, B.zs, B.gs, B.qhat);
             ctx->launches++;
         }
         TreeEval A = {B.startS, B.startT, B.permT, B.keyT, B.xs, B.zs, B.gs, B.qhat, xp, zp, u, w, B.uloc, B.wloc, B.pairs,
-                      fmm ? 1 : 0, (int)np_, gemm ? 1 : 0};
+                      (int)np_};
         cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};
         if (stats) {
             for (int k = 1; k < 3; k++) CUDA_TRY(cudaEventCreate(&ev[k]));
             CUDA_TRY(cudaEventRecord(ev[1], st));
         }
         // passes of <= 512 targets of one leaf are spread over blockIdx.y: enough of it for the most crowded leaf
-        const long items = (long)ncell + (fmm ? level_offset(L + 1) : 0);
+        const long items = (long)ncell + level_offset(L + 1);
         int ysplit = std::max(4, (maxcnt[1] + 4 * TE_THREADS - 1) / (4 * TE_THREADS));
         ysplit = (int)std::max(1L, std::min<long>(ysplit, (1L << 24) / items));
-        if (const char *ye = getenv("LUDVM_TREE_YSPLIT")) ysplit = std::max(1, std::min(64, atoi(ye)));
         k_tree_eval<<<dim3((unsigned)items, ysplit), TE_THREADS, 0, st>>>(G, A);
         ctx->launches++;
-        if (gemm) {
-            CUDA_TRY(cudaMemsetAsync(B.acount, 0, 64 * sizeof(int), st));
-            k_tree_m2l_mats<<<dim3(P2, TM_NOFF, L - 1), 128, 0, st>>>(G, B.Mu, B.Mw);
-            k_tree_alist<<<ceil_div(level_offset(L + 1), 256), 256, 0, st>>>(G, B.startS, B.startT, B.alist, B.acount);
-            long tiles = 0;
-            for (int l = 2; l <= L; l++) tiles += 4 * (((1L << (2 * (l - 1))) + TM_TC - 1) / TM_TC);
-            if (!getenv("LUDVM_TREE_NO_DMMA")) {   // FP64 tensor cores (default); the CUDA-core kernel stays for A/B
-                long td = 0;
-                for (int l = 2; l <= L; l++) td += 4 * (((1L << (2 * (l - 1))) + TD_TC - 1) / TD_TC);
-                k_tree_m2l_dmma<<<dim3((P2 + TD_TI - 1) / TD_TI, (unsigned)td), 256, 0, st>>>(G, B.startS, B.alist, B.acount, B.Mu, B.Mw,
-                                                                                            B.qhat, B.uloc, B.wloc);
-            } else
-            k_tree_m2l_gemm<<<dim3((P2 + TM_TI - 1) / TM_TI, (unsigned)tiles), 256, 0, st>>>(G, B.startS, B.alist, B.acount, B.Mu,
-                                                                                             B.Mw, B.qhat, B.uloc, B.wloc);
-            ctx->launches += 3;
-        }
-        if (fmm) {
-            for (int l = 3; l <= L; l++) {
-                k_tree_l2l<<<1 << (2 * l), 256, 0, st>>>(G, l, B.startS, B.startT, B.uloc, B.wloc);
-                ctx->launches++;
-            }
-            if (P1 <= 4 * L2P_KS && !getenv("LUDVM_TREE_L2P_SCALAR")) k_tree_l2p_mma<<<ncell, 128, 0, st>>>(G, A);
-            else k_tree_l2p<<<ceil_div(np_, 128), 128, 0, st>>>(G, A);
+        CUDA_TRY(cudaMemsetAsync(B.acount, 0, 64 * sizeof(int), st));
+        k_tree_m2l_mats<<<dim3(P2, TM_NOFF, L - 1), 128, 0, st>>>(G, B.Mu, B.Mw);
+        k_tree_alist<<<ceil_div(level_offset(L + 1), 256), 256, 0, st>>>(G, B.startS, B.startT, B.alist, B.acount);
+        long tiles = 0;
+        for (int l = 2; l <= L; l++) tiles += 4 * (((1L << (2 * (l - 1))) + TD_TC - 1) / TD_TC);
+        k_tree_m2l_dmma<<<dim3((P2 + TD_TI - 1) / TD_TI, (unsigned)tiles), 256, 0, st>>>(G, B.startS, B.alist, B.acount, B.Mu, B.Mw,
+                                                                                       B.qhat, B.uloc, B.wloc);
+        ctx->launches += 3;
+        for (int l = 3; l <= L; l++) {
+            k_tree_l2l<<<1 << (2 * l), 256, 0, st>>>(G, l, B.startS, B.startT, B.uloc, B.wloc);
             ctx->launches++;
         }
+        if (P1 <= 4 * L2P_KS) k_tree_l2p_mma<<<ncell, 128, 0, st>>>(G, A);
+        else k_tree_l2p<<<ceil_div(np_, 128), 128, 0, st>>>(G, A);
+        ctx->launches++;
         if (stats) CUDA_TRY(cudaEventRecord(ev[2], st));
         CUDA_TRY(cudaGetLastError());
         ctx->plan[0] = LUDVM_K_TREE; ctx->plan[1] = 4; ctx->plan[2] = L; ctx->plan[3] = 0; ctx->plan[4] = 1;
-        ctx->plan[5] = order; ctx->plan[6] = TE_THREADS / 32; ctx->plan[7] = fmm ? 1 : 0;
+        ctx->plan[5] = order; ctx->plan[6] = TE_THREADS / 32; ctx->plan[7] = 1;
         if (stats) {
             unsigned long long pairs = 0;
             CUDA_TRY(cudaMemcpyAsync(&pairs, B.pairs, sizeof(pairs), cudaMemcpyDeviceToHost, st));

@@ -1,4 +1,4 @@
-"""Device time of the README-size time loop: single-cluster kernel (16 / 8 CTAs), persistent cooperative grid, CUDA-graph replay."""
+"""Device time of the README-size time loop: single-cluster kernel, persistent cooperative grid, CUDA-graph replay."""
 import ctypes as C, json, os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from ludvm_b200 import LUDVM, _lib
@@ -6,14 +6,9 @@ L = _lib.load()
 TF = float(os.environ.get("PROBE_TF", "20"))
 README = dict(t0=0, tf=TF, dt=5e-2, chord=1, rho=1.225, Uinf=1, Npoints=81, Ncoeffs=30, LESPcrit=0.2, Naca="0012")
 NS = int(round(TF / 5e-2))
-GRIDS = [int(a) for a in sys.argv[1:]]   # optional: persistent-grid sizes to try (LUDVM_COOP_GRID); 1000 + w = cluster path up to wake w
-VARIANTS = [("cluster16", {}), ("cluster16 x 512 threads", {"LUDVM_CLUSTER_THREADS": "512"}),
-            ("cluster8", {"LUDVM_CLUSTER_CTAS": "8"}), ("coop", {"LUDVM_NO_CLUSTER": "1"}),
-            ("graph", {"LUDVM_NO_CLUSTER": "1", "LUDVM_NO_COOP": "1"})] + \
-           [("coop%d" % g, {"LUDVM_NO_CLUSTER": "1", "LUDVM_COOP_GRID": str(g)}) for g in GRIDS if g < 1000] + \
-           [("cluster16<=%d" % (g - 1000), {"LUDVM_CLUSTER_MAX_WAKE": str(g - 1000)}) for g in GRIDS if g >= 1000]
+VARIANTS = [("cluster", {}), ("coop", {"LUDVM_NO_CLUSTER": "1"}), ("graph", {"LUDVM_NO_CLUSTER": "1", "LUDVM_NO_COOP": "1"})]
 for label, env in VARIANTS:
-    for k in ("LUDVM_NO_COOP", "LUDVM_COOP_GRID", "LUDVM_NO_CLUSTER", "LUDVM_CLUSTER_CTAS", "LUDVM_CLUSTER_MAX_WAKE", "LUDVM_CLUSTER_THREADS"):
+    for k in ("LUDVM_NO_COOP", "LUDVM_NO_CLUSTER"):
         os.environ.pop(k, None)
     os.environ.update(env)
     for mode in ("exact", "fast"):

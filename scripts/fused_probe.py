@@ -1,5 +1,5 @@
 """Time the fused single-launch self-convection kernel against the partial-sum path (1 GPU):
-N = 2^20 full launch and the 131072-row shard of one rank of eight, source-loop unroll 1/2/4."""
+N = 2^20 full launch and the 131072-row shard of one rank of eight, 16 and 8 source chunks."""
 import os
 import sys
 
@@ -37,16 +37,10 @@ def timed(nrows, reps=3):
 
 dfma = ctx.fp64_fma_rate(300.0)
 print("dfma/s %.4g" % dfma)
-CONFIGS = [{"LUDVM_NO_FUSED": "1"}, {"LUDVM_FUSED_UNROLL": "2"}, {"LUDVM_FUSED_UNROLL": "4"},
-           {"LUDVM_FUSED_WARPS": "16", "LUDVM_FUSED_UNROLL": "2"}, {"LUDVM_FUSED_WARPS": "16", "LUDVM_FUSED_UNROLL": "4"},
-           {"LUDVM_FAST_CHUNKS": "8", "LUDVM_NO_FUSED": "1"}, {"LUDVM_FAST_CHUNKS": "8", "LUDVM_FUSED_UNROLL": "2"},
-           {"LUDVM_FAST_CHUNKS": "8", "LUDVM_FUSED_UNROLL": "4"}]
-if os.environ.get("PROBE_UNROLLS"):
-    CONFIGS = [dict(LUDVM_FUSED_UNROLL=u, **w) for u in os.environ["PROBE_UNROLLS"].split(",")
-               for w in ({}, {"LUDVM_FUSED_WARPS": "16"})]
+CONFIGS = [{}, {"LUDVM_NO_FUSED": "1"}, {"LUDVM_FAST_CHUNKS": "8"}]
 if os.environ.get("PROBE_FUSED_ONLY"):
     CONFIGS = [c for c in CONFIGS if "LUDVM_NO_FUSED" not in c]
-KEYS = ("LUDVM_NO_FUSED", "LUDVM_FUSED_UNROLL", "LUDVM_FUSED_WARPS", "LUDVM_FAST_CHUNKS")
+KEYS = ("LUDVM_NO_FUSED", "LUDVM_FAST_CHUNKS")
 print("lib", _lib.LIB_PATH)
 for nrows in (N, N // 8):
     for env in CONFIGS:

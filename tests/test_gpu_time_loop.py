@@ -269,13 +269,16 @@ def test_propulsive_efficiency_formula():
     assert np.array_equal(s.etap, exp, equal_nan=True) and biteq(s.tt, tt)
 
 
-@pytest.mark.parametrize("drv", ["coop", "graph", "cta"])
+@pytest.mark.parametrize("drv", ["cluster", "coop", "graph", "cta"])
 def test_exact_time_loop_outside_the_range_proof(oracle, drv, monkeypatch):
     """Exact mode skips the per-pair range words while every coordinate stays inside the proof's window
     (SimDev::range_bad).  A free vortex at z = 1e-300 and one at a subnormal x break the proof from step 0: the run
     must fall back to the flagged instantiation (-> library division / square root for tiny operands) and stay
-    bit-equal to the oracle, on the cooperative, the graph and the one-CTA (Ramesh) driver."""
+    bit-equal to the oracle, on the single-cluster, the cooperative, the graph and the one-CTA (Ramesh) driver.  The
+    wake stays below SIM_CLUSTER_MAX_WAKE, so the cooperative and graph cases switch the drivers before them off."""
     from ludvm_b200 import LUDVM
+    if drv in ("coop", "graph"):
+        monkeypatch.setenv("LUDVM_NO_CLUSTER", "1")
     if drv == "graph":
         monkeypatch.setenv("LUDVM_NO_COOP", "1")
     xy = np.array([[-1.0, -2.0, -1e-310, -3.0], [0.3, 1e-300, -0.2, -1e-300]])
