@@ -104,28 +104,24 @@ k_fast32x2_tiled(SrcView S, Tgt T, int nrows, int chunk_len, double *pu, double 
 // memory, Euler update and peer stores in the epilogue (biot_savart.cuh, "fast fused").
 template <int R, int CL, int V, class Tgt>
 __global__ void __launch_bounds__(32 * FW_WARPS, 2)
-k_fast_fused(SrcView S, Tgt T, int nrows, int chunk_len, int nchunks, FusedOut O)
+k_fast_fused(SrcView S, Tgt T, int nrows, int chunk_len, int nchunks, RowOut O)
 {
     extern __shared__ __align__(128) unsigned char fw_raw[];
     fast_fused_block<R, CL, V>(S, T, nrows, chunk_len, nchunks, O, *reinterpret_cast<FwSmem *>(fw_raw));
 }
 
-// Fold partials.  exact: nfold = tree depth d; fast: nfold = number of chunks.  Optional second partial set
-// (the reference's `u_wake + u_foil`, LUDVM.py:1108, :1219) and optional forward-Euler update (LUDVM.py:1108-1127).
+// One set of partial row sums.  exact: nfold = tree depth d; fast: nfold = number of chunks.
+struct Partials {
+    double *u, *w;   // [fold][nrows]; nullptr: no such set
+    int nfold;
+};
+
+// Fold partials, plus an optional second set (the reference's `u_wake + u_foil`, LUDVM.py:1108, :1219).
 struct CombineArgs {
-    const double *pu, *pw;   // [fold][nrows]
-    const double *qu, *qw;   // second set or nullptr
-    int nfold, qfold;
+    Partials p, q;
     int exact;
     int nrows;
-    double *u, *w;           // nullable
-    const double *x, *z;     // Euler: inputs (already offset to the shard's first row)
-    double *xo, *zo;         // Euler: outputs (nullable)
-    double dt;
-    // fused all-gather: the updated rows are also stored into every peer's buffers (NVLink peer stores),
-    // already offset to the shard's first row
-    int npeers;
-    double *xo_peer[LUDVM_MAX_PEERS], *zo_peer[LUDVM_MAX_PEERS];
+    RowOut out;
 };
 
 __global__ void __launch_bounds__(256) k_combine(CombineArgs a)
@@ -134,36 +130,22 @@ __global__ void __launch_bounds__(256) k_combine(CombineArgs a)
     if (row >= a.nrows) return;
     double u, w;
     if (a.exact) {
-        u = exact_combine_row(a.pu, a.nrows, row, a.nfold);
-        w = exact_combine_row(a.pw, a.nrows, row, a.nfold);
-        if (a.qu) {
-            u = __dadd_rn(u, exact_combine_row(a.qu, a.nrows, row, a.qfold));
-            w = __dadd_rn(w, exact_combine_row(a.qw, a.nrows, row, a.qfold));
+        u = exact_combine_row(a.p.u, a.nrows, row, a.p.nfold);
+        w = exact_combine_row(a.p.w, a.nrows, row, a.p.nfold);
+        if (a.q.u) {
+            u = __dadd_rn(u, exact_combine_row(a.q.u, a.nrows, row, a.q.nfold));
+            w = __dadd_rn(w, exact_combine_row(a.q.w, a.nrows, row, a.q.nfold));
         }
     } else {
-        u = fast_combine_row(a.pu, a.nrows, row, a.nfold);
-        w = fast_combine_row(a.pw, a.nrows, row, a.nfold);
-        if (a.qu) {
-            u += fast_combine_row(a.qu, a.nrows, row, a.qfold);
-            w += fast_combine_row(a.qw, a.nrows, row, a.qfold);
+        u = fast_combine_row(a.p.u, a.nrows, row, a.p.nfold);
+        w = fast_combine_row(a.p.w, a.nrows, row, a.p.nfold);
+        if (a.q.u) {
+            u += fast_combine_row(a.q.u, a.nrows, row, a.q.nfold);
+            w += fast_combine_row(a.q.w, a.nrows, row, a.q.nfold);
         }
     }
-    if (a.u) {
-        a.u[row] = u;
-        a.w[row] = w;
-    }
-    if (a.xo || a.npeers) {
-        double xn = __dadd_rn(a.x[row], __dmul_rn(a.dt, u));
-        double zn = __dadd_rn(a.z[row], __dmul_rn(a.dt, w));
-        if (a.xo) {
-            a.xo[row] = xn;
-            a.zo[row] = zn;
-        }
-        for (int p = 0; p < a.npeers; p++) {  // st.global on mapped peer pointers: the all-gather, fused
-            a.xo_peer[p][row] = xn;
-            a.zo_peer[p][row] = zn;
-        }
-    }
+    store_row(a.out, 0, row, u);
+    store_row(a.out, 1, row, w);
 }
 
 // Vorticity stencil, LUDVM.py:1222-1292: clamped neighbours reproduce the centred / one-sided variants.
@@ -232,7 +214,7 @@ static int prove_exact_ranges(ludvm_ctx *ctx, const SrcView &S, const Tgt &T, lo
     *flag = nullptr;
     if (S.vc4 != nullptr || !vc4_in_safe_window(S.vc4s) || S.n0 != S.n || getenv("LUDVM_EXACT_FLAGS")) return LUDVM_OK;
     void *p;
-    int rc = scratch_reserve(ctx, 7, 256, &p);
+    int rc = scratch_reserve(ctx, SLOT_FLAG, 256, &p);
     if (rc) return rc;
     int *bad = (int *)((char *)p + 128);
     CUDA_TRY(cudaMemsetAsync(bad, 0, sizeof(int), ctx->stream));
@@ -250,7 +232,7 @@ static int prove_exact_ranges(ludvm_ctx *ctx, const SrcView &S, const Tgt &T, lo
 
 template <int R, int CL, int V, class Tgt>
 static int launch_fused_inst(ludvm_ctx *ctx, const SrcView &S, const Tgt &T, int nrows, int chunk_len, int nchunks,
-                             const FusedOut &O)
+                             const RowOut &O)
 {
     auto kern = k_fast_fused<R, CL, V, Tgt>;
     static bool configured[16] = {};                       // per device; a function attribute is per device
@@ -282,7 +264,7 @@ static int launch_fused_inst(ludvm_ctx *ctx, const SrcView &S, const Tgt &T, int
 // source chunks (>= 8192 sources) and enough rows for >= ~6 waves of 2 CTAs/SM.  *launched = false: not eligible, the
 // caller takes the partial-sum path.
 template <class Tgt>
-static int try_launch_fused(ludvm_ctx *ctx, int mode, const SrcView &S, const Tgt &T, long nrows, const FusedOut &O,
+static int try_launch_fused(ludvm_ctx *ctx, int mode, const SrcView &S, const Tgt &T, long nrows, const RowOut &O,
                             bool *launched)
 {
     *launched = false;
@@ -318,36 +300,37 @@ static int try_launch_fused(ludvm_ctx *ctx, int mode, const SrcView &S, const Tg
     return LUDVM_OK;
 }
 
-// Evaluate partial row sums for `nrows` targets against S; on return *nfold and the partial buffers (scratch
-// slots slot/slot+1) describe what k_combine must fold.
+// Evaluate partial row sums for `nrows` targets against S into scratch slots slot / slot + 1; *P describes what
+// k_combine must fold.
 template <class Tgt>
-static int launch_partials(ludvm_ctx *ctx, int mode, const SrcView &S, const Tgt &T, long nrows, int slot,
-                           double **pu, double **pw_, int *nfold)
+static int launch_partials(ludvm_ctx *ctx, int mode, const SrcView &S, const Tgt &T, long nrows, int slot, Partials *P)
 {
     const int sm = ctx->sm_count;
+    // both partial buffers, `per_row` values per row
+    auto reserve = [&](size_t per_row, int nfold) -> int {
+        const size_t bytes = sizeof(double) * (size_t)nrows * per_row;
+        void *a, *b;
+        int rc;
+        if ((rc = scratch_reserve(ctx, slot, bytes, &a))) return rc;
+        if ((rc = scratch_reserve(ctx, slot + 1, bytes, &b))) return rc;
+        *P = {(double *)a, (double *)b, nfold};
+        return LUDVM_OK;
+    };
+    int rc;
     if (mode == LUDVM_FAST12_F64) mode = LUDVM_FAST_F64;   // outside the fused kernel: the (more accurate) 13-slot pair
     if (mode == LUDVM_EXACT_F64) {
         const int *bad;
-        {
-            int rc = prove_exact_ranges(ctx, S, T, nrows, &bad);
-            if (rc) return rc;
-        }
+        if ((rc = prove_exact_ranges(ctx, S, T, nrows, &bad))) return rc;
         if (nrows >= 4096 && (S.n >= 1024 || nrows >= (long)sm * ET_THREADS * 3)) {   // (few sources: only if the rows alone fill the GPU)
             // Many rows: one thread per row, sources staged through shared memory; the tree is cut at depth d so
             // that >= ~6 waves of 4 CTAs/SM are in flight.
             long rblocks = (nrows + ET_THREADS - 1) / ET_THREADS;
             int want = ilog2_ceil(std::max(1L, (long)sm * 24 / rblocks));
             int d = std::min(pw_max_depth(S.n), want);
-            size_t bytes = sizeof(double) * (size_t)nrows * ((size_t)1 << d);
-            void *a, *b;
-            int rc;
-            if ((rc = scratch_reserve(ctx, slot, bytes, &a))) return rc;
-            if ((rc = scratch_reserve(ctx, slot + 1, bytes, &b))) return rc;
-            k_exact_tiled<<<dim3((unsigned)rblocks, 1u << d), ET_THREADS, 0, ctx->stream>>>(S, T, (int)nrows, d, (double *)a,
-                                                                                            (double *)b, bad);
+            if ((rc = reserve((size_t)1 << d, d))) return rc;
+            k_exact_tiled<<<dim3((unsigned)rblocks, 1u << d), ET_THREADS, 0, ctx->stream>>>(S, T, (int)nrows, d, P->u, P->w, bad);
             ctx->launches++;
             set_plan(ctx, LUDVM_K_EXACT_TILED, 1, d, 0, 1, bad ? 1 : 0);
-            *pu = (double *)a; *pw_ = (double *)b; *nfold = d;
             return LUDVM_OK;
         }
         // Few rows (or few rows and few sources): 8 lanes per row, tree nodes spread over warps.
@@ -355,17 +338,12 @@ static int launch_partials(ludvm_ctx *ctx, int mode, const SrcView &S, const Tgt
         long nquads = (nrows + 4 * R - 1) / (4 * R);
         int want = ilog2_ceil(std::max(1L, (long)sm * 64 / std::max(1L, nquads)));
         int d = std::min(pw_max_depth(S.n), want);
-        size_t bytes = sizeof(double) * (size_t)nrows * ((size_t)1 << d);
-        void *a, *b;
-        int rc;
-        if ((rc = scratch_reserve(ctx, slot, bytes, &a))) return rc;
-        if ((rc = scratch_reserve(ctx, slot + 1, bytes, &b))) return rc;
+        if ((rc = reserve((size_t)1 << d, d))) return rc;
         long ntasks = nquads << d;
         int blocks = (int)std::min((ntasks + 7) / 8, (long)sm * 16);
-        k_exact_rows<R><<<blocks, 256, 0, ctx->stream>>>(S, T, (int)nrows, d, (double *)a, (double *)b, bad);
+        k_exact_rows<R><<<blocks, 256, 0, ctx->stream>>>(S, T, (int)nrows, d, P->u, P->w, bad);
         ctx->launches++;
         set_plan(ctx, LUDVM_K_EXACT_ROWS, R, d, 0, 1, bad ? 1 : 0);
-        *pu = (double *)a; *pw_ = (double *)b; *nfold = d;
         return LUDVM_OK;
     }
     const bool f32 = (mode == LUDVM_FAST_F32);
@@ -382,61 +360,57 @@ static int launch_partials(ludvm_ctx *ctx, int mode, const SrcView &S, const Tgt
             while (R > 1 && (long)ceil_div(nrows, FT_THREADS * R) * chunks < (long)sm * 2 * 6) R >>= 1;
         }
         int row_blocks = ceil_div(nrows, FT_THREADS * R);
-        size_t bytes = sizeof(double) * (size_t)nrows * (size_t)chunks;
-        void *a, *b;
-        int rc;
-        if ((rc = scratch_reserve(ctx, slot, bytes, &a))) return rc;
-        if ((rc = scratch_reserve(ctx, slot + 1, bytes, &b))) return rc;
+        if ((rc = reserve((size_t)chunks, (int)chunks))) return rc;
         dim3 grid(row_blocks, (unsigned)chunks);
         // one contiguous, 16-byte aligned source segment with a scalar core: TMA-staged tiles
         const bool tma = !f32 && S.vc4 == nullptr && S.gstride == 1 && S.n0 == S.n &&
                          (((uintptr_t)S.x | (uintptr_t)S.z | (uintptr_t)S.g) & 15) == 0;
-        if (f32x2) k_fast32x2_tiled<<<grid, FT_THREADS, 0, ctx->stream>>>(S, T, (int)nrows, chunk_len, (double *)a, (double *)b);
-        else if (f32) k_fast32_tiled<4><<<grid, FT_THREADS, 0, ctx->stream>>>(S, T, (int)nrows, chunk_len, (double *)a, (double *)b);
-        else if (tma && R == 4) k_fast_tiled_tma<4><<<grid, FT_THREADS, 0, ctx->stream>>>(S, T, (int)nrows, chunk_len, (double *)a, (double *)b);
-        else if (tma && R == 2) k_fast_tiled_tma<2><<<grid, FT_THREADS, 0, ctx->stream>>>(S, T, (int)nrows, chunk_len, (double *)a, (double *)b);
-        else if (tma) k_fast_tiled_tma<1><<<grid, FT_THREADS, 0, ctx->stream>>>(S, T, (int)nrows, chunk_len, (double *)a, (double *)b);
-        else if (R == 4) k_fast_tiled<4><<<grid, FT_THREADS, 0, ctx->stream>>>(S, T, (int)nrows, chunk_len, (double *)a, (double *)b);
-        else if (R == 2) k_fast_tiled<2><<<grid, FT_THREADS, 0, ctx->stream>>>(S, T, (int)nrows, chunk_len, (double *)a, (double *)b);
-        else k_fast_tiled<1><<<grid, FT_THREADS, 0, ctx->stream>>>(S, T, (int)nrows, chunk_len, (double *)a, (double *)b);
+        if (f32x2) k_fast32x2_tiled<<<grid, FT_THREADS, 0, ctx->stream>>>(S, T, (int)nrows, chunk_len, P->u, P->w);
+        else if (f32) k_fast32_tiled<4><<<grid, FT_THREADS, 0, ctx->stream>>>(S, T, (int)nrows, chunk_len, P->u, P->w);
+        else if (tma && R == 4) k_fast_tiled_tma<4><<<grid, FT_THREADS, 0, ctx->stream>>>(S, T, (int)nrows, chunk_len, P->u, P->w);
+        else if (tma && R == 2) k_fast_tiled_tma<2><<<grid, FT_THREADS, 0, ctx->stream>>>(S, T, (int)nrows, chunk_len, P->u, P->w);
+        else if (tma) k_fast_tiled_tma<1><<<grid, FT_THREADS, 0, ctx->stream>>>(S, T, (int)nrows, chunk_len, P->u, P->w);
+        else if (R == 4) k_fast_tiled<4><<<grid, FT_THREADS, 0, ctx->stream>>>(S, T, (int)nrows, chunk_len, P->u, P->w);
+        else if (R == 2) k_fast_tiled<2><<<grid, FT_THREADS, 0, ctx->stream>>>(S, T, (int)nrows, chunk_len, P->u, P->w);
+        else k_fast_tiled<1><<<grid, FT_THREADS, 0, ctx->stream>>>(S, T, (int)nrows, chunk_len, P->u, P->w);
         ctx->launches++;
         set_plan(ctx, f32x2 ? LUDVM_K_FAST32X2_TILED : f32 ? LUDVM_K_FAST32_TILED : tma ? LUDVM_K_FAST_TILED_TMA : LUDVM_K_FAST_TILED,
                  R, (int)chunks, tma ? 1 : 0, 1);
-        *pu = (double *)a; *pw_ = (double *)b; *nfold = (int)chunks;
         return LUDVM_OK;
     }
     long nquads = (nrows + 3) / 4;
     long chunks = std::max(1L, std::min((long)sm * 64 / std::max(1L, nquads), ((long)S.n + 63) / 64));
-    size_t bytes = sizeof(double) * (size_t)nrows * (size_t)chunks;
-    void *a, *b;
-    int rc;
-    if ((rc = scratch_reserve(ctx, slot, bytes, &a))) return rc;
-    if ((rc = scratch_reserve(ctx, slot + 1, bytes, &b))) return rc;
+    if ((rc = reserve((size_t)chunks, (int)chunks))) return rc;
     long ntasks = nquads * chunks;
     int blocks = (int)std::min((ntasks + 7) / 8, (long)sm * 16);
-    k_fast_rows<<<blocks, 256, 0, ctx->stream>>>(S, T, (int)nrows, (int)chunks, (double *)a, (double *)b);
+    k_fast_rows<<<blocks, 256, 0, ctx->stream>>>(S, T, (int)nrows, (int)chunks, P->u, P->w);
     ctx->launches++;
     set_plan(ctx, LUDVM_K_FAST_ROWS, 1, (int)chunks, 0, 1);
-    *pu = (double *)a; *pw_ = (double *)b; *nfold = (int)chunks;
     return LUDVM_OK;
 }
 
-static int launch_combine(ludvm_ctx *ctx, const CombineArgs &a)
+// The all-pairs evaluation of every entry point: the row sums of S (plus those of S2, if given) at the `nrows` targets
+// T, stored as O says.  One source set: the fused single launch when eligible.  Otherwise partial sums (S in
+// SLOT_PART_A, S2 in SLOT_PART_B) folded by k_combine.
+template <class Tgt>
+static int eval_rows(ludvm_ctx *ctx, int mode, const SrcView &S, const SrcView *S2, const Tgt &T, long nrows,
+                     const RowOut &O)
 {
-    k_combine<<<ceil_div(a.nrows, 256), 256, 0, ctx->stream>>>(a);
+    int rc;
+    if (!S2) {
+        bool fused;
+        if ((rc = try_launch_fused(ctx, mode, S, T, nrows, O, &fused)) || fused) return rc;
+    }
+    CombineArgs a{};
+    if ((rc = launch_partials(ctx, mode, S, T, nrows, SLOT_PART_A, &a.p))) return rc;
+    if (S2 && (rc = launch_partials(ctx, mode, *S2, T, nrows, SLOT_PART_B, &a.q))) return rc;
+    CUDA_TRY(cudaGetLastError());
+    a.exact = (mode == LUDVM_EXACT_F64);
+    a.nrows = (int)nrows;
+    a.out = O;
+    k_combine<<<ceil_div(nrows, 256), 256, 0, ctx->stream>>>(a);
     ctx->launches++;
     CUDA_TRY(cudaGetLastError());
-    return LUDVM_OK;
-}
-
-// Copy a host array to device scratch (slot) on the context's stream.
-static int stage_in(ludvm_ctx *ctx, int slot, const double *host, size_t n, double **dev)
-{
-    void *p;
-    int rc = scratch_reserve(ctx, slot, std::max<size_t>(n, 1) * sizeof(double), &p);
-    if (rc) return rc;
-    if (n) CUDA_TRY(cudaMemcpyAsync(p, host, n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-    *dev = (double *)p;
     return LUDVM_OK;
 }
 
@@ -447,11 +421,37 @@ static int check_mode(int mode)
     return LUDVM_OK;
 }
 
+// The self-convection step of rows [row0, row0 + nrows) of one cloud.  O holds the velocity outputs, indexed from the
+// first row, and the position outputs, indexed by vortex; the latter are offset to row0 here, and x, z, dt filled in.
+static int selfconv_rows(ludvm_ctx *ctx, int mode, const double *gamma, const double *x, const double *z,
+                         const double *vc4_per_source, double vc4, long n, long row0, long nrows, double dt, RowOut O)
+{
+    ARG_CHECK(ctx != nullptr);
+    int rc = check_mode(mode);
+    if (rc) return rc;
+    ARG_CHECK(n > 0 && n < (1L << 30) && row0 >= 0 && nrows >= 0 && row0 + nrows <= n);
+    ARG_CHECK(gamma && x && z);
+    if (nrows == 0) return LUDVM_OK;
+    DeviceGuard g(ctx->device);
+    O.x = x + row0;
+    O.z = z + row0;
+    O.dt = dt;
+    if (O.xo) {
+        O.xo += row0;
+        O.zo += row0;
+    }
+    for (int p = 0; p < O.npeers; p++) {
+        O.xo_peer[p] += row0;
+        O.zo_peer[p] += row0;
+    }
+    SrcView S = make_src(gamma, 1, x, z, vc4_per_source, vc4, (int)n);
+    return eval_rows(ctx, mode, S, nullptr, TgtArray{x + row0, z + row0}, nrows, O);
+}
+
 }  // namespace ludvm
 
 using namespace ludvm;
 
-// Scratch slot map for the generic entry points: 0,1 partials A; 2,3 partials B; 4 inputs; 5 outputs; 6 grid axes.
 LUDVM_API int ludvm_induced_velocity(ludvm_ctx *ctx, int mode, const double *gamma, long ngamma, const double *xw,
                                      const double *zw, const double *vc4_per_source, double vc4, long nw,
                                      const double *xp, const double *zp, long np_, double *u, double *w, int ptr_kind)
@@ -467,148 +467,52 @@ LUDVM_API int ludvm_induced_velocity(ludvm_ctx *ctx, int mode, const double *gam
     ARG_CHECK(nw == 0 || (gamma && xw && zw));
     DeviceGuard g(ctx->device);
 
+    const bool host = ptr_kind == LUDVM_PTR_HOST;
     const double *dg = gamma, *dxw = xw, *dzw = zw, *dvc = vc4_per_source, *dxp = xp, *dzp = zp;
     double *du = u, *dw = w;
-    if (ptr_kind == LUDVM_PTR_HOST) {
-        // one staging buffer: [g | xw | zw | vc | xp | zp], outputs in slot 5
-        size_t nsrc = (size_t)nw, ntg = (size_t)np_;
-        size_t total = (size_t)ngamma + 2 * nsrc + (vc4_per_source ? nsrc : 0) + 2 * ntg;
-        void *p;
-        if ((rc = scratch_reserve(ctx, 4, (total + 8) * sizeof(double), &p))) return rc;
-        double *b = (double *)p;
-        auto put = [&](const double *h, size_t n, const double **d) -> int {
-            if (n) CUDA_TRY(cudaMemcpyAsync(b, h, n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-            *d = b;
-            b += n;
-            return LUDVM_OK;
-        };
-        if (nw) {
-            if ((rc = put(gamma, (size_t)ngamma, &dg))) return rc;
-            if ((rc = put(xw, nsrc, &dxw))) return rc;
-            if ((rc = put(zw, nsrc, &dzw))) return rc;
-            if (vc4_per_source && (rc = put(vc4_per_source, nsrc, &dvc))) return rc;
-        }
-        if ((rc = put(xp, ntg, &dxp))) return rc;
-        if ((rc = put(zp, ntg, &dzp))) return rc;
-        void *o;
-        if ((rc = scratch_reserve(ctx, 5, 2 * ntg * sizeof(double), &o))) return rc;
-        du = (double *)o;
-        dw = du + ntg;
-    }
+    if (host && ((rc = stage_in(ctx, {{gamma, nw ? ngamma : 0, &dg}, {xw, nw, &dxw}, {zw, nw, &dzw},
+                                      {vc4_per_source, vc4_per_source ? nw : 0, &dvc}, {xp, np_, &dxp}, {zp, np_, &dzp}})) ||
+                 (rc = stage_out(ctx, {{u, np_, &du}, {w, np_, &dw}}))))
+        return rc;
     if (nw == 0) {  // np.sum over an empty axis
         CUDA_TRY(cudaMemsetAsync(du, 0, (size_t)np_ * sizeof(double), ctx->stream));
         CUDA_TRY(cudaMemsetAsync(dw, 0, (size_t)np_ * sizeof(double), ctx->stream));
     } else {
+        RowOut O{};
+        O.u = du;
+        O.w = dw;
         SrcView S = make_src(dg, ngamma == nw ? 1 : 0, dxw, dzw, dvc, vc4, (int)nw);
-        TgtArray T{dxp, dzp};
-        FusedOut fo{};
-        fo.u = du;
-        fo.w = dw;
-        bool fused;
-        if ((rc = try_launch_fused(ctx, mode, S, T, np_, fo, &fused))) return rc;
-        if (!fused) {
-            CombineArgs a{};
-            if ((rc = launch_partials(ctx, mode, S, T, np_, 0, (double **)&a.pu, (double **)&a.pw, &a.nfold))) return rc;
-            CUDA_TRY(cudaGetLastError());
-            a.exact = (mode == LUDVM_EXACT_F64);
-            a.nrows = (int)np_;
-            a.u = du;
-            a.w = dw;
-            if ((rc = launch_combine(ctx, a))) return rc;
-        }
+        if ((rc = eval_rows(ctx, mode, S, nullptr, TgtArray{dxp, dzp}, np_, O))) return rc;
     }
-    if (ptr_kind == LUDVM_PTR_HOST) {
-        CUDA_TRY(cudaMemcpyAsync(u, du, (size_t)np_ * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        CUDA_TRY(cudaMemcpyAsync(w, dw, (size_t)np_ * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    }
-    return LUDVM_OK;
+    return host ? copy_back(ctx, {{u, np_, &du}, {w, np_, &dw}}) : LUDVM_OK;
 }
 
 LUDVM_API int ludvm_selfconv_step(ludvm_ctx *ctx, int mode, const double *gamma, const double *x, const double *z,
                                   const double *vc4_per_source, double vc4, long n, long row0, long nrows, double dt,
                                   double *x_out, double *z_out, double *u_out, double *w_out)
 {
-    ARG_CHECK(ctx != nullptr);
-    int rc = check_mode(mode);
-    if (rc) return rc;
-    ARG_CHECK(n > 0 && n < (1L << 30) && row0 >= 0 && nrows >= 0 && row0 + nrows <= n);
-    ARG_CHECK(gamma && x && z && x_out && z_out);
-    if (nrows == 0) return LUDVM_OK;
-    DeviceGuard g(ctx->device);
-    SrcView S = make_src(gamma, 1, x, z, vc4_per_source, vc4, (int)n);
-    TgtArray T{x + row0, z + row0};
-    {
-        FusedOut fo{};
-        fo.u = u_out;
-        fo.w = w_out;
-        fo.x = x + row0;
-        fo.z = z + row0;
-        fo.xo = x_out + row0;
-        fo.zo = z_out + row0;
-        fo.dt = dt;
-        bool fused;
-        if ((rc = try_launch_fused(ctx, mode, S, T, nrows, fo, &fused))) return rc;
-        if (fused) return LUDVM_OK;
-    }
-    CombineArgs a{};
-    if ((rc = launch_partials(ctx, mode, S, T, nrows, 0, (double **)&a.pu, (double **)&a.pw, &a.nfold))) return rc;
-    CUDA_TRY(cudaGetLastError());
-    a.exact = (mode == LUDVM_EXACT_F64);
-    a.nrows = (int)nrows;
-    a.u = u_out;
-    a.w = w_out;
-    a.x = x + row0;
-    a.z = z + row0;
-    a.xo = x_out + row0;
-    a.zo = z_out + row0;
-    a.dt = dt;
-    return launch_combine(ctx, a);
+    ARG_CHECK(x_out && z_out);
+    RowOut O{};
+    O.u = u_out;
+    O.w = w_out;
+    O.xo = x_out;
+    O.zo = z_out;
+    return selfconv_rows(ctx, mode, gamma, x, z, vc4_per_source, vc4, n, row0, nrows, dt, O);
 }
 
 LUDVM_API int ludvm_selfconv_step_p2p(ludvm_ctx *ctx, int mode, const double *gamma, const double *x, const double *z,
                                       const double *vc4_per_source, double vc4, long n, long row0, long nrows,
                                       double dt, int npeers, double *const *x_out_peers, double *const *z_out_peers)
 {
-    ARG_CHECK(ctx != nullptr);
-    int rc = check_mode(mode);
-    if (rc) return rc;
-    ARG_CHECK(n > 0 && n < (1L << 30) && row0 >= 0 && nrows >= 0 && row0 + nrows <= n);
-    ARG_CHECK(gamma && x && z && x_out_peers && z_out_peers && npeers >= 1 && npeers <= LUDVM_MAX_PEERS);
-    if (nrows == 0) return LUDVM_OK;
-    DeviceGuard g(ctx->device);
-    SrcView S = make_src(gamma, 1, x, z, vc4_per_source, vc4, (int)n);
-    TgtArray T{x + row0, z + row0};
-    for (int p = 0; p < npeers; p++) ARG_CHECK(x_out_peers[p] && z_out_peers[p]);
-    {
-        FusedOut fo{};
-        fo.x = x + row0;
-        fo.z = z + row0;
-        fo.dt = dt;
-        fo.npeers = npeers;
-        for (int p = 0; p < npeers; p++) {
-            fo.xo_peer[p] = x_out_peers[p] + row0;
-            fo.zo_peer[p] = z_out_peers[p] + row0;
-        }
-        bool fused;
-        if ((rc = try_launch_fused(ctx, mode, S, T, nrows, fo, &fused))) return rc;
-        if (fused) return LUDVM_OK;
-    }
-    CombineArgs a{};
-    if ((rc = launch_partials(ctx, mode, S, T, nrows, 0, (double **)&a.pu, (double **)&a.pw, &a.nfold))) return rc;
-    CUDA_TRY(cudaGetLastError());
-    a.exact = (mode == LUDVM_EXACT_F64);
-    a.nrows = (int)nrows;
-    a.x = x + row0;
-    a.z = z + row0;
-    a.dt = dt;
-    a.npeers = npeers;
+    ARG_CHECK(x_out_peers && z_out_peers && npeers >= 1 && npeers <= LUDVM_MAX_PEERS);
+    RowOut O{};
+    O.npeers = npeers;
     for (int p = 0; p < npeers; p++) {
         ARG_CHECK(x_out_peers[p] && z_out_peers[p]);
-        a.xo_peer[p] = x_out_peers[p] + row0;
-        a.zo_peer[p] = z_out_peers[p] + row0;
+        O.xo_peer[p] = x_out_peers[p];
+        O.zo_peer[p] = z_out_peers[p];
     }
-    return launch_combine(ctx, a);
+    return selfconv_rows(ctx, mode, gamma, x, z, vc4_per_source, vc4, n, row0, nrows, dt, O);
 }
 
 LUDVM_API int ludvm_flowfield_velocity(ludvm_ctx *ctx, int mode, const double *ga, const double *xa, const double *za,
@@ -625,57 +529,21 @@ LUDVM_API int ludvm_flowfield_velocity(ludvm_ctx *ctx, int mode, const double *g
     ARG_CHECK(ptr_kind == LUDVM_PTR_HOST || ptr_kind == LUDVM_PTR_DEVICE);
     if (nrows == 0) return LUDVM_OK;
     DeviceGuard g(ctx->device);
-    long npts = nrows * nz;
+    const long npts = nrows * nz;
+    const bool host = ptr_kind == LUDVM_PTR_HOST;
     const double *dga = ga, *dxa = xa, *dza = za, *dgb = gb, *dxb = xb, *dzb = zb, *dx1 = x1, *dz1 = z1;
     double *du = u, *dw = w;
-    if (ptr_kind == LUDVM_PTR_HOST) {
-        size_t total = 3 * (size_t)na + 3 * (size_t)nb + (size_t)nx + (size_t)nz + 8;
-        void *p;
-        if ((rc = scratch_reserve(ctx, 4, total * sizeof(double), &p))) return rc;
-        double *b = (double *)p;
-        auto put = [&](const double *h, size_t n, const double **d) -> int {
-            if (n) CUDA_TRY(cudaMemcpyAsync(b, h, n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-            *d = b;
-            b += n;
-            return LUDVM_OK;
-        };
-        if ((rc = put(ga, na, &dga)) || (rc = put(xa, na, &dxa)) || (rc = put(za, na, &dza))) return rc;
-        if (nb && ((rc = put(gb, nb, &dgb)) || (rc = put(xb, nb, &dxb)) || (rc = put(zb, nb, &dzb)))) return rc;
-        if ((rc = put(x1, nx, &dx1)) || (rc = put(z1, nz, &dz1))) return rc;
-        void *o;
-        if ((rc = scratch_reserve(ctx, 5, 2 * (size_t)npts * sizeof(double), &o))) return rc;
-        du = (double *)o;
-        dw = du + npts;
-    }
-    TgtGrid T{dx1, dz1, (int)nz, (int)row0};
-    SrcView SA = make_src(dga, 1, dxa, dza, nullptr, vc4, (int)na);
-    bool fused = false;
-    if (nb == 0) {   // one source set: the whole sum in one launch when eligible
-        FusedOut fo{};
-        fo.u = du;
-        fo.w = dw;
-        if ((rc = try_launch_fused(ctx, mode, SA, T, npts, fo, &fused))) return rc;
-    }
-    if (!fused) {
-        CombineArgs a{};
-        if ((rc = launch_partials(ctx, mode, SA, T, npts, 0, (double **)&a.pu, (double **)&a.pw, &a.nfold))) return rc;
-        if (nb) {
-            SrcView SB = make_src(dgb, 1, dxb, dzb, nullptr, vc4, (int)nb);
-            if ((rc = launch_partials(ctx, mode, SB, T, npts, 2, (double **)&a.qu, (double **)&a.qw, &a.qfold))) return rc;
-        }
-        CUDA_TRY(cudaGetLastError());
-        a.exact = (mode == LUDVM_EXACT_F64);
-        a.nrows = (int)npts;
-        a.u = du;
-        a.w = dw;
-        if ((rc = launch_combine(ctx, a))) return rc;
-    }
-    if (ptr_kind == LUDVM_PTR_HOST) {
-        CUDA_TRY(cudaMemcpyAsync(u, du, (size_t)npts * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        CUDA_TRY(cudaMemcpyAsync(w, dw, (size_t)npts * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    }
-    return LUDVM_OK;
+    if (host && ((rc = stage_in(ctx, {{ga, na, &dga}, {xa, na, &dxa}, {za, na, &dza}, {gb, nb, &dgb}, {xb, nb, &dxb},
+                                      {zb, nb, &dzb}, {x1, nx, &dx1}, {z1, nz, &dz1}})) ||
+                 (rc = stage_out(ctx, {{u, npts, &du}, {w, npts, &dw}}))))
+        return rc;
+    RowOut O{};
+    O.u = du;
+    O.w = dw;
+    const SrcView SA = make_src(dga, 1, dxa, dza, nullptr, vc4, (int)na);
+    const SrcView SB = make_src(dgb, 1, dxb, dzb, nullptr, vc4, (int)nb);
+    if ((rc = eval_rows(ctx, mode, SA, nb ? &SB : nullptr, TgtGrid{dx1, dz1, (int)nz, (int)row0}, npts, O))) return rc;
+    return host ? copy_back(ctx, {{u, npts, &du}, {w, npts, &dw}}) : LUDVM_OK;
 }
 
 // Velocity and vorticity of one snapshot in one call: with host buffers the fields make one trip (u, w, ome out) instead
@@ -688,46 +556,21 @@ LUDVM_API int ludvm_flowfield(ludvm_ctx *ctx, int mode, const double *ga, const 
     ARG_CHECK(ctx && ome && u && w && x1 && z1);
     ARG_CHECK(ptr_kind == LUDVM_PTR_HOST || ptr_kind == LUDVM_PTR_DEVICE);
     ARG_CHECK(nrows >= 2 && nz >= 2 && row0 >= 0 && row0 + nrows <= nx);
-    if (ptr_kind == LUDVM_PTR_DEVICE) {
-        int rc = ludvm_flowfield_velocity(ctx, mode, ga, xa, za, na, gb, xb, zb, nb, vc4, x1, nx, z1, nz, row0, nrows, u, w,
-                                          ptr_kind);
-        if (rc) return rc;
-        return ludvm_flowfield_vorticity(ctx, x1 + row0, nrows, z1, nz, u, w, 1, ome, ptr_kind);
-    }
     DeviceGuard g(ctx->device);
-    // device-resident u, w, ome and axes in scratch slot 5 / 6; the velocity call stages sources and axes itself (slot 4)
-    const size_t npts = (size_t)nrows * (size_t)nz;
-    void *p, *q;
+    const long npts = nrows * nz;
+    const bool host = ptr_kind == LUDVM_PTR_HOST;
+    const double *dga = ga, *dxa = xa, *dza = za, *dgb = gb, *dxb = xb, *dzb = zb, *dx1 = x1, *dz1 = z1;
+    double *du = u, *dw = w, *dome = ome;
     int rc;
-    if ((rc = scratch_reserve(ctx, 5, 3 * npts * sizeof(double), &p))) return rc;
-    if ((rc = scratch_reserve(ctx, 6, ((size_t)nx + nz + 8) * sizeof(double), &q))) return rc;
-    double *du = (double *)p, *dw = du + npts, *dome = dw + npts, *dx1 = (double *)q, *dz1 = dx1 + nx;
-    CUDA_TRY(cudaMemcpyAsync(dx1, x1, (size_t)nx * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(dz1, z1, (size_t)nz * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-    // sources: staged by a host-pointer call would also download u, w; stage them here and run on device pointers
-    const size_t nsrc = 3 * (size_t)na + 3 * (size_t)nb;
-    void *sp;
-    if ((rc = scratch_reserve(ctx, 4, (nsrc + 8) * sizeof(double), &sp))) return rc;
-    double *b = (double *)sp;
-    const double *hsrc[6] = {ga, xa, za, gb, xb, zb};
-    const double *dsrc[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    for (int k = 0; k < 6; k++) {
-        const size_t n = k < 3 ? (size_t)na : (size_t)nb;
-        if (n == 0) continue;
-        ARG_CHECK(hsrc[k] != nullptr);
-        CUDA_TRY(cudaMemcpyAsync(b, hsrc[k], n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-        dsrc[k] = b;
-        b += n;
-    }
-    if ((rc = ludvm_flowfield_velocity(ctx, mode, dsrc[0], dsrc[1], dsrc[2], na, dsrc[3], dsrc[4], dsrc[5], nb, vc4, dx1, nx,
-                                       dz1, nz, row0, nrows, du, dw, LUDVM_PTR_DEVICE)))
+    if (host && ((rc = stage_in(ctx, {{ga, na, &dga}, {xa, na, &dxa}, {za, na, &dza}, {gb, nb, &dgb}, {xb, nb, &dxb},
+                                      {zb, nb, &dzb}, {x1, nx, &dx1}, {z1, nz, &dz1}})) ||
+                 (rc = stage_out(ctx, {{u, npts, &du}, {w, npts, &dw}, {ome, npts, &dome}}))))
         return rc;
-    if ((rc = ludvm_flowfield_vorticity(ctx, dx1 + row0, nrows, dz1, nz, du, dw, 1, dome, LUDVM_PTR_DEVICE))) return rc;
-    CUDA_TRY(cudaMemcpyAsync(u, du, npts * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(w, dw, npts * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(ome, dome, npts * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    return LUDVM_OK;
+    if ((rc = ludvm_flowfield_velocity(ctx, mode, dga, dxa, dza, na, dgb, dxb, dzb, nb, vc4, dx1, nx, dz1, nz, row0, nrows,
+                                       du, dw, LUDVM_PTR_DEVICE)) ||
+        (rc = ludvm_flowfield_vorticity(ctx, dx1 + row0, nrows, dz1, nz, du, dw, 1, dome, LUDVM_PTR_DEVICE)))
+        return rc;
+    return host ? copy_back(ctx, {{u, npts, &du}, {w, npts, &dw}, {ome, npts, &dome}}) : LUDVM_OK;
 }
 
 LUDVM_API int ludvm_flowfield_vorticity(ludvm_ctx *ctx, const double *x1, long nx, const double *z1, long nz,
@@ -737,35 +580,16 @@ LUDVM_API int ludvm_flowfield_vorticity(ludvm_ctx *ctx, const double *x1, long n
     ARG_CHECK(nx >= 2 && nz >= 2 && ns >= 1);
     ARG_CHECK(ptr_kind == LUDVM_PTR_HOST || ptr_kind == LUDVM_PTR_DEVICE);
     DeviceGuard g(ctx->device);
-    size_t tot = (size_t)ns * nx * nz;
+    const long tot = ns * nx * nz;
+    const bool host = ptr_kind == LUDVM_PTR_HOST;
     const double *dx1 = x1, *dz1 = z1, *du = u, *dw = w;
     double *dome = ome;
     int rc;
-    if (ptr_kind == LUDVM_PTR_HOST) {
-        double *a, *b, *c;
-        if ((rc = stage_in(ctx, 6, x1, nx, &a))) return rc;
-        dx1 = a;
-        void *p;
-        if ((rc = scratch_reserve(ctx, 4, (2 * tot + nz + 8) * sizeof(double), &p))) return rc;
-        b = (double *)p;
-        CUDA_TRY(cudaMemcpyAsync(b, z1, nz * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-        dz1 = b;
-        b += nz;
-        CUDA_TRY(cudaMemcpyAsync(b, u, tot * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-        du = b;
-        b += tot;
-        CUDA_TRY(cudaMemcpyAsync(b, w, tot * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-        dw = b;
-        if ((rc = scratch_reserve(ctx, 5, tot * sizeof(double), &p))) return rc;
-        c = (double *)p;
-        dome = c;
-    }
-    k_vorticity<<<ceil_div((long)tot, 256), 256, 0, ctx->stream>>>(dx1, (int)nx, dz1, (int)nz, du, dw, (int)ns, dome);
+    if (host && ((rc = stage_in(ctx, {{x1, nx, &dx1}, {z1, nz, &dz1}, {u, tot, &du}, {w, tot, &dw}})) ||
+                 (rc = stage_out(ctx, {{ome, tot, &dome}}))))
+        return rc;
+    k_vorticity<<<ceil_div(tot, 256), 256, 0, ctx->stream>>>(dx1, (int)nx, dz1, (int)nz, du, dw, (int)ns, dome);
     ctx->launches++;
     CUDA_TRY(cudaGetLastError());
-    if (ptr_kind == LUDVM_PTR_HOST) {
-        CUDA_TRY(cudaMemcpyAsync(ome, dome, tot * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    }
-    return LUDVM_OK;
+    return host ? copy_back(ctx, {{ome, tot, &dome}}) : LUDVM_OK;
 }

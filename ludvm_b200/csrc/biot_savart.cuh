@@ -696,7 +696,8 @@ struct FwSmem {
     uint64_t full[FW_WARPS][FW_STAGES];
 };
 
-struct FusedOut {
+// Where the finished row sums go, for the fused kernel and k_combine alike.
+struct RowOut {
     double *u, *w;           // velocities (nullable)
     const double *x, *z;     // Euler inputs, already offset to the first row (nullable: no update)
     double *xo, *zo;         // Euler outputs (nullable)
@@ -704,6 +705,21 @@ struct FusedOut {
     int npeers;
     double *xo_peer[LUDVM_MAX_PEERS], *zo_peer[LUDVM_MAX_PEERS];
 };
+
+// Store one finished row sum s of component comp (0: u and x, 1: w and z): the velocity, the forward Euler update
+// (LUDVM.py:1108-1127) and its copies in the peers' buffers (the all-gather, fused: st.global on mapped peer pointers).
+__device__ __forceinline__ void store_row(const RowOut &O, int comp, int row, double s)
+{
+    double *vout = comp ? O.w : O.u;
+    if (vout) vout[row] = s;
+    const double *pin = comp ? O.z : O.x;
+    if (pin) {
+        const double pn = __dadd_rn(pin[row], __dmul_rn(O.dt, s));
+        double *pout = comp ? O.zo : O.xo;
+        if (pout) pout[row] = pn;
+        for (int p = 0; p < O.npeers; p++) (comp ? O.zo_peer[p] : O.xo_peer[p])[row] = pn;
+    }
+}
 
 __device__ __forceinline__ void cluster_sync_all()
 {
@@ -720,7 +736,7 @@ __device__ __forceinline__ const double *cluster_map(const double *p, unsigned r
 
 template <int R, int CL, int V, class Tgt>
 __device__ __forceinline__ void fast_fused_block(const SrcView &S, const Tgt &T, int nrows, int chunk_len, int nchunks,
-                                                 const FusedOut &O, FwSmem &sm)
+                                                 const RowOut &O, FwSmem &sm)
 {
     constexpr int UNROLL = fw_unroll(R);
     constexpr int ROWS = 32 * R;
@@ -808,17 +824,7 @@ __device__ __forceinline__ void fast_fused_block(const SrcView &S, const Tgt &T,
             for (int wq = 0; wq < FW_WARPS; wq++)
                 if (q * FW_WARPS + wq < nchunks) s += p[wq * (sizeof(FwWarpStage) * FW_STAGES / sizeof(double))];
         }
-        if (row < nrows) {
-            double *vout = comp ? O.w : O.u;
-            if (vout) vout[row] = s;
-            const double *pin = comp ? O.z : O.x;
-            if (pin) {
-                const double pn = __dadd_rn(pin[row], __dmul_rn(O.dt, s));
-                double *pout = comp ? O.zo : O.xo;
-                if (pout) pout[row] = pn;
-                for (int p = 0; p < O.npeers; p++) (comp ? O.zo_peer[p] : O.xo_peer[p])[row] = pn;   // fused all-gather
-            }
-        }
+        if (row < nrows) store_row(O, comp, row, s);
     }
     if (CL > 1) cluster_sync_all();                     // nobody leaves while a peer still reads its shared memory
 }

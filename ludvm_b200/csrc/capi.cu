@@ -36,24 +36,45 @@ int scratch_reserve(ludvm_ctx *ctx, int slot, size_t bytes, void **out)
     return LUDVM_OK;
 }
 
-int pinned_reserve(ludvm_ctx *ctx, size_t bytes, void **out)
+int stage_in(ludvm_ctx *ctx, std::initializer_list<HostIn> in)
 {
-    Scratch &s = ctx->pinned;
-    if (s.bytes < bytes) {
-        if (s.ptr) {
-            CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-            CUDA_TRY(cudaFreeHost(s.ptr));
-            s.ptr = nullptr;
-            s.bytes = 0;
-        }
-        cudaError_t e = cudaMallocHost(&s.ptr, bytes);
-        if (e != cudaSuccess) {
-            cudaGetLastError();
-            return set_error(LUDVM_E_NOMEM, "cudaMallocHost(%zu) failed: %s", bytes, cudaGetErrorString(e));
-        }
-        s.bytes = bytes;
+    size_t total = 0;
+    for (const HostIn &a : in) {
+        ARG_CHECK(a.n >= 0 && (a.n == 0 || a.host != nullptr));
+        total += (size_t)a.n;
     }
-    *out = s.ptr;
+    void *p;
+    int rc = scratch_reserve(ctx, SLOT_IN, total * sizeof(double), &p);
+    if (rc) return rc;
+    double *b = (double *)p;
+    for (const HostIn &a : in) {
+        *a.dev = a.n ? b : nullptr;
+        if (a.n) CUDA_TRY(cudaMemcpyAsync(b, a.host, (size_t)a.n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+        b += a.n;
+    }
+    return LUDVM_OK;
+}
+
+int stage_out(ludvm_ctx *ctx, std::initializer_list<HostOut> out)
+{
+    size_t total = 0;
+    for (const HostOut &a : out) total += (size_t)a.n;
+    void *p;
+    int rc = scratch_reserve(ctx, SLOT_OUT, total * sizeof(double), &p);
+    if (rc) return rc;
+    double *b = (double *)p;
+    for (const HostOut &a : out) {
+        *a.dev = b;
+        b += a.n;
+    }
+    return LUDVM_OK;
+}
+
+int copy_back(ludvm_ctx *ctx, std::initializer_list<HostOut> out)
+{
+    for (const HostOut &a : out)
+        if (a.n) CUDA_TRY(cudaMemcpyAsync(a.host, *a.dev, (size_t)a.n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     return LUDVM_OK;
 }
 
@@ -80,7 +101,7 @@ static int measure_rate(ludvm_ctx *ctx, double ms_target, double *rate)
     DeviceGuard g(ctx->device);
     T *dummy;
     void *p;
-    int rc = scratch_reserve(ctx, 7, 256, &p);
+    int rc = scratch_reserve(ctx, SLOT_FLAG, 256, &p);
     if (rc) return rc;
     dummy = (T *)p;
     cudaEvent_t e0, e1;
@@ -168,7 +189,6 @@ LUDVM_API int ludvm_ctx_destroy(ludvm_ctx *ctx)
     cudaStreamSynchronize(ctx->stream);
     for (auto &s : ctx->dev)
         if (s.ptr) cudaFree(s.ptr);
-    if (ctx->pinned.ptr) cudaFreeHost(ctx->pinned.ptr);
     if (ctx->own_stream) cudaStreamDestroy(ctx->stream);
     delete ctx;
     return LUDVM_OK;

@@ -1586,20 +1586,6 @@ __global__ void __launch_bounds__(256) k_sweep_gather(const SimDev *cases, int n
     }
 }
 
-// Bump allocator over one device arena; with base == nullptr it only measures.
-struct Arena {
-    char *base = nullptr;
-    size_t off = 0;
-    template <typename T>
-    T *take(size_t n)
-    {
-        off = (off + 255) & ~(size_t)255;
-        T *p = base ? (T *)(base + off) : nullptr;
-        off += std::max<size_t>(n, 1) * sizeof(T);
-        return p;
-    }
-};
-
 struct DevTables {  // device copies of one ludvm_sim_tables
     const double *cos_a, *sin_a, *alpha_dot, *h_dot, *gp, *le, *te;
     const double *detadx_p, *eta_p, *x_p, *theta_p, *dtheta, *cos_tp, *sin_tp, *cosn, *sinn, *free_g, *free_xz;
@@ -2201,30 +2187,6 @@ LUDVM_API int ludvm_sim_field_bytes(ludvm_sim *s, int field, size_t *out)
     return field_info(s, field, &p, out);
 }
 
-LUDVM_API int ludvm_sim_fetch(ludvm_sim *s, int field, void *dst, size_t bytes)
-{
-    ARG_CHECK(s && dst);
-    DeviceGuard g(s->ctx->device);
-    const void *p;
-    size_t want;
-    int rc = field_info(s, field, &p, &want);
-    if (rc) return rc;
-    if (bytes != want) return set_error(LUDVM_E_ARG, "field %d holds %zu bytes, caller passed %zu", field, want, bytes);
-    cudaStream_t st = s->ctx->stream;
-    if (field == LUDVM_F_CUR_TEV || field == LUDVM_F_CUR_LEV || field == LUDVM_F_CUR_FREE) {
-        const SimDev &D = s->d;
-        size_t off = field == LUDVM_F_CUR_TEV ? 0 : (field == LUDVM_F_CUR_LEV ? D.nv : 2 * (size_t)D.nv);
-        size_t n = field == LUDVM_F_CUR_FREE ? D.nfree : D.nv;
-        CUDA_TRY(cudaMemcpyAsync(dst, D.wx + off, n * sizeof(double), cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaMemcpyAsync((double *)dst + n, D.wz + off, n * sizeof(double), cudaMemcpyDeviceToHost, st));
-    } else {
-        if (!p) return set_error(LUDVM_E_STATE, "field %d was not kept (store_history = 0)", field);
-        CUDA_TRY(cudaMemcpyAsync(dst, p, bytes, cudaMemcpyDeviceToHost, st));
-    }
-    CUDA_TRY(cudaStreamSynchronize(st));
-    return LUDVM_OK;
-}
-
 // Several result fields in one call: every copy is enqueued, then ONE synchronisation (a run's results are ~25 fields;
 // fetching them one by one costs a stream synchronisation each).
 LUDVM_API int ludvm_sim_fetch_many(ludvm_sim *s, int nfields, const int *fields, void *const *dsts, const size_t *bytes)
@@ -2253,6 +2215,11 @@ LUDVM_API int ludvm_sim_fetch_many(ludvm_sim *s, int nfields, const int *fields,
     }
     CUDA_TRY(cudaStreamSynchronize(st));
     return LUDVM_OK;
+}
+
+LUDVM_API int ludvm_sim_fetch(ludvm_sim *s, int field, void *dst, size_t bytes)
+{
+    return ludvm_sim_fetch_many(s, 1, &field, &dst, &bytes);
 }
 
 LUDVM_API int ludvm_sim_destroy(ludvm_sim *s)

@@ -1116,17 +1116,6 @@ __global__ void __launch_bounds__(256) k_tree_euler(const double *x, const doubl
 // ---------------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------------
-struct Arena {
-    char *base;
-    size_t off = 0;
-    template <class T> T *take(size_t n)
-    {
-        T *p = base ? (T *)(base + off) : nullptr;
-        off += (n * sizeof(T) + 255) & ~(size_t)255;
-        return p;
-    }
-};
-
 struct TreeBufs {
     int *keyS, *slotS, *keyT, *slotT, *cntS, *cntT, *startS, *startT, *tmpS, *permS, *tmpT, *permT;
     double *xs, *zs, *gs, *qhat, *uloc, *wloc;
@@ -1169,7 +1158,7 @@ static int tree_velocity_device(ludvm_ctx *ctx, const double *g, const double *x
     cudaStream_t st = ctx->stream;
     void *p;
     int rc;
-    if ((rc = scratch_reserve(ctx, 9, 256, &p))) return rc;
+    if ((rc = scratch_reserve(ctx, SLOT_TREE_COUNTERS, 256, &p))) return rc;
     unsigned long long *mm = (unsigned long long *)p;
     {
         unsigned long long init[8] = {~0ull, 0, ~0ull, 0, ~0ull, 0, ~0ull, 0};
@@ -1215,10 +1204,10 @@ static int tree_velocity_device(ludvm_ctx *ctx, const double *g, const double *x
         if ((order & 1) == 0) G.s[order / 2] = 0.0;
         for (int k = 0; k < P1 / 2; k++) G.s[order - k] = -G.s[k];
 
-        Arena sizer{nullptr};
+        Arena sizer;
         TreeBufs B;
         const size_t bytes = tree_layout(sizer, B, nw, np_, L, P2);
-        if ((rc = scratch_reserve(ctx, 8, bytes, &p))) return rc;
+        if ((rc = scratch_reserve(ctx, SLOT_TREE_ARENA, bytes, &p))) return rc;
         Arena ar{(char *)p};
         tree_layout(ar, B, nw, np_, L, P2);
         const int ncell = 1 << (2 * L);
@@ -1334,26 +1323,12 @@ LUDVM_API int ludvm_induced_velocity_tree(ludvm_ctx *ctx, const double *gamma, c
     ARG_CHECK(nw == 0 || (gamma && xw && zw));
     DeviceGuard g(ctx->device);
     int rc;
+    const bool host = ptr_kind == LUDVM_PTR_HOST;
     const double *dg = gamma, *dxw = xw, *dzw = zw, *dxp = xp, *dzp = zp;
     double *du = u, *dw = w;
-    if (ptr_kind == LUDVM_PTR_HOST) {
-        const size_t total = 3 * (size_t)nw + 2 * (size_t)np_;
-        void *p;
-        if ((rc = scratch_reserve(ctx, 4, (total + 8) * sizeof(double), &p))) return rc;
-        double *b = (double *)p;
-        const double *h[5] = {gamma, xw, zw, xp, zp};
-        const double **d[5] = {&dg, &dxw, &dzw, &dxp, &dzp};
-        for (int k = 0; k < 5; k++) {
-            const size_t n = k < 3 ? (size_t)nw : (size_t)np_;
-            if (n) CUDA_TRY(cudaMemcpyAsync(b, h[k], n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-            *d[k] = b;
-            b += n;
-        }
-        void *o;
-        if ((rc = scratch_reserve(ctx, 5, 2 * (size_t)np_ * sizeof(double), &o))) return rc;
-        du = (double *)o;
-        dw = du + np_;
-    }
+    if (host && ((rc = stage_in(ctx, {{gamma, nw, &dg}, {xw, nw, &dxw}, {zw, nw, &dzw}, {xp, np_, &dxp}, {zp, np_, &dzp}})) ||
+                 (rc = stage_out(ctx, {{u, np_, &du}, {w, np_, &dw}}))))
+        return rc;
     if (nw == 0) {
         CUDA_TRY(cudaMemsetAsync(du, 0, (size_t)np_ * sizeof(double), ctx->stream));
         CUDA_TRY(cudaMemsetAsync(dw, 0, (size_t)np_ * sizeof(double), ctx->stream));
@@ -1361,12 +1336,7 @@ LUDVM_API int ludvm_induced_velocity_tree(ludvm_ctx *ctx, const double *gamma, c
     } else if ((rc = tree_velocity_device(ctx, dg, dxw, dzw, vc4, nw, dxp, dzp, np_, order, leaf, du, dw, stats))) {
         return rc;
     }
-    if (ptr_kind == LUDVM_PTR_HOST) {
-        CUDA_TRY(cudaMemcpyAsync(u, du, (size_t)np_ * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        CUDA_TRY(cudaMemcpyAsync(w, dw, (size_t)np_ * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    }
-    return LUDVM_OK;
+    return host ? copy_back(ctx, {{u, np_, &du}, {w, np_, &dw}}) : LUDVM_OK;
 }
 
 LUDVM_API int ludvm_selfconv_step_tree(ludvm_ctx *ctx, const double *gamma, const double *x, const double *z, double vc4, long n,
@@ -1382,7 +1352,7 @@ LUDVM_API int ludvm_selfconv_step_tree(ludvm_ctx *ctx, const double *gamma, cons
     double *du = u_out, *dw = w_out;
     if (!du || !dw) {
         void *o;
-        if ((rc = scratch_reserve(ctx, 5, 2 * (size_t)nrows * sizeof(double), &o))) return rc;
+        if ((rc = scratch_reserve(ctx, SLOT_OUT, 2 * (size_t)nrows * sizeof(double), &o))) return rc;
         du = (double *)o;
         dw = du + nrows;
     }
@@ -1424,36 +1394,18 @@ LUDVM_API int ludvm_flowfield_velocity_tree(ludvm_ctx *ctx, const double *ga, co
     DeviceGuard g(ctx->device);
     const long npts = nrows * nz;
     int rc;
+    const bool host = ptr_kind == LUDVM_PTR_HOST;
     const double *dga = ga, *dxa = xa, *dza = za, *dx1 = x1, *dz1 = z1;
     double *du = u, *dw = w;
-    if (ptr_kind == LUDVM_PTR_HOST) {
-        void *p;
-        if ((rc = scratch_reserve(ctx, 4, (3 * (size_t)na + (size_t)nx + (size_t)nz + 8) * sizeof(double), &p))) return rc;
-        double *b = (double *)p;
-        const double *h[5] = {ga, xa, za, x1, z1};
-        const double **d[5] = {&dga, &dxa, &dza, &dx1, &dz1};
-        const size_t n[5] = {(size_t)na, (size_t)na, (size_t)na, (size_t)nx, (size_t)nz};
-        for (int k = 0; k < 5; k++) {
-            CUDA_TRY(cudaMemcpyAsync(b, h[k], n[k] * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-            *d[k] = b;
-            b += n[k];
-        }
-        void *o;
-        if ((rc = scratch_reserve(ctx, 5, 2 * (size_t)npts * sizeof(double), &o))) return rc;
-        du = (double *)o;
-        dw = du + npts;
-    }
+    if (host && ((rc = stage_in(ctx, {{ga, na, &dga}, {xa, na, &dxa}, {za, na, &dza}, {x1, nx, &dx1}, {z1, nz, &dz1}})) ||
+                 (rc = stage_out(ctx, {{u, npts, &du}, {w, npts, &dw}}))))
+        return rc;
     void *tp;
-    if ((rc = scratch_reserve(ctx, 6, (2 * (size_t)npts + 4) * sizeof(double), &tp))) return rc;
+    if ((rc = scratch_reserve(ctx, SLOT_TREE_GRID, (2 * (size_t)npts + 4) * sizeof(double), &tp))) return rc;
     double *xp = (double *)tp, *zp = xp + npts, *box = zp + npts;
     k_tree_grid_points<<<ceil_div(npts, 256), 256, 0, ctx->stream>>>(dx1, (int)nx, dz1, (int)nz, (int)row0, npts, xp, zp, box);
     ctx->launches++;
     if ((rc = tree_velocity_device(ctx, dga, dxa, dza, vc4, na, xp, zp, npts, order, leaf, du, dw, stats, tgt_density, box, box + 2, 2)))
         return rc;
-    if (ptr_kind == LUDVM_PTR_HOST) {
-        CUDA_TRY(cudaMemcpyAsync(u, du, (size_t)npts * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        CUDA_TRY(cudaMemcpyAsync(w, dw, (size_t)npts * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    }
-    return LUDVM_OK;
+    return host ? copy_back(ctx, {{u, npts, &du}, {w, npts, &dw}}) : LUDVM_OK;
 }

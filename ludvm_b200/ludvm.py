@@ -365,11 +365,6 @@ class LUDVM:
                 ilev += 1
         return BC
 
-    def _fetch(self, field, shape, dtype=np.float64):
-        a = np.empty(shape, dtype=dtype)
-        check(load().ludvm_sim_fetch(self._sim, FIELDS[field], a.ctypes.data, a.nbytes))
-        return a
-
     def _fetch_results(self, nt, P, Nc, nf, nv):
         # every result field in ONE C call (one stream synchronisation instead of one per field)
         want = [('G_TEV', nv), ('G_LEV', nv), ('G_BOUND', nv), ('G_AIRFOIL', (nv, P)), ('GAMMA_AIRFOIL', (nv, P)),
