@@ -212,6 +212,13 @@ int ludvm_sim_steps_done(ludvm_sim *sim, long *out);
  * with CUDA events around each.  ms_out[0..3] = summed milliseconds of wake-on-foil, solve, convection partials,
  * finish; ms_out[4] = their total.  Synchronises. */
 int ludvm_sim_profile_steps(ludvm_sim *sim, long nsteps, double *ms_out);
+/* Opt in to the chordwise pressure jump LUDVM_F_DP, which the reference allocates but never fills (LUDVM.py:1059-1064).
+ * For step i >= 1 and gamma point j, with itev = i - 1:
+ *   dp[i,j] = rho ((Uinf cos a_i + hdot_i sin a_i + u_j) gamma_airfoil[itev,j] + (Gamma_airfoil[itev,j] - Gamma_airfoil[itev-1,j]) / dt)
+ * u_j = the tangential wake velocity at gamma point j that the loads integrate (LUDVM.py:1049-1057), Gamma_airfoil[-1] = 0;
+ * row 0 and the rows of steps not yet run are zero.  Allocates and zeroes [nt,P] doubles.  Valid only before the first step
+ * is run (LUDVM_E_STATE after); a second call does nothing. */
+int ludvm_sim_enable_pressure(ludvm_sim *sim);
 
 enum {
     LUDVM_F_PATH_TEV = 0,  /* [(nt-1)/k+1,2,nt-1]  needs store_history = k >= 1  LUDVM.py:615 */
@@ -235,7 +242,8 @@ enum {
     LUDVM_F_RANGE_BAD = 23, /* int32[1], exact mode: 0 = every coordinate seen so far lay inside the window in which the
                                pair arithmetic needs no per-pair range words (the flag-free instantiation ran), 1 = the
                                flagged instantiation took over (sticky) */
-    LUDVM_F__COUNT = 24
+    LUDVM_F_DP = 24,       /* [nt,P] pressure jump; LUDVM_E_STATE unless ludvm_sim_enable_pressure was called */
+    LUDVM_F__COUNT = 25
 };
 /* Copy a result field to a host buffer of `bytes` bytes (must equal the field's size).  Synchronises. */
 int ludvm_sim_fetch(ludvm_sim *sim, int field, void *dst, size_t bytes);

@@ -43,7 +43,7 @@ class SimTables(C.Structure):
 
 FIELDS = dict(PATH_TEV=0, PATH_LEV=1, PATH_FREE=2, G_TEV=3, G_LEV=4, G_BOUND=5, G_AIRFOIL=6, GAMMA_AIRFOIL=7,
               GAMMA_INT_AIRFOIL=8, FOURIER=9, LESP=10, LESP_PREV=11, LEV_SHED=12, FN=13, FS=14, L=15, D=16, T=17,
-              M=18, CUR_TEV=19, CUR_LEV=20, CUR_FREE=21, COUNTERS=22, RANGE_BAD=23)
+              M=18, CUR_TEV=19, CUR_LEV=20, CUR_FREE=21, COUNTERS=22, RANGE_BAD=23, DP=24)
 
 # name -> (restype, argtypes); every symbol include/ludvm_b200.h declares
 SIGNATURES = {
@@ -77,6 +77,7 @@ SIGNATURES = {
     "ludvm_sim_run": (C.c_int, [c_vp, C.c_long]),
     "ludvm_sim_steps_done": (C.c_int, [c_vp, C.POINTER(C.c_long)]),
     "ludvm_sim_profile_steps": (C.c_int, [c_vp, C.c_long, c_dp]),
+    "ludvm_sim_enable_pressure": (C.c_int, [c_vp]),
     "ludvm_sim_fetch": (C.c_int, [c_vp, C.c_int, c_vp, C.c_size_t]),
     "ludvm_sim_fetch_many": (C.c_int, [c_vp, C.c_int, C.POINTER(C.c_int), C.POINTER(c_vp), C.POINTER(C.c_size_t)]),
     "ludvm_sim_field_bytes": (C.c_int, [c_vp, C.c_int, C.POINTER(C.c_size_t)]),

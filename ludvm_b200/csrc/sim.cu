@@ -80,6 +80,7 @@ struct SimDev {
     double *g_bound, *g_airfoil, *gamma_airfoil, *Gamma_airfoil, *fourier, *lesp, *lesp_prev, *lev_shed;
     double *Fn, *Fs, *L, *D, *T, *M;
     double *path_tev, *path_lev, *path_free;  // nullable
+    double *dp;           // nullable: chordwise pressure jump [nt,P] (ludvm_sim_enable_pressure)
     // step bookkeeping
     long long *counters;  // [0] steps done, [1] itev of the last step, [2] ilev of the last step, [3] error flags
     int *ilev_arr;        // [nt+1]: ilev at the start of step i
@@ -708,14 +709,38 @@ __device__ void phase_solve(const SimDev &S, const Step &st, double *tab, double
     TRACE(10);
 }
 
-// Gamma_j = np.sum(dGamma[:j+1]) (LUDVM.py:1008-1010); nothing in the step consumes it, so it runs beside the loads.
+// Gamma_j = np.sum(dGamma[:j+1]) (LUDVM.py:1008-1010) of one row of dGamma
+__device__ __forceinline__ double gamma_cum_at(const double *dG, int j)
+{
+    auto f = [&](int kk) { return dG[kk]; };
+    return 0.0 + pw_seq(f, 0, j + 1);
+}
+
+// Nothing in the step consumes Gamma, so it runs beside the loads.
 __device__ __forceinline__ void phase_gamma_cumsum(const SimDev &S, const Step &st, int t0, int nthreads)
 {
     const double *dG = S.g_airfoil + (size_t)st.itev * S.af_stride;
     double *out = S.Gamma_airfoil + (size_t)st.itev * S.af_stride;
-    for (int j = t0; j < S.P; j += nthreads) {
-        auto f = [&](int kk) { return dG[kk]; };
-        out[j] = 0.0 + pw_seq(f, 0, j + 1);
+    for (int j = t0; j < S.P; j += nthreads) out[j] = gamma_cum_at(dG, j);
+}
+
+// Pressure jump of step i, the array the reference allocates but never fills (LUDVM.py:1059-1064):
+//   dp[i,j] = rho ((Uinf cos a + hdot sin a + u_j) gamma[itev,j] + (Gamma[itev,j] - Gamma[itev-1,j]) / dt)
+// u_j = the loads' tangential wake velocity at gamma point j, which phase_finish_loads left in dp[i,j] (same thread, same
+// j).  Gamma row itev is summed by another CTA while the loads run (or after them, in the one-CTA driver), so it is formed
+// again here with the same expression; row itev - 1 is complete.  Called after the loads, where little else is live
+// (inside the loads' loop, or out of line, it cost the kernels around it spills); on the graph path it is a kernel of its
+// own after k_finish / k_finish_ov (k_pressure), which keep their register allocation.
+__device__ __forceinline__ void pressure_row(const SimDev &S, const Step &st)
+{
+    const int i = st.i, itev = st.itev;
+    const double vrel = S.Uinf * S.cos_a[i] + S.h_dot[i] * S.sin_a[i];
+    const double *gam = S.gamma_airfoil + (size_t)itev * S.af_stride, *dG = S.g_airfoil + (size_t)itev * S.af_stride;
+    const double *Gprev = S.Gamma_airfoil + (size_t)(itev - 1) * S.af_stride;
+    double *row = S.dp + (size_t)i * S.P;
+    for (int j = threadIdx.x; j < S.P; j += blockDim.x) {
+        const double u = row[j], G = gamma_cum_at(dG, j), Gp = itev >= 1 ? Gprev[j] : 0.0;
+        row[j] = S.rho * ((vrel + u) * gam[j] + (G - Gp) / S.dt);
     }
 }
 
@@ -768,6 +793,9 @@ __device__ __forceinline__ int conv_fold(const SimDev &S, const Step &st, int ti
 
 // `tab` = shared memory of resident StepTables, or nullptr: then the three tables needed here are built in `sm`.
 // `ov`: the wake velocity at the gamma points was already assembled in S.gp_u / S.gp_w (overlapped step).
+// DP: the driver can carry the pressure jump (S.dp non-null): u is left in the dp row for pressure_row; the sweep
+// drivers cannot, and compile without it.
+template <bool DP>
 __device__ void phase_finish_loads(const SimDev &S, const Step &st, double *tab, double *sm, int tiled_chunks, int cap,
                                    bool ov = false)  // LUDVM.py:1035-1090
 {
@@ -803,6 +831,7 @@ __device__ void phase_finish_loads(const SimDev &S, const Step &st, double *tab,
     for (int j = tid; j < P; j += nth) {
         double u1 = ug[j], w1 = ugx[j];
         double u = u1 * ca - w1 * sa;
+        if (DP && S.dp) S.dp[(size_t)i * P + j] = u;   // pressure_row's input
         ug[j] = u * gam[j];
         ugx[j] = u * gam[j] * xp[j];
     }
@@ -1105,7 +1134,7 @@ __global__ void __launch_bounds__(256) k_finish_ov(SimDev S, int s, int R, int s
     Step st;
     if (!step_begin(S, s, st)) return;
     if (blockIdx.x == 0) {
-        phase_finish_loads(S, st, nullptr, sm, 1, FINISH_STAGE, true);
+        phase_finish_loads<true>(S, st, nullptr, sm, 1, FINISH_STAGE, true);
         return;
     }
     if (blockIdx.x == 1) {
@@ -1155,7 +1184,7 @@ __global__ void __launch_bounds__(256) k_finish(SimDev S, int s, int tiled_chunk
     Step st;
     if (!step_begin(S, s, st)) return;
     if (blockIdx.x == 0) {
-        phase_finish_loads(S, st, nullptr, sm, tiled_chunks, FINISH_STAGE);
+        phase_finish_loads<true>(S, st, nullptr, sm, tiled_chunks, FINISH_STAGE);
         return;
     }
     if (blockIdx.x == 1) {
@@ -1164,6 +1193,14 @@ __global__ void __launch_bounds__(256) k_finish(SimDev S, int s, int tiled_chunk
     }
     phase_finish_update(S, st, (long)(blockIdx.x - 2) * blockDim.x + threadIdx.x, (long)(gridDim.x - 2) * blockDim.x,
                         tiled_chunks);
+}
+
+// Graph path with the pressure jump enabled: row i of dp after k_finish / k_finish_ov (one CTA).
+__global__ void __launch_bounds__(256) k_pressure(SimDev S, int s)
+{
+    Step st;
+    if (!step_begin(S, s, st)) return;
+    pressure_row(S, st);
 }
 
 __global__ void k_advance(SimDev S, int k)
@@ -1260,8 +1297,10 @@ __global__ void __launch_bounds__(256, 1) k_sim_persist(SimDev S, int nsteps, un
 #endif
     auto deferred_tail = [&](int ip) {
         Step sp{ip, ip - 1, ((volatile int *)S.ilev_arr)[ip]};
-        if (blockIdx.x == 1) phase_finish_loads(S, sp, tab, scr, 0, S.sum_nodes);
-        else if (blockIdx.x == 2) phase_gamma_cumsum(S, sp, threadIdx.x, blockDim.x);
+        if (blockIdx.x == 1) {
+            phase_finish_loads<true>(S, sp, tab, scr, 0, S.sum_nodes);
+            if (S.dp) pressure_row(S, sp);
+        } else if (blockIdx.x == 2) phase_gamma_cumsum(S, sp, threadIdx.x, blockDim.x);
     };
     for (int i = first; i <= last; i++) {
         Step st{i, i - 1, ((volatile int *)S.ilev_arr)[i]};
@@ -1531,7 +1570,8 @@ __global__ void __launch_bounds__(THREADS, THREADS <= 128 ? 6 : (THREADS <= 256 
                 cta_conv_partials(S, st);
             __syncthreads();
             CTA_T(2);
-            phase_finish_loads(S, st, tab, scr, 0, S.sum_nodes);
+            phase_finish_loads<THREADS == RAMESH_THREADS>(S, st, tab, scr, 0, S.sum_nodes);   // single-simulation Ramesh runs only
+            if (THREADS == RAMESH_THREADS && S.dp) pressure_row(S, st);
             CTA_T(3);
             cta_finish_update(S, st);
             phase_gamma_cumsum(S, st, threadIdx.x, blockDim.x);
@@ -1663,6 +1703,7 @@ static void layout_case(SimDev &D, const ludvm_sim_params &p, const DevTables &t
     } else {
         D.path_tev = D.path_lev = D.path_free = nullptr;
     }
+    D.dp = nullptr;   // ludvm_sim_enable_pressure
     D.counters = a.take<long long>(4);
     D.ilev_arr = a.take<int>(nt + 2);
     D.lespcrit_cur = a.take<double>(1);
@@ -1848,7 +1889,8 @@ static StepPlan plan_step(const ludvm_sim *s, int bracket)
 }
 
 // Enqueue kernel `which` of step offset k: 0 wake-on-foil, 1 solve, 2 convection partials, 3 finish; for the overlapped
-// step 2 = old-wake convection (independent of 0 and 1), 4 = the new-vortex / bound-vortex terms, 3 = finish.
+// step 2 = old-wake convection (independent of 0 and 1), 4 = the new-vortex / bound-vortex terms, 3 = finish.  With the
+// pressure jump enabled, 3 is followed by k_pressure.
 static void enqueue_step_kernel(const ludvm_sim *s, const StepPlan &pl, int which, int k, cudaStream_t cs)
 {
     const SimDev &D = s->d;
@@ -1870,6 +1912,7 @@ static void enqueue_step_kernel(const ludvm_sim *s, const StepPlan &pl, int whic
     default:
         if (pl.ov) k_finish_ov<<<pl.g4, 256, s->finish_smem, cs>>>(D, k, pl.R, pl.slots);
         else k_finish<<<pl.g4, 256, s->finish_smem, cs>>>(D, k, pl.tchunks);
+        if (D.dp) k_pressure<<<1, 256, 0, cs>>>(D, k);
         break;
     }
 }
@@ -2013,6 +2056,24 @@ LUDVM_API int ludvm_sim_create(ludvm_ctx *ctx, const ludvm_sim_params *p, const 
     return LUDVM_OK;
 }
 
+LUDVM_API int ludvm_sim_enable_pressure(ludvm_sim *s)
+{
+    ARG_CHECK(s != nullptr);
+    if (s->steps_enqueued > 0) return set_error(LUDVM_E_STATE, "ludvm_sim_enable_pressure must precede the first step");
+    if (s->d.dp) return LUDVM_OK;
+    DeviceGuard g(s->ctx->device);
+    const size_t bytes = (size_t)s->d.nt * s->d.P * sizeof(double);
+    void *p;
+    int rc = dev_malloc(s->ctx, s->allocs, bytes, &p);
+    if (rc) return rc;
+    CUDA_TRY(cudaMemsetAsync(p, 0, bytes, s->ctx->stream));   // row 0 and rows of steps not run stay zero
+    s->d.dp = (double *)p;
+    // the one-CTA driver reads the device copy of the descriptor; the other drivers take `d` by value at launch
+    CUDA_TRY(cudaMemcpyAsync(s->d_case, &s->d, sizeof(SimDev), cudaMemcpyHostToDevice, s->ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(s->ctx->stream));
+    return LUDVM_OK;
+}
+
 LUDVM_API int ludvm_sim_run(ludvm_sim *s, long nsteps)
 {
     ARG_CHECK(s != nullptr && nsteps >= 0);
@@ -2082,7 +2143,7 @@ LUDVM_API int ludvm_sim_run(ludvm_sim *s, long nsteps)
             it = s->graphs.emplace(key, ge).first;
         }
         CUDA_TRY(cudaGraphLaunch(it->second, s->ctx->stream));
-        s->ctx->launches += (plan_step(s, b).ov ? 5L : 4L) * k + 1;
+        s->ctx->launches += (plan_step(s, b).ov ? 5L : 4L) * k + (s->d.dp ? k : 0) + 1;
         s->steps_enqueued += k;
         todo -= k;
     }
@@ -2120,7 +2181,7 @@ LUDVM_API int ludvm_sim_profile_steps(ludvm_sim *s, long nsteps, double *ms_out)
             ms_out[which] += ms;
             ms_out[4] += ms;
         }
-        s->ctx->launches += 5;
+        s->ctx->launches += s->d.dp ? 6 : 5;
         s->steps_enqueued += 1;
     }
     CUDA_TRY(cudaStreamSynchronize(st));
@@ -2173,6 +2234,7 @@ static int field_info(ludvm_sim *s, int field, const void **ptr, size_t *bytes)
     case LUDVM_F_M: *ptr = D.M; *bytes = nt * d8; break;
     case LUDVM_F_COUNTERS: *ptr = D.counters; *bytes = 4 * sizeof(long long); break;
     case LUDVM_F_RANGE_BAD: *ptr = D.range_bad; *bytes = sizeof(int); break;
+    case LUDVM_F_DP: *ptr = D.dp; *bytes = nt * P * d8; break;
     case LUDVM_F_CUR_TEV: case LUDVM_F_CUR_LEV: case LUDVM_F_CUR_FREE:
         *ptr = nullptr; *bytes = 2 * (field == LUDVM_F_CUR_FREE ? nf : nv) * d8; break;
     default: return set_error(LUDVM_E_ARG, "unknown field %d", field);
@@ -2209,6 +2271,7 @@ LUDVM_API int ludvm_sim_fetch_many(ludvm_sim *s, int nfields, const int *fields,
             CUDA_TRY(cudaMemcpyAsync(dsts[k], D.wx + off, n * sizeof(double), cudaMemcpyDeviceToHost, st));
             CUDA_TRY(cudaMemcpyAsync((double *)dsts[k] + n, D.wz + off, n * sizeof(double), cudaMemcpyDeviceToHost, st));
         } else {
+            if (!p && fields[k] == LUDVM_F_DP) return set_error(LUDVM_E_STATE, "the pressure jump was not enabled (ludvm_sim_enable_pressure)");
             if (!p) return set_error(LUDVM_E_STATE, "field %d was not kept (store_history = 0)", fields[k]);
             CUDA_TRY(cudaMemcpyAsync(dsts[k], p, want, cudaMemcpyDeviceToHost, st));
         }

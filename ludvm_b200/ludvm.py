@@ -8,7 +8,9 @@ What runs on the GPU through the C ABI: `induced_velocity` (LUDVM.py:549), `airf
 `time_loop` (LUDVM.py:597), `flowfield` (LUDVM.py:1186).
 
 Extra keyword-only arguments (not in the reference): `mode` ('exact' bit-reproduces numpy, 'fast' uses FMA
-arithmetic), `device`, `store_history`, `motion`, `run`, `steps_per_graph`.
+arithmetic), `device`, `store_history`, `motion`, `run`, `steps_per_graph`, `pressure` (True: `time_loop` fills the
+chordwise pressure jump `dp` [nt, Npoints-1] and so `Cp`, which the reference allocates but leaves zero; see
+`time_loop`).
 """
 import ctypes as C
 import timeit
@@ -58,7 +60,7 @@ class LUDVM:
                  LESPcrit=0.2, Naca='0012', foil_filename=None, G=1, T=2, alpha_m=0, alpha_max=10,
                  k=0.2 * np.pi, phi=90, h_max=1, verbose=True, method='Faure',
                  circulation_freevort=None, xy_freevort=None, *, mode='exact', device=0, store_history=True,
-                 motion='cos', run=True, steps_per_graph=0, ctx=None):
+                 motion='cos', run=True, steps_per_graph=0, ctx=None, pressure=False):
         # LUDVM.py:237-260
         self.t0, self.tf, self.dt = t0, tf, dt
         self.chord, self.rho, self.Uinf = chord, rho, Uinf
@@ -92,6 +94,7 @@ class LUDVM:
         if self.store_history < 0:
             raise ValueError('store_history must be >= 0')
         self.steps_per_graph = int(steps_per_graph)
+        self.pressure = bool(pressure)
         self._ctx = ctx
         self._sim = None
 
@@ -266,7 +269,14 @@ class LUDVM:
             free_g=free_g, free_xz=f64(self.xy_freevort))
 
     def time_loop(self, print_dt=50, BCcheck=False, tables=None, nsteps=None):
-        """The time integrator (LUDVM.py:597-1171) on the device: CUDA-graph replay of the 4-kernel step."""
+        """The time integrator (LUDVM.py:597-1171) on the device: CUDA-graph replay of the 4-kernel step.
+
+        With `pressure=True` the device also fills dp[i, j], the pressure jump at gamma point j of step i (row 0 and the
+        rows of steps not run stay zero):
+            dp[i] = rho * ((Uinf*cos(alpha[i]) + h_dot[i]*sin(alpha[i]) + u) * gamma_airfoil[i-1]
+                           + (Gamma_airfoil[i-1] - Gamma_airfoil[i-2]) / dt)
+        where u is the tangential wake velocity at the gamma points that the normal force integrates
+        (LUDVM.py:1049-1057); at i = 1 the Gamma_airfoil[i-2] term is 0."""
         if BCcheck and not (self.store_history == 1 and nsteps is None):
             raise ValueError("BCcheck=True is evaluated from the full vortex-path history (store_history=True, whole run)")
         tb = tables if tables is not None else self.step_tables()
@@ -295,6 +305,8 @@ class LUDVM:
         sim = _lib.c_vp()
         check(L.ludvm_sim_create(self.ctx.handle, C.byref(p), C.byref(t), C.byref(sim)))
         self._sim = sim
+        if self.pressure:
+            check(L.ludvm_sim_enable_pressure(sim))
         total = nv if nsteps is None else min(int(nsteps), nv)
         K = self.steps_per_graph if self.steps_per_graph > 0 else 50
         chunk = max(K, (max(print_dt, 1) // K) * K) if self.verbose else total
@@ -375,6 +387,8 @@ class LUDVM:
             want += [('PATH_TEV', (hrows, 2, nv)), ('PATH_LEV', (hrows, 2, nv)), ('PATH_FREE', (nt, 2, nf))]
         else:   # only the latest positions exist (the O(nt^2) history is the memory wall at dt=2e-3, tf=40)
             want += [('CUR_TEV', (2, nv)), ('CUR_LEV', (2, nv)), ('CUR_FREE', (2, nf))]
+        if self.pressure:
+            want.append(('DP', (nt, P)))
         got = {name: np.empty(shape) for name, shape in want}
         got['COUNTERS'], got['RANGE_BAD'] = np.empty(4, dtype=np.int64), np.empty(1, dtype=np.int32)
         n = len(got)
@@ -393,7 +407,8 @@ class LUDVM:
         self.fourier = got['FOURIER']
         self.LESP, self.LESP_prev, self.LEV_shed = got['LESP'], got['LESP_PREV'], got['LEV_SHED']
         self.Fn, self.Fs, self.L, self.D, self.T, self.M = (got[k] for k in ('FN', 'FS', 'L', 'D', 'T', 'M'))
-        self.dp = np.zeros([nt, P])                      # never assigned by the reference (LUDVM.py:1059-1064)
+        # never assigned by the reference (LUDVM.py:1059-1064): zero unless pressure=True
+        self.dp = got['DP'] if self.pressure else np.zeros([nt, P])
         self.BC = np.zeros([nv, self.Npoints])
         cnt = got['COUNTERS']
         self.steps_done, self.itev, self.ilev = int(cnt[0]), int(cnt[1]), int(cnt[2])

@@ -36,10 +36,13 @@ def run_sweep(cases, mode="exact", ctx=None, device=0, case_slice=None):
     of [ncases, nt] arrays: the load histories, coefficients (LUDVM.py:1173-1184), LESP, LEV_shed, circulations."""
     import time
     t_host = time.perf_counter()
-    ctx = ctx or _lib.default_context(device)
     sel = list(cases[case_slice] if case_slice is not None else cases)
     if not sel:
         raise ValueError("empty sweep")
+    if any(kw.get("pressure") for kw in sel):
+        raise ValueError("run_sweep does not compute the pressure jump (its cases keep no bound-vortex history); "
+                         "run LUDVM(..., pressure=True) per case instead")
+    ctx = ctx or _lib.default_context(device)
     # The host tables and the parameter / table structs depend on everything but LESPcrit: built once per distinct
     # motion, copied per case (filling 4096 structs field by field cost more than the fast-mode kernel's launch).
     shared, params, tables, objs = {}, [], [], []
