@@ -265,6 +265,11 @@ enum { LUDVM_SW_FN = 0, LUDVM_SW_FS, LUDVM_SW_L, LUDVM_SW_D, LUDVM_SW_T, LUDVM_S
        LUDVM_SW_LESP_PREV, LUDVM_SW_LEV_SHED, LUDVM_SW_G_TEV, LUDVM_SW_G_LEV, LUDVM_SW_G_BOUND };
 int ludvm_sweep_run(ludvm_ctx *ctx, long ncases, const ludvm_sim_params *params, const ludvm_sim_tables *tables,
                     double *out, size_t out_doubles_per_case);
+/* ludvm_sweep_run plus the pressure jump of ludvm_sim_enable_pressure for every case: dp is a host buffer
+ * [ncases][nt][P] (dp_doubles_per_case = nt * P), row 0 of each case zero.  Same arguments and checks otherwise.
+ * The call allocates ncases * nt * P doubles of device memory for it (LUDVM_E_NOMEM if that fails). */
+int ludvm_sweep_run_pressure(ludvm_ctx *ctx, long ncases, const ludvm_sim_params *params, const ludvm_sim_tables *tables,
+                             double *out, size_t out_doubles_per_case, double *dp, size_t dp_doubles_per_case);
 
 /*
  * Roofline denominator: sustained FP64 FMA issue rate of this GPU, measured with a register-resident DFMA

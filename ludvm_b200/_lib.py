@@ -83,6 +83,8 @@ SIGNATURES = {
     "ludvm_sim_field_bytes": (C.c_int, [c_vp, C.c_int, C.POINTER(C.c_size_t)]),
     "ludvm_sim_destroy": (C.c_int, [c_vp]),
     "ludvm_sweep_run": (C.c_int, [c_vp, C.c_long, C.POINTER(SimParams), C.POINTER(SimTables), c_vp, C.c_size_t]),
+    "ludvm_sweep_run_pressure": (C.c_int, [c_vp, C.c_long, C.POINTER(SimParams), C.POINTER(SimTables), c_vp, C.c_size_t,
+                                           c_vp, C.c_size_t]),
     "ludvm_measure_fp64_fma_rate": (C.c_int, [c_vp, C.c_double, C.POINTER(C.c_double)]),
     "ludvm_measure_fp32_fma_rate": (C.c_int, [c_vp, C.c_double, C.POINTER(C.c_double)]),
 }

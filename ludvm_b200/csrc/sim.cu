@@ -730,7 +730,10 @@ __device__ __forceinline__ void phase_gamma_cumsum(const SimDev &S, const Step &
 // j).  Gamma row itev is summed by another CTA while the loads run (or after them, in the one-CTA driver), so it is formed
 // again here with the same expression; row itev - 1 is complete.  Called after the loads, where little else is live
 // (inside the loads' loop, or out of line, it cost the kernels around it spills); on the graph path it is a kernel of its
-// own after k_finish / k_finish_ov (k_pressure), which keep their register allocation.
+// own after k_finish / k_finish_ov (k_pressure), which keep their register allocation.  In the one-CTA driver
+// (single-simulation Ramesh and the DP sweep instantiations) it runs before that CTA's own phase_gamma_cumsum, so a
+// compact sweep case, whose one Gamma row every step overwrites (af_stride = 0), still holds row itev - 1 in it here:
+// each thread reads Gprev[j] before the same thread (same j mapping) writes that element in phase_gamma_cumsum.
 __device__ __forceinline__ void pressure_row(const SimDev &S, const Step &st)
 {
     const int i = st.i, itev = st.itev;
@@ -793,8 +796,8 @@ __device__ __forceinline__ int conv_fold(const SimDev &S, const Step &st, int ti
 
 // `tab` = shared memory of resident StepTables, or nullptr: then the three tables needed here are built in `sm`.
 // `ov`: the wake velocity at the gamma points was already assembled in S.gp_u / S.gp_w (overlapped step).
-// DP: the driver can carry the pressure jump (S.dp non-null): u is left in the dp row for pressure_row; the sweep
-// drivers cannot, and compile without it.
+// DP: the driver can carry the pressure jump (S.dp non-null): u is left in the dp row for pressure_row.  The sweep
+// instantiations of k_sim_cta without it compile without the store.
 template <bool DP>
 __device__ void phase_finish_loads(const SimDev &S, const Step &st, double *tab, double *sm, int tiled_chunks, int cap,
                                    bool ov = false)  // LUDVM.py:1035-1090
@@ -1515,7 +1518,8 @@ __device__ __noinline__ void cta_finish_update(const SimDev &S, const Step &st)
                               // at 80 registers (more spills): 4096-case sweep 0.582 -> 0.564 s fast, 1.008 -> 0.896 s exact
                               // (profiles/r02o_sweep_occupancy.txt); 4 would need 280 KB of shared memory per SM
 #endif
-template <int THREADS, int METHOD>
+// DP: the cases may carry the pressure jump (S.dp non-null); without it the store of u and pressure_row are compiled out.
+template <int THREADS, int METHOD, bool DP>
 __global__ void __launch_bounds__(THREADS, THREADS <= 128 ? 6 : (THREADS <= 256 ? SWEEP_CTAS_PER_SM : 1)) k_sim_cta(const SimDev *cases, int ncases, int *next_case, int nsteps)
 {
     extern __shared__ double sm[];
@@ -1570,8 +1574,8 @@ __global__ void __launch_bounds__(THREADS, THREADS <= 128 ? 6 : (THREADS <= 256 
                 cta_conv_partials(S, st);
             __syncthreads();
             CTA_T(2);
-            phase_finish_loads<THREADS == RAMESH_THREADS>(S, st, tab, scr, 0, S.sum_nodes);   // single-simulation Ramesh runs only
-            if (THREADS == RAMESH_THREADS && S.dp) pressure_row(S, st);
+            phase_finish_loads<DP>(S, st, tab, scr, 0, S.sum_nodes);
+            if (DP && S.dp) pressure_row(S, st);
             CTA_T(3);
             cta_finish_update(S, st);
             phase_gamma_cumsum(S, st, threadIdx.x, blockDim.x);
@@ -1964,10 +1968,13 @@ static int set_smem_limits(size_t solve_smem, size_t finish_smem)
     if (solve_smem > 48 * 1024) {
         CUDA_TRY(cudaFuncSetAttribute(k_solve, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
         CUDA_TRY(cudaFuncSetAttribute(k_solve_small, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
-        CUDA_TRY(cudaFuncSetAttribute(k_sim_cta<CTA_THREADS, LUDVM_METHOD_FAURE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
-        CUDA_TRY(cudaFuncSetAttribute(k_sim_cta<128, LUDVM_METHOD_FAURE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
-        CUDA_TRY(cudaFuncSetAttribute(k_sim_cta<CTA_THREADS, LUDVM_METHOD_RAMESH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
-        CUDA_TRY(cudaFuncSetAttribute(k_sim_cta<RAMESH_THREADS, LUDVM_METHOD_RAMESH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
+        CUDA_TRY(cudaFuncSetAttribute(k_sim_cta<CTA_THREADS, LUDVM_METHOD_FAURE, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
+        CUDA_TRY(cudaFuncSetAttribute(k_sim_cta<128, LUDVM_METHOD_FAURE, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
+        CUDA_TRY(cudaFuncSetAttribute(k_sim_cta<CTA_THREADS, LUDVM_METHOD_RAMESH, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
+        CUDA_TRY(cudaFuncSetAttribute(k_sim_cta<CTA_THREADS, LUDVM_METHOD_FAURE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
+        CUDA_TRY(cudaFuncSetAttribute(k_sim_cta<128, LUDVM_METHOD_FAURE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
+        CUDA_TRY(cudaFuncSetAttribute(k_sim_cta<CTA_THREADS, LUDVM_METHOD_RAMESH, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
+        CUDA_TRY(cudaFuncSetAttribute(k_sim_cta<RAMESH_THREADS, LUDVM_METHOD_RAMESH, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
     }
     if (finish_smem > 48 * 1024)
         CUDA_TRY(cudaFuncSetAttribute(k_finish, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)finish_smem));
@@ -2083,7 +2090,7 @@ LUDVM_API int ludvm_sim_run(ludvm_sim *s, long nsteps)
     if (todo <= 0) return LUDVM_OK;
     if (s->p.method == LUDVM_METHOD_RAMESH) {  // CTA path
         CUDA_TRY(cudaMemsetAsync(s->d_next, 0, sizeof(int), s->ctx->stream));
-        k_sim_cta<RAMESH_THREADS, LUDVM_METHOD_RAMESH><<<1, RAMESH_THREADS, s->solve_smem, s->ctx->stream>>>(s->d_case, 1, s->d_next, (int)todo);
+        k_sim_cta<RAMESH_THREADS, LUDVM_METHOD_RAMESH, true><<<1, RAMESH_THREADS, s->solve_smem, s->ctx->stream>>>(s->d_case, 1, s->d_next, (int)todo);
         CUDA_TRY(cudaGetLastError());
         s->ctx->launches++;
         s->steps_enqueued += todo;
@@ -2303,8 +2310,19 @@ LUDVM_API int ludvm_sim_destroy(ludvm_sim *s)
 // ---------------------------------------------------------------------------------------------------
 // batched parameter sweep (BASELINE.json configs[3]): ncases independent simulations, one CTA per case
 // ---------------------------------------------------------------------------------------------------
-LUDVM_API int ludvm_sweep_run(ludvm_ctx *ctx, long ncases, const ludvm_sim_params *params,
-                              const ludvm_sim_tables *tables, double *out, size_t out_doubles_per_case)
+namespace ludvm {
+
+using SweepKernel = void (*)(const SimDev *, int, int *, int);
+
+template <int THREADS, int METHOD>
+static SweepKernel sweep_kernel(bool dp)
+{
+    return dp ? k_sim_cta<THREADS, METHOD, true> : k_sim_cta<THREADS, METHOD, false>;
+}
+
+// ludvm_sweep_run (dp null) and ludvm_sweep_run_pressure: dp, if set, is a host buffer [ncases][nt][P].
+static int sweep_run(ludvm_ctx *ctx, long ncases, const ludvm_sim_params *params, const ludvm_sim_tables *tables,
+                     double *out, size_t out_doubles_per_case, double *dp, size_t dp_doubles_per_case)
 {
     ARG_CHECK(ctx && params && tables && out && ncases > 0 && ncases < (1 << 24));
     int rc;
@@ -2316,6 +2334,7 @@ LUDVM_API int ludvm_sweep_run(ludvm_ctx *ctx, long ncases, const ludvm_sim_param
     }
     const size_t nt = p0.nt;
     ARG_CHECK(out_doubles_per_case == (size_t)LUDVM_SWEEP_FIELDS * nt);
+    if (dp) ARG_CHECK(dp_doubles_per_case == nt * (size_t)p0.P);
     DeviceGuard g(ctx->device);
     std::vector<void *> allocs;
     auto cleanup = [&]() { for (void *p : allocs) cudaFreeAsync(p, ctx->stream); };
@@ -2351,6 +2370,14 @@ LUDVM_API int ludvm_sweep_run(ludvm_ctx *ctx, long ncases, const ludvm_sim_param
     Arena real;
     real.base = (char *)base;
     for (long c = 0; c < ncases; c++) layout_case(host_cases[c], params[c], dts[c], real, target, sum_nodes, true, cta_threads);
+    // the pressure jump lives outside the arena (a sweep without it keeps the arena's layout); row 0 of each case stays 0
+    void *ddp = nullptr;
+    const size_t dp_bytes = dp ? sizeof(double) * (size_t)ncases * dp_doubles_per_case : 0;
+    if (dp) {
+        TRY(dev_malloc(ctx, allocs, dp_bytes, &ddp));
+        CU(cudaMemsetAsync(ddp, 0, dp_bytes, ctx->stream));
+        for (long c = 0; c < ncases; c++) host_cases[c].dp = (double *)ddp + (size_t)c * dp_doubles_per_case;
+    }
     void *dcases, *dnext;
     TRY(dev_malloc(ctx, allocs, sizeof(SimDev) * (size_t)ncases + 256, &dcases));
     TRY(dev_malloc(ctx, allocs, 256, &dnext));
@@ -2360,14 +2387,13 @@ LUDVM_API int ludvm_sweep_run(ludvm_ctx *ctx, long ncases, const ludvm_sim_param
     auto t1 = now();
     size_t smem = solve_smem_bytes(host_cases[0]);
     TRY(set_smem_limits(smem, 0));
+    const SweepKernel kern = cta_threads == 128 ? sweep_kernel<128, LUDVM_METHOD_FAURE>(dp)
+                             : ramesh          ? sweep_kernel<CTA_THREADS, LUDVM_METHOD_RAMESH>(dp)
+                                               : sweep_kernel<CTA_THREADS, LUDVM_METHOD_FAURE>(dp);
     int per_sm = 1;
-    if (cta_threads == 128) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sim_cta<128, LUDVM_METHOD_FAURE>, 128, smem));
-    else if (ramesh) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sim_cta<CTA_THREADS, LUDVM_METHOD_RAMESH>, CTA_THREADS, smem));
-    else CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sim_cta<CTA_THREADS, LUDVM_METHOD_FAURE>, CTA_THREADS, smem));
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, cta_threads, smem));
     int grid = (int)std::min<long>(ncases, (long)ctx->sm_count * std::max(per_sm, 1));
-    if (cta_threads == 128) k_sim_cta<128, LUDVM_METHOD_FAURE><<<grid, 128, smem, ctx->stream>>>((const SimDev *)dcases, (int)ncases, (int *)dnext, (int)nt);
-    else if (ramesh) k_sim_cta<CTA_THREADS, LUDVM_METHOD_RAMESH><<<grid, CTA_THREADS, smem, ctx->stream>>>((const SimDev *)dcases, (int)ncases, (int *)dnext, (int)nt);
-    else k_sim_cta<CTA_THREADS, LUDVM_METHOD_FAURE><<<grid, CTA_THREADS, smem, ctx->stream>>>((const SimDev *)dcases, (int)ncases, (int *)dnext, (int)nt);
+    kern<<<grid, cta_threads, smem, ctx->stream>>>((const SimDev *)dcases, (int)ncases, (int *)dnext, (int)nt);
     ctx->launches += 2;
     CU(cudaGetLastError());
     auto t2 = now();
@@ -2378,6 +2404,7 @@ LUDVM_API int ludvm_sweep_run(ludvm_ctx *ctx, long ncases, const ludvm_sim_param
     ctx->launches++;
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(out, dout, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    if (dp) CU(cudaMemcpyAsync(dp, ddp, dp_bytes, cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
     auto t3 = now();
 #undef CU
@@ -2386,8 +2413,25 @@ LUDVM_API int ludvm_sweep_run(ludvm_ctx *ctx, long ncases, const ludvm_sim_param
     if (tm) {
         auto t4 = std::chrono::steady_clock::now();
         auto ms = [](auto a, auto b) { return std::chrono::duration<double, std::milli>(b - a).count(); };
-        fprintf(stderr, "ludvm_sweep_run: upload+alloc+init %.1f ms, kernel %.1f ms, gather+D2H %.1f ms, free %.1f ms (arena %.0f MB)\n",
-                ms(t0, t1), ms(t1, t2), ms(t2, t3), ms(t3, t4), measure.off / 1048576.0);
+        fprintf(stderr, "ludvm_sweep_run: upload+alloc+init %.1f ms, kernel %.1f ms, gather+D2H %.1f ms, free %.1f ms (arena %.0f MB, "
+                "dp %.0f MB, %d cases resident per SM)\n",
+                ms(t0, t1), ms(t1, t2), ms(t2, t3), ms(t3, t4), measure.off / 1048576.0, dp_bytes / 1048576.0, per_sm);
     }
     return LUDVM_OK;
+}
+
+}  // namespace ludvm
+
+LUDVM_API int ludvm_sweep_run(ludvm_ctx *ctx, long ncases, const ludvm_sim_params *params,
+                              const ludvm_sim_tables *tables, double *out, size_t out_doubles_per_case)
+{
+    return sweep_run(ctx, ncases, params, tables, out, out_doubles_per_case, nullptr, 0);
+}
+
+LUDVM_API int ludvm_sweep_run_pressure(ludvm_ctx *ctx, long ncases, const ludvm_sim_params *params,
+                                       const ludvm_sim_tables *tables, double *out, size_t out_doubles_per_case,
+                                       double *dp, size_t dp_doubles_per_case)
+{
+    ARG_CHECK(dp != nullptr);
+    return sweep_run(ctx, ncases, params, tables, out, out_doubles_per_case, dp, dp_doubles_per_case);
 }
