@@ -80,7 +80,8 @@ int ludvm_ctx_launch_count(ludvm_ctx *ctx, long long *out);
  * 1 = the flagged instantiation ran; reading it synchronises the context's stream), fused kernel: 1 = 12-slot pair arithmetic. */
 enum { LUDVM_K_NONE = 0, LUDVM_K_EXACT_ROWS = 1, LUDVM_K_EXACT_TILED = 2, LUDVM_K_FAST_ROWS = 3, LUDVM_K_FAST_TILED = 4,
        LUDVM_K_FAST_TILED_TMA = 5, LUDVM_K_FAST32_TILED = 6, LUDVM_K_FAST32X2_TILED = 7, LUDVM_K_FAST_FUSED = 8,
-       LUDVM_K_TREE = 9 /* out[2] = leaf level of the quadtree, out[5] = interpolation order */ };
+       LUDVM_K_TREE = 9 /* out[2] = leaf level of the quadtree, out[5] = interpolation order */,
+       LUDVM_K_FAST_SYM = 10 /* ludvm_selfconv_step_all: out[1] = rows per lane, out[5] = columns per staged block */ };
 int ludvm_ctx_last_plan(ludvm_ctx *ctx, int32_t out[8]);
 
 /*
@@ -104,6 +105,18 @@ int ludvm_induced_velocity(ludvm_ctx *ctx, int mode, const double *gamma, long n
 int ludvm_selfconv_step(ludvm_ctx *ctx, int mode, const double *gamma, const double *x, const double *z,
                         const double *vc4_per_source, double vc4, long n, long row0, long nrows, double dt,
                         double *x_out, double *z_out, double *u_out, double *w_out);
+
+/*
+ * The same step for the whole cloud (row0 = 0, nrows = n), with the same results bit for bit.  In fast mode with one
+ * finite core vc4 > 0 (vc4_per_source NULL), 16-byte aligned arrays and n >= 2^17 it evaluates every unordered pair
+ * once and applies the shared part of the term to both vortices (LUDVM_K_FAST_SYM: 8 FP64-pipe slots per term instead
+ * of 13); otherwise it does exactly what ludvm_selfconv_step(..., row0 = 0, nrows = n, ...) does.  A LUDVM_K_FAST_SYM
+ * launch that stops making progress gives up instead of hanging; the next ludvm_selfconv_step_all or
+ * ludvm_ctx_synchronize on the context then returns LUDVM_E_CUDA.
+ */
+int ludvm_selfconv_step_all(ludvm_ctx *ctx, int mode, const double *gamma, const double *x, const double *z,
+                            const double *vc4_per_source, double vc4, long n, double dt, double *x_out, double *z_out,
+                            double *u_out, double *w_out);
 
 /*
  * Same step with the all-gather fused into the kernel epilogue: instead of writing the shard's rows locally for a

@@ -58,6 +58,8 @@ SIGNATURES = {
                                          c_vp, c_vp, C.c_long, c_vp, c_vp, C.c_int]),
     "ludvm_selfconv_step": (C.c_int, [c_vp, C.c_int, c_vp, c_vp, c_vp, c_vp, C.c_double, C.c_long, C.c_long,
                                       C.c_long, C.c_double, c_vp, c_vp, c_vp, c_vp]),
+    "ludvm_selfconv_step_all": (C.c_int, [c_vp, C.c_int, c_vp, c_vp, c_vp, c_vp, C.c_double, C.c_long, C.c_double,
+                                          c_vp, c_vp, c_vp, c_vp]),
     "ludvm_selfconv_step_p2p": (C.c_int, [c_vp, C.c_int, c_vp, c_vp, c_vp, c_vp, C.c_double, C.c_long, C.c_long,
                                           C.c_long, C.c_double, C.c_int, C.POINTER(c_vp), C.POINTER(c_vp)]),
     "ludvm_induced_velocity_tree": (C.c_int, [c_vp, c_vp, c_vp, c_vp, C.c_double, C.c_long, c_vp, c_vp, C.c_long, C.c_int,
@@ -125,6 +127,15 @@ def ptr(a):
     return a.data_ptr()
 
 
+def _pair_slots(kernel, variant_word):
+    """FP64-pipe slots per evaluated term: fast_sym shares 10 of the pair's 13 slots between the terms (i, j) and (j, i)."""
+    if kernel == "fast_sym":
+        return 8
+    if kernel == "fast_fused" and variant_word == 1:
+        return 12
+    return 13 if kernel.startswith("fast_") else 0
+
+
 class Context:
     """One device + stream + scratch.  `stream` is a raw cudaStream_t (int), e.g.
     `torch.cuda.current_stream().cuda_stream`; 0 means the legacy default stream (PyTorch's default stream);
@@ -153,7 +164,7 @@ class Context:
         return n.value
 
     KERNELS = ("none", "exact_rows", "exact_tiled", "fast_rows", "fast_tiled", "fast_tiled_tma", "fast32_tiled",
-               "fast32x2_tiled", "fast_fused", "tree")
+               "fast32x2_tiled", "fast_fused", "tree", "fast_sym")
 
     def last_plan(self):
         """The all-pairs kernel the last call chose: dict(kernel, rows_per_thread, fold, tma, cluster, variant)."""
@@ -162,7 +173,7 @@ class Context:
         k = self.KERNELS[out[0]]
         return dict(kernel=k, rows_per_thread=out[1], fold=out[2], tma=bool(out[3]), cluster=out[4], variant=out[5],
                     warps=out[6], range_bad=out[7] if k.startswith("exact") else 0,
-                    pair_slots=(12 if (k == "fast_fused" and out[7] == 1) else 13) if k.startswith("fast_") else 0)
+                    pair_slots=_pair_slots(k, out[7]))
 
     def fp64_fma_rate(self, ms=200.0):
         r = C.c_double(0)

@@ -1,5 +1,7 @@
 // biot_savart.cu -- generic all-pairs entry points: ludvm_induced_velocity (LUDVM.py:549-570),
 // ludvm_selfconv_step (LUDVM.py:1095-1127 without the aerofoil), ludvm_flowfield_* (LUDVM.py:1186-1298).
+#include <cmath>
+
 #include "biot_savart.cuh"
 
 namespace ludvm {
@@ -108,6 +110,14 @@ k_fast_fused(SrcView S, Tgt T, int nrows, int chunk_len, int nchunks, RowOut O)
 {
     extern __shared__ __align__(128) unsigned char fw_raw[];
     fast_fused_block<R, CL, V>(S, T, nrows, chunk_len, nchunks, O, *reinterpret_cast<FwSmem *>(fw_raw));
+}
+
+// Whole-cloud self-convection with each unordered pair evaluated once (biot_savart.cuh, "fast symmetric"): chain
+// states / partial sums [chunk][n] for k_combine.
+__global__ void __launch_bounds__(32 * FS_WARPS, 2) k_fast_sym(SymArgs A)
+{
+    extern __shared__ __align__(128) unsigned char fs_raw[];
+    fast_sym_warp(A, reinterpret_cast<FsSmem *>(fs_raw)->w[threadIdx.x >> 5]);
 }
 
 // One set of partial row sums.  exact: nfold = tree depth d; fast: nfold = number of chunks.
@@ -414,6 +424,77 @@ static int eval_rows(ludvm_ctx *ctx, int mode, const SrcView &S, const SrcView *
     return LUDVM_OK;
 }
 
+// Smallest cloud for k_fast_sym: from 2^17 vortices fast_chunking cuts 16 chunks, whose 136 chunk pairs x 128-row blocks
+// give ~8700 strips and more for the 2368 warps of the persistent grid.
+#define FS_MIN_N (1L << 17)
+
+// The whole-cloud step through k_fast_sym + k_combine when the cloud is eligible: fast f64 with the 13-slot pair, one
+// finite core vc^4 > 0 for all sources, 16-byte aligned arrays and n >= FS_MIN_N.  *launched = false otherwise.
+static int try_launch_sym(ludvm_ctx *ctx, int mode, const double *gamma, const double *x, const double *z,
+                          const double *vc4_per_source, double vc4, long n, const RowOut &O, bool *launched)
+{
+    *launched = false;
+    if (mode != LUDVM_FAST_F64 || vc4_per_source || !(vc4 > 0.0 && std::isfinite(vc4)) || n < FS_MIN_N ||
+        (((uintptr_t)x | (uintptr_t)z | (uintptr_t)gamma) & 15) != 0)
+        return LUDVM_OK;
+    int chunk_len;
+    long chunks;
+    fast_chunking((int)n, &chunk_len, &chunks);
+    SymArgs A;
+    A.x = x; A.z = z; A.g = gamma; A.vc4 = vc4;
+    A.n = (int)n; A.chunk_len = chunk_len; A.nchunks = (int)chunks;
+    A.bpc = chunk_len / FS_ROWS;
+    A.blast = ceil_div(n - (chunks - 1) * chunk_len, FS_ROWS);
+    A.npairs = (int)(chunks * (chunks + 1) / 2);
+    A.nitems = (long)A.blast * A.npairs + (long)(A.bpc - A.blast) * (A.npairs - 1);
+    const long nblocks = (long)(chunks - 1) * A.bpc + A.blast;
+    int rc;
+    void *pa, *pb, *sync;
+    const size_t part_bytes = sizeof(double) * (size_t)n * chunks;
+    const size_t sync_bytes = 256 + sizeof(unsigned) * (size_t)nblocks * chunks;
+    if ((rc = scratch_reserve(ctx, SLOT_PART_A, part_bytes, &pa)) || (rc = scratch_reserve(ctx, SLOT_PART_A + 1, part_bytes, &pb)) ||
+        (rc = scratch_reserve(ctx, SLOT_SYM_SYNC, sync_bytes, &sync)))
+        return rc;
+    if (!ctx->sym_timeout) {
+        CUDA_TRY(cudaHostAlloc((void **)&ctx->sym_timeout, sizeof(int), cudaHostAllocMapped));
+        *(volatile int *)ctx->sym_timeout = 0;
+    }
+    int *timeout_dev;
+    CUDA_TRY(cudaHostGetDevicePointer((void **)&timeout_dev, ctx->sym_timeout, 0));
+    A.pu = (double *)pa;
+    A.pw = (double *)pb;
+    A.ticket = (unsigned *)sync;
+    A.abort = (int *)((char *)sync + 128);
+    A.progress = (unsigned *)((char *)sync + 256);
+    A.timeout = timeout_dev;
+    CUDA_TRY(cudaMemsetAsync(sync, 0, sync_bytes, ctx->stream));
+    static bool configured[16] = {};                       // per device; a function attribute is per device
+    static int ctas_per_sm[16] = {};
+    if (!configured[ctx->device & 15]) {
+        CUDA_TRY(cudaFuncSetAttribute(k_fast_sym, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FsSmem)));
+        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm[ctx->device & 15], k_fast_sym,
+                                                               32 * FS_WARPS, sizeof(FsSmem)));
+        configured[ctx->device & 15] = true;
+    }
+    // persistent: every CTA that fits at once (a waiting warp only waits on a warp that holds an earlier ticket and
+    // is therefore running, so co-residency is not needed for progress)
+    const int grid = ctx->sm_count * std::max(1, ctas_per_sm[ctx->device & 15]);
+    k_fast_sym<<<grid, 32 * FS_WARPS, sizeof(FsSmem), ctx->stream>>>(A);
+    ctx->launches++;
+    CUDA_TRY(cudaGetLastError());
+    CombineArgs ca{};
+    ca.p = {A.pu, A.pw, (int)chunks};
+    ca.nrows = (int)n;
+    ca.out = O;
+    k_combine<<<ceil_div(n, 256), 256, 0, ctx->stream>>>(ca);
+    ctx->launches++;
+    CUDA_TRY(cudaGetLastError());
+    set_plan(ctx, LUDVM_K_FAST_SYM, 4, (int)chunks, 1, 1, FS_STAGE);
+    ctx->plan[6] = FS_WARPS;
+    *launched = true;
+    return LUDVM_OK;
+}
+
 static int check_mode(int mode)
 {
     if (mode != LUDVM_EXACT_F64 && mode != LUDVM_FAST_F64 && mode != LUDVM_FAST_F32 && mode != LUDVM_FAST12_F64)
@@ -498,6 +579,30 @@ LUDVM_API int ludvm_selfconv_step(ludvm_ctx *ctx, int mode, const double *gamma,
     O.xo = x_out;
     O.zo = z_out;
     return selfconv_rows(ctx, mode, gamma, x, z, vc4_per_source, vc4, n, row0, nrows, dt, O);
+}
+
+LUDVM_API int ludvm_selfconv_step_all(ludvm_ctx *ctx, int mode, const double *gamma, const double *x, const double *z,
+                                      const double *vc4_per_source, double vc4, long n, double dt, double *x_out,
+                                      double *z_out, double *u_out, double *w_out)
+{
+    ARG_CHECK(ctx != nullptr);
+    int rc = check_mode(mode);
+    if (rc) return rc;
+    ARG_CHECK(n > 0 && n < (1L << 30));
+    ARG_CHECK(gamma && x && z && x_out && z_out);
+    if ((rc = sym_timeout_check(ctx))) return rc;
+    DeviceGuard g(ctx->device);
+    RowOut O{};
+    O.u = u_out;
+    O.w = w_out;
+    O.x = x;
+    O.z = z;
+    O.xo = x_out;
+    O.zo = z_out;
+    O.dt = dt;
+    bool sym;
+    if ((rc = try_launch_sym(ctx, mode, gamma, x, z, vc4_per_source, vc4, n, O, &sym)) || sym) return rc;
+    return ludvm_selfconv_step(ctx, mode, gamma, x, z, vc4_per_source, vc4, n, 0, n, dt, x_out, z_out, u_out, w_out);
 }
 
 LUDVM_API int ludvm_selfconv_step_p2p(ludvm_ctx *ctx, int mode, const double *gamma, const double *x, const double *z,

@@ -829,6 +829,279 @@ __device__ __forceinline__ void fast_fused_block(const SrcView &S, const Tgt &T,
     if (CL > 1) cluster_sync_all();                     // nobody leaves while a peer still reads its shared memory
 }
 
+// ---------------------------------------------------------------------------------------------------
+// fast symmetric ("k_fast_sym"): the whole-cloud self-convection sum with every unordered pair evaluated ONCE.
+// Terms (i, j) and (j, i) share r^2, q and y = rsqrt_fast(q) (10 of pair_fast's 13 FP64 slots); only gg = G y and the
+// two accumulating FMAs belong to each direction, so a term costs 8 slots instead of 13.  Because RN(-a) = -RN(a),
+// the transposed term fma(G_i y, -dz_ij, u_j), fma(G_i y, dx_ij, w_j) is bit for bit what pair_fast computes for
+// target j (a signed zero only matters on a -0 accumulator, and one that starts at +0 never becomes -0).
+//
+// Summation order is kept: every (target, source chunk) chain -- the chunks of fast_chunking -- is fed its terms in
+// source order from +0, then scaled by 1/(2 pi) into the [chunk][target] partials that k_combine folds.  The rows are
+// cut into 128-row blocks.  A work item ("strip") is one row block p of chunk a against the columns of chunk c >= a:
+//   row role     the chains (i in p, chunk c) advance over the strip's columns, held in registers;
+//   column role  each column's chain (j, chunk a) comes in from strip p - 1 (through the partials array), advances
+//                over the 128 rows of p in order and goes out to strip p + 1.
+// For c == a the strip starts at the diagonal block (p, p): the chains of p's rows arrive in column form, take their
+// own block's 128 ordered terms unshared (pair_fast, self term included, as k_fast_fused) and continue in row role
+// over the columns after the block.
+//
+// Inside a strip one warp holds the 128 rows (lane k: rows 4k..4k+3) and runs a skewed (systolic) schedule: at step
+// s lane k evaluates column s - k against its four rows in order, then hands that column's (u, w) to lane k + 1 with
+// a shuffle.  Lane 0 takes incoming column states from shared memory, lane 31 stores outgoing ones.  Row chains see
+// columns in increasing order, column chains see rows in increasing order.  Source data comes from a warp-private
+// ring of bulk-copy stages.
+//
+// Scheduling: a persistent grid; warps take strips from one atomic ticket in an order where the producer of every
+// strip (p - 1, same chunk pair) holds a smaller ticket, so a waiting warp only ever waits on a running one.  Column
+// states are published per (row block, chunk) as a progress counter (release / acquire at GPU scope).  A wait that
+// exceeds FS_SPIN_LIMIT sets an error flag and abandons the launch instead of hanging the GPU.
+// ---------------------------------------------------------------------------------------------------
+#define FS_ROWS 128          // rows of a row block (one warp, four rows per lane)
+#define FS_STAGE 64          // columns per bulk-copy stage = steps per block of the step loop
+#define FS_RING 4            // stages in a warp's ring: the 31-step skew reads two, one is in flight
+#define FS_WARPS 8
+#define FS_SPIN_LIMIT (1u << 24)   // polls of 64+ ns: a lost producer becomes an error, not a hung GPU
+
+struct FsWarpSmem {
+    double x[FS_RING * FS_STAGE], z[FS_RING * FS_STAGE], g[FS_RING * FS_STAGE];   // column c of the strip at c % ring
+    double2 cin[2][FS_STAGE];   // incoming column states (u, w) of this block of steps and the next
+    uint64_t full[FS_RING];
+};
+struct FsSmem {
+    FsWarpSmem w[FS_WARPS];
+};
+
+struct SymArgs {
+    const double *x, *z, *g;
+    double vc4;
+    int n, chunk_len, nchunks;
+    int bpc, blast;          // row blocks of a full chunk / of the last chunk
+    int npairs;              // chunk pairs a <= c
+    long nitems;             // strips
+    double *pu, *pw;         // [chunk][n] chain states, then partial sums
+    unsigned *progress;      // [row block][chunk]: absolute end of the column states stored by that strip
+    unsigned *ticket;
+    int *abort;              // device: a warp gave up, the others stop waiting
+    int *timeout;            // host-mapped copy of the same verdict, read by the host without a synchronisation
+};
+
+__device__ __forceinline__ unsigned ld_acquire_gpu(const unsigned *p)
+{
+    unsigned v;
+    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+    return v;
+}
+__device__ __forceinline__ void st_release_gpu(unsigned *p, unsigned v)
+{
+    asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+
+// Wait (all lanes) until *p >= need.  false: the limit was hit or another warp already gave up.
+__device__ __forceinline__ bool fs_wait(const SymArgs &A, const unsigned *p, unsigned need)
+{
+    unsigned spins = 0;
+    while (ld_acquire_gpu(p) < need) {
+        if (*(volatile int *)A.abort) return false;
+        if (++spins > FS_SPIN_LIMIT) {
+            *(volatile int *)A.abort = 1;
+            *(volatile int *)A.timeout = 1;
+            return false;
+        }
+        __nanosleep(64);
+    }
+    return true;
+}
+
+// One step for the lane's four rows against column (xj, zj, gj): row chains au, aw and the column chain cu, cw.
+// MASK: the lane's column lies outside the strip (skew prologue / epilogue), its row chains must not move.
+template <bool MASK>
+__device__ __forceinline__ void fs_step(const double (&xr)[4], const double (&zr)[4], const double (&gr)[4],
+                                        double (&au)[4], double (&aw)[4], double xj, double zj, double gj, double vc4,
+                                        double &cu, double &cw, bool valid)
+{
+#pragma unroll
+    for (int r = 0; r < 4; r++) {
+        const double dx = xr[r] - xj;
+        const double dz = zr[r] - zj;
+        const double r2 = fma(dz, dz, dx * dx);
+        const double q = fma(r2, r2, vc4);
+        const double y = rsqrt_fast(q);
+        const double ggr = gj * y, ggc = gr[r] * y;
+        const double nu = fma(ggr, dz, au[r]), nw = fma(-ggr, dx, aw[r]);
+        au[r] = (!MASK || valid) ? nu : au[r];
+        aw[r] = (!MASK || valid) ? nw : aw[r];
+        cu = fma(ggc, -dz, cu);
+        cw = fma(ggc, dx, cw);
+    }
+}
+
+__device__ __forceinline__ void fast_sym_warp(const SymArgs &A, FsWarpSmem &sm)
+{
+    const unsigned full = 0xffffffffu;
+    const int lane = threadIdx.x & 31;
+    double vc4;   // opaque copy: keeps ptxas from re-reading the kernel parameter inside the step loop
+    asm volatile("mov.f64 %0, %1;" : "=d"(vc4) : "d"(A.vc4));
+    const int last = A.nchunks - 1;
+    const size_t n = (size_t)A.n;
+    for (;;) {
+        unsigned tk = 0;
+        if (lane == 0) tk = atomicAdd(A.ticket, 1u);
+        const long t = (long)__shfl_sync(full, tk, 0);
+        if (t >= A.nitems || *(volatile int *)A.abort) return;
+        // ticket -> (round r, chunk pair): round-major, the pair (last, last) -- fewer row blocks -- listed last
+        int r, pr;
+        const long head = (long)A.blast * A.npairs;
+        if (t < head) { r = (int)(t / A.npairs); pr = (int)(t % A.npairs); }
+        else { r = A.blast + (int)((t - head) / (A.npairs - 1)); pr = (int)((t - head) % (A.npairs - 1)); }
+        int a = last, c = last;
+        if (pr < A.npairs - 1) {
+            a = 0;
+            while (pr >= last - a + 1) { pr -= last - a + 1; a++; }
+            c = a + pr;
+        }
+        const int p = a * A.bpc + r;
+        const int c0 = c * A.chunk_len, c1 = min(A.n, c0 + A.chunk_len);
+        const int cstart = min(c1, a == c ? (p + 1) * FS_ROWS : c0);   // first column of the skewed stream
+        const int L = c1 - cstart;
+        const bool has_prev = r > 0;
+        const unsigned *prog_in = A.progress + (size_t)max(p - 1, 0) * A.nchunks + c;   // read only if has_prev
+        unsigned *prog_out = A.progress + (size_t)p * A.nchunks + c;
+        double *cu_g = A.pu + (size_t)a * n, *cw_g = A.pw + (size_t)a * n;   // column chains (j, a)
+
+        const int row0 = p * FS_ROWS + 4 * lane;
+        double xr[4], zr[4], gr[4], au[4], aw[4];
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+            const int i = min(row0 + k, A.n - 1);
+            xr[k] = A.x[i]; zr[k] = A.z[i]; gr[k] = A.g[i];
+            au[k] = 0.0; aw[k] = 0.0;
+        }
+        if (a == c) {   // diagonal block: the rows' chains arrive as column states
+            const int dend = min(c1, (p + 1) * FS_ROWS);
+            if (has_prev) {
+                if (!fs_wait(A, prog_in, (unsigned)dend)) return;
+#pragma unroll
+                for (int k = 0; k < 4; k++)
+                    if (row0 + k < A.n) { au[k] = __ldcg(cu_g + row0 + k); aw[k] = __ldcg(cw_g + row0 + k); }
+            }
+            for (int j = p * FS_ROWS; j < dend; j++) {
+                const double xj = A.x[j], zj = A.z[j], gj = A.g[j];
+#pragma unroll
+                for (int k = 0; k < 4; k++) pair_fast(xr[k], zr[k], xj, zj, gj, vc4, au[k], aw[k]);
+            }
+        }
+
+        if (L > 0) {
+            const int nst = (L + FS_STAGE - 1) / FS_STAGE;
+            const int nblk = (L + 31 + FS_STAGE - 1) / FS_STAGE;
+            if (lane == 0) {
+#pragma unroll
+                for (int k = 0; k < FS_RING; k++) mbar_init(&sm.full[k], 1);
+                asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // lane-filled stages of the last strip
+            }
+            __syncwarp();
+            // stage m = columns [64 m, 64 m + 64) of the stream: the copy engine for a whole stage, the lanes for a ragged
+            // last one
+            auto issue = [&](int m) {
+                const int t0 = cstart + m * FS_STAGE, cnt = min(FS_STAGE, c1 - t0), o = (m % FS_RING) * FS_STAGE;
+                if (cnt == FS_STAGE) {
+                    if (lane == 0) {
+                        uint64_t *bar = &sm.full[m % FS_RING];
+                        mbar_expect_tx(bar, 3 * FS_STAGE * sizeof(double));
+                        bulk_g2s(sm.x + o, A.x + t0, FS_STAGE * sizeof(double), bar);
+                        bulk_g2s(sm.z + o, A.z + t0, FS_STAGE * sizeof(double), bar);
+                        bulk_g2s(sm.g + o, A.g + t0, FS_STAGE * sizeof(double), bar);
+                    }
+                } else {
+                    for (int j = lane; j < cnt; j += 32) {
+                        sm.x[o + j] = A.x[t0 + j];
+                        sm.z[o + j] = A.z[t0 + j];
+                        sm.g[o + j] = A.g[t0 + j];
+                    }
+                }
+            };
+            // incoming column states of stream columns [64 b, 64 b + 64): two per lane
+            double2 pre[2] = {make_double2(0.0, 0.0), make_double2(0.0, 0.0)};
+            auto fetch = [&](int b) -> bool {
+                const int e = min(L, (b + 1) * FS_STAGE);
+                if (!fs_wait(A, prog_in, (unsigned)(cstart + e))) return false;
+#pragma unroll
+                for (int h = 0; h < 2; h++) {
+                    const int jr = b * FS_STAGE + 32 * h + lane;
+                    if (jr < e) pre[h] = make_double2(__ldcg(cu_g + cstart + jr), __ldcg(cw_g + cstart + jr));
+                }
+                return true;
+            };
+            if (has_prev) {
+                if (!fetch(0)) return;
+                sm.cin[0][lane] = pre[0];
+                sm.cin[0][lane + 32] = pre[1];
+            } else {   // the first row block of chunk a starts every column chain at +0
+                sm.cin[0][lane] = sm.cin[0][lane + 32] = sm.cin[1][lane] = sm.cin[1][lane + 32] = make_double2(0.0, 0.0);
+            }
+            issue(0);
+            double cu = 0.0, cw = 0.0;
+            for (int b = 0; b < nblk; b++) {
+                __syncwarp();   // stage b - 2 and cin[(b + 1) & 1] are no longer read; lane-filled data is visible
+                if (b + 1 < nst) issue(b + 1);
+                const bool more = has_prev && (b + 1) * FS_STAGE < L;
+                if (more && !fetch(b + 1)) return;
+                if (b < nst && min(FS_STAGE, c1 - (cstart + b * FS_STAGE)) == FS_STAGE)
+                    mbar_wait(&sm.full[b % FS_RING], (b / FS_RING) & 1);
+                const double2 *cin = sm.cin[b & 1];
+                const int s0 = b * FS_STAGE;
+                if (s0 >= 31 && s0 + FS_STAGE <= L) {
+#pragma unroll 2
+                    for (int tt = 0; tt < FS_STAGE; tt++) {
+                        const int idx = (s0 + tt - lane) & (FS_RING * FS_STAGE - 1);
+                        const double xj = sm.x[idx], zj = sm.z[idx], gj = sm.g[idx];
+                        cu = __shfl_up_sync(full, cu, 1);
+                        cw = __shfl_up_sync(full, cw, 1);
+                        if (lane == 0) { const double2 v = cin[tt]; cu = v.x; cw = v.y; }
+                        fs_step<false>(xr, zr, gr, au, aw, xj, zj, gj, vc4, cu, cw, true);
+                        if (lane == 31) { __stcg(cu_g + cstart + s0 + tt - 31, cu); __stcg(cw_g + cstart + s0 + tt - 31, cw); }
+                    }
+                } else {
+                    for (int tt = 0; tt < FS_STAGE; tt++) {
+                        const int jr = s0 + tt - lane;
+                        const bool valid = jr >= 0 && jr < L;
+                        const int idx = jr & (FS_RING * FS_STAGE - 1);
+                        const double xj = sm.x[idx], zj = sm.z[idx], gj = sm.g[idx];
+                        cu = __shfl_up_sync(full, cu, 1);
+                        cw = __shfl_up_sync(full, cw, 1);
+                        if (lane == 0) { const double2 v = cin[tt]; cu = v.x; cw = v.y; }
+                        fs_step<true>(xr, zr, gr, au, aw, xj, zj, gj, vc4, cu, cw, valid);
+                        if (lane == 31 && valid) { __stcg(cu_g + cstart + jr, cu); __stcg(cw_g + cstart + jr, cw); }
+                    }
+                }
+                if (more) {
+                    sm.cin[(b + 1) & 1][lane] = pre[0];
+                    sm.cin[(b + 1) & 1][lane + 32] = pre[1];
+                }
+                // lane 31 has stored stream columns [0, 64 b + 33)
+                if (lane == 31) st_release_gpu(prog_out, (unsigned)(cstart + min(L, s0 + FS_STAGE - 31)));
+            }
+            if (a < c && r == A.bpc - 1) {   // the last row block of chunk a: its column chains are finished, scale them
+                __syncwarp();
+                for (int j = cstart + lane; j < c1; j += 32) {
+                    cu_g[j] = __ldcg(cu_g + j) * LUDVM_INV_TWO_PI;
+                    cw_g[j] = __ldcg(cw_g + j) * LUDVM_INV_TWO_PI;
+                }
+            }
+        }
+        // the rows' chains (i, c) are finished
+#pragma unroll
+        for (int k = 0; k < 4; k++)
+            if (row0 + k < A.n) {
+                A.pu[(size_t)c * n + row0 + k] = au[k] * LUDVM_INV_TWO_PI;
+                A.pw[(size_t)c * n + row0 + k] = aw[k] * LUDVM_INV_TWO_PI;
+            }
+        __syncwarp();   // the next strip re-initialises the ring's barriers
+    }
+}
+
 // fp32 pair arithmetic; R rows per thread.
 template <int R, class Tgt>
 __device__ __forceinline__ void fast32_tiled_block(const SrcView &S, const Tgt &T, int nrows, int row_block, int c0,

@@ -36,6 +36,14 @@ int scratch_reserve(ludvm_ctx *ctx, int slot, size_t bytes, void **out)
     return LUDVM_OK;
 }
 
+int sym_timeout_check(ludvm_ctx *ctx)
+{
+    if (!ctx->sym_timeout || !*(volatile int *)ctx->sym_timeout) return LUDVM_OK;
+    *(volatile int *)ctx->sym_timeout = 0;
+    return set_error(LUDVM_E_CUDA, "k_fast_sym: a warp waited too long for the column states of its predecessor and the "
+                                   "launch was abandoned; the results of that step are not valid");
+}
+
 int stage_in(ludvm_ctx *ctx, std::initializer_list<HostIn> in)
 {
     size_t total = 0;
@@ -189,6 +197,7 @@ LUDVM_API int ludvm_ctx_destroy(ludvm_ctx *ctx)
     cudaStreamSynchronize(ctx->stream);
     for (auto &s : ctx->dev)
         if (s.ptr) cudaFree(s.ptr);
+    if (ctx->sym_timeout) cudaFreeHost(ctx->sym_timeout);
     if (ctx->own_stream) cudaStreamDestroy(ctx->stream);
     delete ctx;
     return LUDVM_OK;
@@ -199,7 +208,7 @@ LUDVM_API int ludvm_ctx_synchronize(ludvm_ctx *ctx)
     ARG_CHECK(ctx != nullptr);
     DeviceGuard g(ctx->device);
     CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    return LUDVM_OK;
+    return sym_timeout_check(ctx);
 }
 
 LUDVM_API int ludvm_ctx_launch_count(ludvm_ctx *ctx, long long *out)

@@ -124,6 +124,13 @@ def selfconv_step(ctx, mode, g, x, z, vc4, dt, x_out, z_out, row0=0, nrows=None,
                                      ptr(w_out)))
 
 
+def selfconv_step_all(ctx, mode, g, x, z, vc4, dt, x_out, z_out, u_out=None, w_out=None, vc4_per_source=None):
+    """`selfconv_step` of the whole cloud (all rows), bit for bit; in fast mode with one core radius it evaluates each
+    pair of vortices once (kernel fast_sym, see ludvm_selfconv_step_all)."""
+    check(load().ludvm_selfconv_step_all(ctx.handle, _mode(mode), ptr(g), ptr(x), ptr(z), ptr(vc4_per_source), float(vc4),
+                                         x.numel(), float(dt), ptr(x_out), ptr(z_out), ptr(u_out), ptr(w_out)))
+
+
 def selfconv_step_p2p(ctx, mode, g, x, z, vc4, dt, x_out_peer_ptrs, z_out_peer_ptrs, row0, nrows):
     """Self-convection step whose epilogue stores the shard's updated rows into every peer's buffers (raw peer-mapped
     device pointers, this rank included) -- the all-gather fused into the kernel over NVLink."""

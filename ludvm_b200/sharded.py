@@ -150,6 +150,9 @@ class ShardedSelfConvection:
             ops.selfconv_step_tree(self.ctx, g, x, z, vc4, dt, x_out, z_out, row0=row0, nrows=nrows, order=self.order,
                                    leaf=self.leaf)
             return
+        if row0 == 0 and nrows == self.n:      # one rank owns every row: the whole-cloud step (same bits)
+            ops.selfconv_step_all(self.ctx, self.mode, g, x, z, vc4, dt, x_out, z_out)
+            return
         ops.selfconv_step(self.ctx, self.mode, g, x, z, vc4, dt, x_out, z_out, row0=row0, nrows=nrows)
 
     def step(self):
