@@ -232,6 +232,22 @@ int ludvm_sim_profile_steps(ludvm_sim *sim, long nsteps, double *ms_out);
  * row 0 and the rows of steps not yet run are zero.  Allocates and zeroes [nt,P] doubles.  Valid only before the first step
  * is run (LUDVM_E_STATE after); a second call does nothing. */
 int ludvm_sim_enable_pressure(ludvm_sim *sim);
+/* Opt in to the far-field convection (fast mode): every step whose wake bound 2 min(i, nt-1) + 2 + nfree (i = the step's
+ * number, from 1) reaches the library's all-pairs / far-field crossover (SIM_FAR_FIELD_MIN_WAKE in sim.cu, DESIGN.md 4b)
+ * convects the old wake TEV[:itev] ++ LEV[:ilev] ++ FREE through the treecode of ludvm_induced_velocity_tree at this
+ * `order` (2..24; 18 matches the all-pairs fast kernel to ~1e-15 of sum|terms|) instead of all pairs.  Earlier steps are
+ * unchanged.  The result is not bit-equal to the all-pairs run, but it is bitwise reproducible run to run and independent
+ * of steps_per_graph and of how ludvm_sim_run is called.  A far-field step is not captured in a graph: ludvm_sim_run
+ * enqueues it from the host and waits for the device within it (the step's vortex counts, then the tree's bounding box and
+ * largest leaf), so ludvm_sim_run returns once the last far-field step's tree is enqueued.  A step whose cloud the tree
+ * refuses (a leaf of the deepest tree would hold more than 65 536 vortices) runs the all-pairs kernels instead.
+ * Valid only before the first step (LUDVM_E_STATE after); LUDVM_E_UNSUPPORTED in exact mode, for method Ramesh and for
+ * P > 256; LUDVM_E_ARG for an order outside 2..24.  Allocates 3 (2 (nt-1) + nfree) doubles.
+ * ludvm_sim_profile_steps returns LUDVM_E_UNSUPPORTED once it is enabled. */
+int ludvm_sim_enable_far_field(ludvm_sim *sim, int order);
+/* out[0] = steps convected through the far field so far, out[1] = qualifying steps that fell back to all pairs,
+ * out[2] = the order (0: not enabled), out[3] = leaf level of the last tree (0: none yet).  Does not synchronise. */
+int ludvm_sim_far_field_info(ludvm_sim *sim, int64_t out[4]);
 
 enum {
     LUDVM_F_PATH_TEV = 0,  /* [(nt-1)/k+1,2,nt-1]  needs store_history = k >= 1  LUDVM.py:615 */

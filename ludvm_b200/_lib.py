@@ -80,6 +80,8 @@ SIGNATURES = {
     "ludvm_sim_steps_done": (C.c_int, [c_vp, C.POINTER(C.c_long)]),
     "ludvm_sim_profile_steps": (C.c_int, [c_vp, C.c_long, c_dp]),
     "ludvm_sim_enable_pressure": (C.c_int, [c_vp]),
+    "ludvm_sim_enable_far_field": (C.c_int, [c_vp, C.c_int]),
+    "ludvm_sim_far_field_info": (C.c_int, [c_vp, C.POINTER(C.c_int64)]),
     "ludvm_sim_fetch": (C.c_int, [c_vp, C.c_int, c_vp, C.c_size_t]),
     "ludvm_sim_fetch_many": (C.c_int, [c_vp, C.c_int, C.POINTER(C.c_int), C.POINTER(c_vp), C.POINTER(C.c_size_t)]),
     "ludvm_sim_field_bytes": (C.c_int, [c_vp, C.c_int, C.POINTER(C.c_size_t)]),

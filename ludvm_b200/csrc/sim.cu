@@ -16,7 +16,7 @@
 //                        (convection), plus the bound vortices on the wake               (LUDVM.py:1049-1054, 1095-1124)
 //   phase_finish_*       loads Fn, Fs, L, D, T, M; fold partials, forward-Euler update in place, history snapshot
 //                                                                                         (LUDVM.py:1069-1090, 1108-1127)
-// and three drivers run them:
+// and these drivers run them:
 //   * coop path   -- k_sim_persist: one thread-block cluster (smallest wakes) or one persistent cooperative grid (one CTA per SM) runs all steps while the wake is
 //                    small (latency-bound), grid barriers between the phases, the solve CTA's tables resident in
 //                    shared memory.
@@ -25,6 +25,8 @@
 //                    bracket of the wake size).  In fast mode with wakes >= SIM_TILED_MIN_WAKE the step is the
 //                    overlapped one: the old wake's self-convection (shared-memory tiled kernel) on a second graph
 //                    branch beside phase 1 + solve.
+//   * far-field steps -- opt-in (ludvm_sim_enable_far_field), wakes >= SIM_FAR_FIELD_MIN_WAKE: the overlapped step with the
+//                    old wake's self-convection through the treecode (tree.cu), enqueued step by step from the host.
 //   * CTA path    -- k_sim_cta: one persistent CTA runs ALL steps of one case with __syncthreads() between phases;
 //                    cases are pulled from an atomic counter.  Used for batched parameter sweeps (config 4: 4096
 //                    independent cases, no collective) and for method='Ramesh', whose Newton loops have a
@@ -55,6 +57,11 @@ namespace ludvm {
                                   // case, us per step over the 400 steps, exact / fast: cluster up to 128: 32.2 / 26.1, 256: 31.1 / 25.3,
                                   // 384: 30.2 / 24.8, 512: 29.6 / 24.4, all 604: 31.0 / 25.0; cooperative grid alone 33.4 / 26.9
                                   // (profiles/r02l_coop_probe.txt): past ~500 vortices the O(N^2) phases want more than 16 SMs
+#define SIM_FAR_FIELD_MIN_WAKE 65536   // far_field_order set: steps whose wake bound is at least this take the far-field step.
+                                       // Fast-mode ms per step, all pairs / far field at order 18, gust of nfree vortices
+                                       // (profiles/far_field_time_loop_probe.txt; B200, 1000 W): 2^14 0.35 / 1.53,
+                                       // 2^15 1.01 / 1.94, 2^16 3.67 / 2.14, 2^17 14.4 / 2.74
+static_assert(SIM_FAR_FIELD_MIN_WAKE >= SIM_TILED_MIN_WAKE, "the far-field step replaces branch B of the overlapped step");
 #define FINISH_STAGE 4096         // doubles of staging in the loads block of k_finish
 #define SOLVE_SMEM_LIMIT (200 * 1024)   // dynamic shared memory of the solve kernel (bytes)
 #define LUDVM_MAX_PANELS 1024     // Npoints - 1 <= this: 18 doubles per panel of the solve kernel's fixed shared memory
@@ -1131,7 +1138,9 @@ __global__ void __launch_bounds__(256) k_conv_new(SimDev S, int s)
     }
 }
 
-__global__ void __launch_bounds__(256) k_finish_ov(SimDev S, int s, int R, int slots)
+// `chunks` = partial sums per row of pb_u / pb_w: 0 = k_conv_old_tiled's (TiledGeom of the actual wake), 1 = the
+// far-field step's single finished row.
+__global__ void __launch_bounds__(256) k_finish_ov(SimDev S, int s, int R, int slots, int chunks)
 {
     extern __shared__ double sm[];
     Step st;
@@ -1148,7 +1157,7 @@ __global__ void __launch_bounds__(256) k_finish_ov(SimDev S, int s, int R, int s
     const int i = st.i, nv = S.nv, nT = st.itev + 1, nL = st.ilev + 1;
     SrcView W = wake_view(S, nT, nL);
     const int nold = W.n - 2, npart = nold + 3;
-    const int chunks = TiledGeom(npart, nold, R, slots).chunks;
+    if (chunks == 0) chunks = TiledGeom(npart, nold, R, slots).chunks;
     const bool shed = S.lev_shed[i] != -1.0;
     const double dt = S.dt;
     for (long r = (long)(blockIdx.x - 2) * blockDim.x + threadIdx.x; r < W.n; r += (long)(gridDim.x - 2) * blockDim.x) {
@@ -1178,6 +1187,58 @@ __global__ void __launch_bounds__(256) k_finish_ov(SimDev S, int s, int R, int s
             *hx = xn;
             *hz = zn;
         }
+    }
+}
+
+// ---------------------------------------------------------------------------------------------------
+// far-field step (LUDVM(..., far_field_order=p), fast mode, wakes >= SIM_FAR_FIELD_MIN_WAKE): branch B of the
+// overlapped step with the old wake's self-convection evaluated by the treecode (tree.cu) instead of k_conv_old_tiled.
+//   k_ff_gather       the old wake TEV[:itev] ++ LEV[:ilev] ++ FREE, contiguous, in logical order (the tree's sources
+//                     and targets: one sort serves both)
+//   tree              rows 0 .. nold-1 of pb_u / pb_w, one finished sum per row
+//   k_ff_extra_rows   rows nold .. nold+2 (TgtWakePlus: the new TEV, the LEV, the idle LEV slot at the origin) against
+//                     the old wake by all pairs; kept out of the tree, whose bounding box the origin would stretch
+// The join (k_conv_new -> k_finish_ov with one partial per row) is the overlapped step's.  Every sum has a fixed order, so
+// the step is bitwise reproducible run to run.
+// ---------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) k_ff_gather(SimDev S, double *x, double *z, double *g)
+{
+    Step st;
+    if (!step_begin(S, 0, st)) return;
+    const SrcView W = wake_view(S, st.itev, st.ilev);
+    for (long r = (long)blockIdx.x * blockDim.x + threadIdx.x; r < W.n; r += (long)gridDim.x * blockDim.x) {
+        const int p = W.phys((int)r);
+        x[r] = S.wx[p];
+        z[r] = S.wz[p];
+        g[r] = S.wg[p];
+    }
+}
+
+#define FF_EXTRA_THREADS 1024
+__global__ void __launch_bounds__(FF_EXTRA_THREADS) k_ff_extra_rows(SimDev S, const double *x, const double *z,
+                                                                    const double *g, int n)
+{
+    __shared__ double su[FF_EXTRA_THREADS], sw[FF_EXTRA_THREADS];
+    Step st;
+    if (!step_begin(S, 0, st)) return;
+    const int row = blockIdx.x, tid = threadIdx.x;   // 0: the new TEV, 1: the LEV, 2: the idle LEV slot
+    double xp = 0.0, zp = 0.0;
+    if (row == 0) place_tev(S, st.i, st.itev, xp, zp);
+    else if (row == 1) place_lev(S, st.i, st.ilev, xp, zp);
+    double u = 0.0, w = 0.0;
+    for (int j = tid; j < n; j += FF_EXTRA_THREADS) pair_fast(xp, zp, x[j], z[j], g[j] * LUDVM_INV_TWO_PI, S.vc4, u, w);
+    su[tid] = u;
+    sw[tid] = w;
+    for (int h = FF_EXTRA_THREADS / 2; h > 0; h >>= 1) {   // fixed-shape tree: the same sum on every run
+        __syncthreads();
+        if (tid < h) {
+            su[tid] += su[tid + h];
+            sw[tid] += sw[tid + h];
+        }
+    }
+    if (tid == 0) {
+        S.pb_u[n + row] = su[0];
+        S.pb_w[n + row] = sw[0];
     }
 }
 
@@ -1759,6 +1820,11 @@ struct ludvm_sim {
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     cudaStream_t cap_stream = nullptr;  // private stream used only to record graphs (the context's stream may be
                                         // the legacy default stream, which cannot be captured)
+    // far field (ludvm_sim_enable_far_field): order (0 = off), the old wake compacted for the tree [3][2 nv + nfree],
+    // and far_field_info's counters
+    int ff_order = 0;
+    double *ff_xzg = nullptr;
+    long long ff_steps = 0, ff_fallback = 0, ff_leaf_level = 0;
 };
 
 namespace ludvm {
@@ -1914,11 +1980,23 @@ static void enqueue_step_kernel(const ludvm_sim *s, const StepPlan &pl, int whic
         break;
     case 4: k_conv_new<<<pl.g5, 256, 0, cs>>>(D, k); break;
     default:
-        if (pl.ov) k_finish_ov<<<pl.g4, 256, s->finish_smem, cs>>>(D, k, pl.R, pl.slots);
+        if (pl.ov) k_finish_ov<<<pl.g4, 256, s->finish_smem, cs>>>(D, k, pl.R, pl.slots, 0);
         else k_finish<<<pl.g4, 256, s->finish_smem, cs>>>(D, k, pl.tchunks);
         if (D.dp) k_pressure<<<1, 256, 0, cs>>>(D, k);
         break;
     }
+}
+
+static int create_streams(ludvm_sim *s)
+{
+    if (s->cap_stream) return LUDVM_OK;
+    int lo = 0, hi = 0;
+    cudaDeviceGetStreamPriorityRange(&lo, &hi);   // lo = least, hi = greatest priority
+    CUDA_TRY(cudaStreamCreateWithPriority(&s->cap_stream, cudaStreamNonBlocking, hi));   // latency-critical branch
+    CUDA_TRY(cudaStreamCreateWithPriority(&s->cap_stream2, cudaStreamNonBlocking, lo));  // bulk old-wake convection
+    CUDA_TRY(cudaEventCreateWithFlags(&s->ev_fork, cudaEventDisableTiming));
+    CUDA_TRY(cudaEventCreateWithFlags(&s->ev_join, cudaEventDisableTiming));
+    return LUDVM_OK;
 }
 
 static int build_graph(ludvm_sim *s, int bracket, int ksteps, cudaGraphExec_t *out)
@@ -1926,14 +2004,8 @@ static int build_graph(ludvm_sim *s, int bracket, int ksteps, cudaGraphExec_t *o
     const SimDev &D = s->d;
     const StepPlan pl = plan_step(s, bracket);
     cudaGraph_t graph;
-    if (!s->cap_stream) {
-        int lo = 0, hi = 0;
-        cudaDeviceGetStreamPriorityRange(&lo, &hi);   // lo = least, hi = greatest priority
-        CUDA_TRY(cudaStreamCreateWithPriority(&s->cap_stream, cudaStreamNonBlocking, hi));   // latency-critical branch
-        CUDA_TRY(cudaStreamCreateWithPriority(&s->cap_stream2, cudaStreamNonBlocking, lo));  // bulk old-wake convection
-        CUDA_TRY(cudaEventCreateWithFlags(&s->ev_fork, cudaEventDisableTiming));
-        CUDA_TRY(cudaEventCreateWithFlags(&s->ev_join, cudaEventDisableTiming));
-    }
+    int rc = create_streams(s);
+    if (rc) return rc;
     cudaStream_t cs = s->cap_stream, cs2 = s->cap_stream2;
     CUDA_TRY(cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal));
     for (int k = 0; k < ksteps; k++) {
@@ -1959,6 +2031,74 @@ static int build_graph(ludvm_sim *s, int bracket, int ksteps, cudaGraphExec_t *o
     e = cudaGraphInstantiate(out, graph, 0);
     cudaGraphDestroy(graph);
     if (e != cudaSuccess) return set_error(LUDVM_E_CUDA, "graph instantiate failed: %s", cudaGetErrorString(e));
+    return LUDVM_OK;
+}
+
+// First step (0-based, as ludvm_sim::steps_enqueued) that the far field takes: the wake bound of step k alone,
+// 2 min(k + 1, nt - 1) + 2 + nfree (wake_upper over one step), reaches SIM_FAR_FIELD_MIN_WAKE.  It does not depend on
+// steps_per_graph or on how ludvm_sim_run is called, so neither changes which steps take which path.
+static long far_field_first_step(const ludvm_sim *s)
+{
+    long k = 0;
+    while (k < s->p.nt - 1 && 2 * std::min<long>(k + 1, s->p.nt - 1) + 2 + s->p.nfree < SIM_FAR_FIELD_MIN_WAKE) k++;
+    return k;
+}
+
+// One far-field step, enqueued from the host (the tree's depth comes from its bounding box, read back to the host, so
+// the step cannot be captured in a graph).  Forks from the context's stream onto the sim's two private streams and joins
+// back, so the work stays ordered with whatever else the context's stream carries.  `pl` is the plan the graph path
+// would use for this step: branch A, the join and, if the tree refuses the cloud, branch B are its kernels.
+static int far_field_step(ludvm_sim *s, const StepPlan &pl)
+{
+    ludvm_ctx *ctx = s->ctx;
+    const SimDev &D = s->d;
+    int rc = create_streams(s);
+    if (rc) return rc;
+    // nold = itev + ilev + nfree of step i = steps_enqueued + 1 (ilev_arr[i] is written by step i - 1's solve)
+    const long i = s->steps_enqueued + 1;
+    int ilev = 0;
+    CUDA_TRY(cudaMemcpyAsync(&ilev, D.ilev_arr + i, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    const long nold = (i - 1) + ilev + D.nfree;
+    cudaStream_t cs = s->cap_stream, cs2 = s->cap_stream2;
+    CUDA_TRY(cudaEventRecord(s->ev_fork, ctx->stream));
+    CUDA_TRY(cudaStreamWaitEvent(cs, s->ev_fork, 0));
+    CUDA_TRY(cudaStreamWaitEvent(cs2, s->ev_fork, 0));
+    // branch A first, so that it runs while the host waits for the tree's read-backs
+    enqueue_step_kernel(s, pl, 0, 0, cs);
+    enqueue_step_kernel(s, pl, 1, 0, cs);
+    double *xg = s->ff_xzg, *zg = xg + (2 * (size_t)D.nv + D.nfree), *gg = zg + (2 * (size_t)D.nv + D.nfree);
+    k_ff_gather<<<(int)std::min<long>((nold + 255) / 256, (long)ctx->sm_count * 8), 256, 0, cs2>>>(D, xg, zg, gg);
+    ctx->launches += 3;
+    // The tree's scratch (ctx slots SLOT_TREE_*) may be reallocated inside this call: scratch_reserve synchronises the
+    // context's stream before it frees, the tree has synchronised cs2 just before, and branch A on cs never touches
+    // those slots, so no stream can still be using the memory freed.
+    rc = tree_velocity_device(ctx, cs2, gg, xg, zg, D.vc4, nold, xg, zg, nold, s->ff_order, 0, D.pb_u, D.pb_w, nullptr);
+    int chunks = 1;
+    if (rc == LUDVM_E_UNSUPPORTED) {   // a leaf of the deepest tree would hold > 65 536 vortices: all pairs, as the graph
+        enqueue_step_kernel(s, pl, 2, 0, cs2);
+        ctx->launches++;
+        chunks = 0;
+        s->ff_fallback++;
+    } else if (rc) {
+        return rc;
+    } else {
+        k_ff_extra_rows<<<3, FF_EXTRA_THREADS, 0, cs2>>>(D, xg, zg, gg, (int)nold);
+        ctx->launches++;
+        s->ff_steps++;
+        s->ff_leaf_level = ctx->plan[2];
+    }
+    CUDA_TRY(cudaEventRecord(s->ev_join, cs));
+    CUDA_TRY(cudaStreamWaitEvent(ctx->stream, s->ev_join, 0));
+    CUDA_TRY(cudaEventRecord(s->ev_join, cs2));
+    CUDA_TRY(cudaStreamWaitEvent(ctx->stream, s->ev_join, 0));
+    enqueue_step_kernel(s, pl, 4, 0, ctx->stream);
+    k_finish_ov<<<pl.g4, 256, s->finish_smem, ctx->stream>>>(D, 0, pl.R, pl.slots, chunks);
+    if (D.dp) k_pressure<<<1, 256, 0, ctx->stream>>>(D, 0);
+    k_advance<<<1, 1, 0, ctx->stream>>>(D, 1);
+    ctx->launches += 3 + (D.dp ? 1 : 0);
+    CUDA_TRY(cudaGetLastError());
+    s->steps_enqueued++;
     return LUDVM_OK;
 }
 
@@ -2081,6 +2221,40 @@ LUDVM_API int ludvm_sim_enable_pressure(ludvm_sim *s)
     return LUDVM_OK;
 }
 
+LUDVM_API int ludvm_sim_enable_far_field(ludvm_sim *s, int order)
+{
+    ARG_CHECK(s != nullptr);
+    if (s->steps_enqueued > 0) return set_error(LUDVM_E_STATE, "ludvm_sim_enable_far_field must precede the first step");
+    if (s->p.mode == LUDVM_EXACT_F64)
+        return set_error(LUDVM_E_UNSUPPORTED, "the far field is an approximation; exact mode keeps numpy's sums bit for bit");
+    if (s->p.method == LUDVM_METHOD_RAMESH)
+        return set_error(LUDVM_E_UNSUPPORTED, "method='Ramesh' runs on the one-CTA driver, which has no far-field step");
+    if (s->p.P > 256)
+        return set_error(LUDVM_E_UNSUPPORTED, "P = %ld: the far-field step builds on the overlapped step, which needs P <= 256",
+                         (long)s->p.P);
+    if (order < 2 || order > TR_MAX_ORDER)
+        return set_error(LUDVM_E_ARG, "far-field order %d outside 2..%d", order, TR_MAX_ORDER);
+    DeviceGuard g(s->ctx->device);
+    if (!s->ff_xzg) {
+        void *p;
+        int rc = dev_malloc(s->ctx, s->allocs, 3 * (2 * (size_t)s->d.nv + s->d.nfree) * sizeof(double), &p);
+        if (rc) return rc;
+        s->ff_xzg = (double *)p;
+    }
+    s->ff_order = order;
+    return LUDVM_OK;
+}
+
+LUDVM_API int ludvm_sim_far_field_info(ludvm_sim *s, int64_t out[4])
+{
+    ARG_CHECK(s != nullptr && out != nullptr);
+    out[0] = s->ff_steps;
+    out[1] = s->ff_fallback;
+    out[2] = s->ff_order;
+    out[3] = s->ff_leaf_level;
+    return LUDVM_OK;
+}
+
 LUDVM_API int ludvm_sim_run(ludvm_sim *s, long nsteps)
 {
     ARG_CHECK(s != nullptr && nsteps >= 0);
@@ -2137,10 +2311,22 @@ LUDVM_API int ludvm_sim_run(ludvm_sim *s, long nsteps)
             todo -= k;
         }
     }
-    // graphs of K unrolled steps (a shorter one for a tail), cached per (wake-size bracket, length)
+    // graphs of K unrolled steps (a shorter one for a tail), cached per (wake-size bracket, length).  With the far field
+    // enabled, the steps from far_field_first_step on are far-field steps, each with the plan of the graph it stands in for.
+    const long ff_first = s->ff_order ? far_field_first_step(s) : total;
     while (todo > 0) {
         int k = (int)std::min<long>(s->K, todo);
         int b = bracket_of(wake_upper(s, s->steps_enqueued));
+        if (s->steps_enqueued >= ff_first) {
+            const StepPlan pl = plan_step(s, b);
+            for (int j = 0; j < k; j++) {
+                int rc = far_field_step(s, pl);
+                if (rc) return rc;
+            }
+            todo -= k;
+            continue;
+        }
+        k = (int)std::min<long>(k, ff_first - s->steps_enqueued);
         int key = b * 100000 + k;
         auto it = s->graphs.find(key);
         if (it == s->graphs.end()) {
@@ -2164,6 +2350,8 @@ LUDVM_API int ludvm_sim_profile_steps(ludvm_sim *s, long nsteps, double *ms_out)
     ARG_CHECK(s != nullptr && nsteps >= 0 && ms_out != nullptr);
     if (s->p.method == LUDVM_METHOD_RAMESH)
         return set_error(LUDVM_E_UNSUPPORTED, "method='Ramesh' runs as one persistent CTA; there are no phases to time");
+    if (s->ff_order)
+        return set_error(LUDVM_E_UNSUPPORTED, "the far-field step is not one of the graph path's phases; time ludvm_sim_run");
     DeviceGuard g(s->ctx->device);
     for (int q = 0; q < 5; q++) ms_out[q] = 0.0;
     long total = s->p.nt - 1;

@@ -20,8 +20,8 @@
 // Measured error of the representation (scripts/tree_proto.py,
 // numpy model of this file): order 12 -> 2e-11, 16 -> 5e-14, 18 -> 3e-15 of sum |terms|.
 //
-// Everything runs on the context's stream; the only host round trip is the bounding box (32 bytes), which fixes the
-// tree depth.  The order of every sum is fixed (cells sorted by original index, lists walked in slot order), so results
+// Everything runs on one stream (the context's, or the stream a caller such as the time loop's far-field step passes);
+// the host round trips are the bounding box (32 bytes), which fixes the tree depth, and the largest leaf population.  The order of every sum is fixed (cells sorted by original index, lists walked in slot order), so results
 // are bitwise reproducible from run to run and independent of how the target rows are sharded over GPUs.
 #include "common.cuh"
 
@@ -30,7 +30,6 @@
 
 namespace ludvm {
 
-#define TR_MAX_ORDER 24
 #define TR_MAX_P1 (TR_MAX_ORDER + 1)
 #define TR_MAX_LEVEL 10
 #define TR_MAX_SLOTS (9 + 36 * (TR_MAX_LEVEL - 1))
@@ -1144,18 +1143,14 @@ static size_t tree_layout(Arena &a, TreeBufs &b, long nw, long np, int L, int P2
     return a.off;
 }
 
-// Velocities of (gamma, xw, zw)[nw] at (xp, zp)[np], device pointers.  stats (host, nullable): [0] leaf level L,
-// [1] leaf side, [2] pair evaluations, [3] np * nw, [4] proxies per cell, [5] arena bytes; reading [2] synchronises.
-static int tree_velocity_device(ludvm_ctx *ctx, const double *g, const double *xw, const double *zw, double vc4, long nw,
-                                const double *xp, const double *zp, long np_, int order, int leaf, double *u, double *w,
-                                double *stats, double tdens = 0.0, const double *box_x = nullptr, const double *box_z = nullptr,
-                                int nbox = 0)
+int tree_velocity_device(ludvm_ctx *ctx, cudaStream_t st, const double *g, const double *xw, const double *zw, double vc4,
+                         long nw, const double *xp, const double *zp, long np_, int order, int leaf, double *u, double *w,
+                         double *stats, double tdens, const double *box_x, const double *box_z, int nbox)
 {
     // (box_x, box_z)[nbox]: points that span the targets' bounding box, used for it in place of the targets themselves --
     // a slab of a grid passes the full grid's corners, so that every slab builds the tree of the full grid
     if (order <= 0) order = 18;
     if (order < 2 || order > TR_MAX_ORDER) return set_error(LUDVM_E_ARG, "tree order %d outside 2..%d", order, TR_MAX_ORDER);
-    cudaStream_t st = ctx->stream;
     void *p;
     int rc;
     if ((rc = scratch_reserve(ctx, SLOT_TREE_COUNTERS, 256, &p))) return rc;
@@ -1333,7 +1328,7 @@ LUDVM_API int ludvm_induced_velocity_tree(ludvm_ctx *ctx, const double *gamma, c
         CUDA_TRY(cudaMemsetAsync(du, 0, (size_t)np_ * sizeof(double), ctx->stream));
         CUDA_TRY(cudaMemsetAsync(dw, 0, (size_t)np_ * sizeof(double), ctx->stream));
         if (stats) memset(stats, 0, 8 * sizeof(double));
-    } else if ((rc = tree_velocity_device(ctx, dg, dxw, dzw, vc4, nw, dxp, dzp, np_, order, leaf, du, dw, stats))) {
+    } else if ((rc = tree_velocity_device(ctx, ctx->stream, dg, dxw, dzw, vc4, nw, dxp, dzp, np_, order, leaf, du, dw, stats))) {
         return rc;
     }
     return host ? copy_back(ctx, {{u, np_, &du}, {w, np_, &dw}}) : LUDVM_OK;
@@ -1356,7 +1351,7 @@ LUDVM_API int ludvm_selfconv_step_tree(ludvm_ctx *ctx, const double *gamma, cons
         du = (double *)o;
         dw = du + nrows;
     }
-    if ((rc = tree_velocity_device(ctx, gamma, x, z, vc4, n, x + row0, z + row0, nrows, order, leaf, du, dw, stats))) return rc;
+    if ((rc = tree_velocity_device(ctx, ctx->stream, gamma, x, z, vc4, n, x + row0, z + row0, nrows, order, leaf, du, dw, stats))) return rc;
     k_tree_euler<<<ceil_div(nrows, 256), 256, 0, ctx->stream>>>(x + row0, z + row0, du, dw, dt, (int)nrows, x_out + row0,
                                                                 z_out + row0);
     ctx->launches++;
@@ -1405,7 +1400,7 @@ LUDVM_API int ludvm_flowfield_velocity_tree(ludvm_ctx *ctx, const double *ga, co
     double *xp = (double *)tp, *zp = xp + npts, *box = zp + npts;
     k_tree_grid_points<<<ceil_div(npts, 256), 256, 0, ctx->stream>>>(dx1, (int)nx, dz1, (int)nz, (int)row0, npts, xp, zp, box);
     ctx->launches++;
-    if ((rc = tree_velocity_device(ctx, dga, dxa, dza, vc4, na, xp, zp, npts, order, leaf, du, dw, stats, tgt_density, box, box + 2, 2)))
+    if ((rc = tree_velocity_device(ctx, ctx->stream, dga, dxa, dza, vc4, na, xp, zp, npts, order, leaf, du, dw, stats, tgt_density, box, box + 2, 2)))
         return rc;
     return host ? copy_back(ctx, {{u, npts, &du}, {w, npts, &dw}}) : LUDVM_OK;
 }

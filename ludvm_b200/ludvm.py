@@ -10,7 +10,7 @@ What runs on the GPU through the C ABI: `induced_velocity` (LUDVM.py:549), `airf
 Extra keyword-only arguments (not in the reference): `mode` ('exact' bit-reproduces numpy, 'fast' uses FMA
 arithmetic), `device`, `store_history`, `motion`, `run`, `steps_per_graph`, `pressure` (True: `time_loop` fills the
 chordwise pressure jump `dp` [nt, Npoints-1] and so `Cp`, which the reference allocates but leaves zero; see
-`time_loop`).
+`time_loop`), `far_field_order` (fast mode: convect large wakes through the treecode far field; see `time_loop`).
 """
 import ctypes as C
 import timeit
@@ -60,7 +60,7 @@ class LUDVM:
                  LESPcrit=0.2, Naca='0012', foil_filename=None, G=1, T=2, alpha_m=0, alpha_max=10,
                  k=0.2 * np.pi, phi=90, h_max=1, verbose=True, method='Faure',
                  circulation_freevort=None, xy_freevort=None, *, mode='exact', device=0, store_history=True,
-                 motion='cos', run=True, steps_per_graph=0, ctx=None, pressure=False):
+                 motion='cos', run=True, steps_per_graph=0, ctx=None, pressure=False, far_field_order=None):
         # LUDVM.py:237-260
         self.t0, self.tf, self.dt = t0, tf, dt
         self.chord, self.rho, self.Uinf = chord, rho, Uinf
@@ -95,6 +95,19 @@ class LUDVM:
             raise ValueError('store_history must be >= 0')
         self.steps_per_graph = int(steps_per_graph)
         self.pressure = bool(pressure)
+        # far_field_order=p (2..24, 18 documented): time_loop convects large wakes through the treecode (see time_loop)
+        if far_field_order is not None:
+            if mode == 'exact':
+                raise ValueError("far_field_order needs mode='fast': exact mode reproduces numpy's sums bit for bit")
+            if method == 'Ramesh':
+                raise ValueError("far_field_order is not available for method='Ramesh' (one-CTA driver)")
+            if Npoints > 257:
+                raise ValueError("far_field_order supports Npoints <= 257 (the overlapped step needs at most 256 panels)")
+            if isinstance(far_field_order, bool) or int(far_field_order) != far_field_order or not 2 <= far_field_order <= 24:
+                raise ValueError("far_field_order must be an integer in 2..24 (18: the all-pairs fast kernel's accuracy)")
+            far_field_order = int(far_field_order)
+        self.far_field_order = far_field_order
+        self.far_field_info = None
         self._ctx = ctx
         self._sim = None
 
@@ -276,7 +289,13 @@ class LUDVM:
             dp[i] = rho * ((Uinf*cos(alpha[i]) + h_dot[i]*sin(alpha[i]) + u) * gamma_airfoil[i-1]
                            + (Gamma_airfoil[i-1] - Gamma_airfoil[i-2]) / dt)
         where u is the tangential wake velocity at the gamma points that the normal force integrates
-        (LUDVM.py:1049-1057); at i = 1 the Gamma_airfoil[i-2] term is 0."""
+        (LUDVM.py:1049-1057); at i = 1 the Gamma_airfoil[i-2] term is 0.
+
+        With `far_field_order=p` the steps whose wake bound 2*i + 2 + n_freevort reaches the library's all-pairs /
+        far-field crossover (DESIGN.md 4b) convect the old wake through the treecode of `ops.induced_velocity_tree` at
+        order p instead of all pairs (about 1e-15 of sum|terms| at p = 18); a cloud too clustered for the tree falls back
+        to all pairs for that step.  The run is bitwise reproducible but not bit-equal to the all-pairs run.  Afterwards
+        `self.far_field_info` = dict(far_field_steps, fallback_steps, order, leaf_level) (leaf level of the last tree)."""
         if BCcheck and not (self.store_history == 1 and nsteps is None):
             raise ValueError("BCcheck=True is evaluated from the full vortex-path history (store_history=True, whole run)")
         tb = tables if tables is not None else self.step_tables()
@@ -307,6 +326,8 @@ class LUDVM:
         self._sim = sim
         if self.pressure:
             check(L.ludvm_sim_enable_pressure(sim))
+        if self.far_field_order is not None:
+            check(L.ludvm_sim_enable_far_field(sim, self.far_field_order))
         total = nv if nsteps is None else min(int(nsteps), nv)
         K = self.steps_per_graph if self.steps_per_graph > 0 else 50
         chunk = max(K, (max(print_dt, 1) // K) * K) if self.verbose else total
@@ -319,6 +340,10 @@ class LUDVM:
                 self.ctx.synchronize()
                 print('Step {} out of {}. Elapsed time {}'.format(done, nv, timeit.default_timer() - self.start_time))
         self._fetch_results(nt, P, Nc, nf, nv)
+        if self.far_field_order is not None:
+            info = (C.c_int64 * 4)()
+            check(L.ludvm_sim_far_field_info(sim, info))
+            self.far_field_info = dict(far_field_steps=info[0], fallback_steps=info[1], order=info[2], leaf_level=info[3])
         if BCcheck:
             self.BC = self._bc_check()
         return None
