@@ -17,8 +17,8 @@
 // field at their own Chebyshev points (M2L / L2L / L2P, see "evaluation" below), so that a far list acts on P2 points per
 // cell instead of on every target: the black-box FMM of Fong & Darve with this file's proxies; between two cells that both
 // carry proxies that action is a fixed matrix per level and offset, applied on the FP64 tensor cores (k_tree_m2l_dmma).
-// Measured error of the representation (scripts/tree_proto.py,
-// numpy model of this file): order 12 -> 2e-11, 16 -> 5e-14, 18 -> 3e-15 of sum |terms|.
+// Measured error of the representation (oracle/tree_model.py,
+// float64 numpy model of this file): order 12 -> 2e-11, 16 -> 5e-14, 18 -> 3e-15 of sum |terms|.
 //
 // Everything runs on one stream (the context's, or the stream a caller such as the time loop's far-field step passes);
 // the host round trips are the bounding box (32 bytes), which fixes the tree depth, and the largest leaf population.  The order of every sum is fixed (cells sorted by original index, lists walked in slot order), so results

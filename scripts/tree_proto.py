@@ -1,154 +1,23 @@
-"""numpy model of the far-field treecode of csrc/tree.cu (same tree, same lists, same nested Chebyshev proxies), used to
-choose the order / leaf size and to check the algorithm against direct summation before the CUDA version existed.
+"""Command line over oracle/tree_model.py, the float64 numpy model of the far field of csrc/tree.cu: the error of one
+order and leaf size against direct summation on a uniform cloud, and the pairs the tree evaluates.
 Usage: python scripts/tree_proto.py [N] [order] [leaf]"""
+import math
+import os
 import sys
+
 import numpy as np
 
-
-def nodes(p):
-    k = np.arange(p + 1)
-    s = np.sin(np.pi * (p - 2 * k) / (2 * p))          # Chebyshev-Lobatto points, exactly antisymmetric, s[p/2] = 0
-    w = (-1.0) ** k
-    w[0] *= 0.5
-    w[-1] *= 0.5
-    return s, w
-
-
-def basis(s, w, xi):
-    d = xi[:, None] - s[None, :]
-    hit = d == 0.0
-    d[hit] = 1.0
-    t = w[None, :] / d
-    L = t / t.sum(1)[:, None]
-    rows = hit.any(1)
-    L[rows] = hit[rows].astype(float)
-    return L
-
-
-def direct(xt, zt, xs, zs, g, vc4):
-    u, w = np.zeros(len(xt)), np.zeros(len(xt))
-    for i0 in range(0, len(xt), 256):
-        dx = xt[i0:i0 + 256, None] - xs[None, :]
-        dz = zt[i0:i0 + 256, None] - zs[None, :]
-        r2 = dx * dx + dz * dz
-        q = g[None, :] / np.sqrt(r2 * r2 + vc4)
-        u[i0:i0 + 256] = (q * dz).sum(1)
-        w[i0:i0 + 256] = -(q * dx).sum(1)
-    return u, w
-
-
-def morton(ix, iz):
-    def spread(v):
-        v = v.astype(np.int64)
-        v = (v | (v << 8)) & 0x00FF00FF
-        v = (v | (v << 4)) & 0x0F0F0F0F
-        v = (v | (v << 2)) & 0x33333333
-        v = (v | (v << 1)) & 0x55555555
-        return v
-    return spread(ix) | (spread(iz) << 1)
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+from oracle import tree_model  # noqa: E402
+from oracle.tree_model import direct  # noqa: E402,F401  (sum of g / sqrt(r^4 + vc^4) terms, circulations as given)
 
 
 def tree_velocity(g, xs, zs, xt, zt, vc4, p=18, leaf=256, L=None):
-    s, wb = nodes(p)
-    P2 = (p + 1) ** 2
-    x0, z0 = min(xs.min(), xt.min()), min(zs.min(), zt.min())
-    side = max(max(xs.max(), xt.max()) - x0, max(zs.max(), zt.max()) - z0) * (1 + 1e-12) + 1e-300
-    if L is None:
-        area = max((xs.max() - xs.min()) * (zs.max() - zs.min()), 1e-300)
-        a0 = np.sqrt(leaf * area / len(xs))
-        L = int(np.clip(np.round(np.log2(side / a0)), 2, 10))
-    nc = 1 << L
-    a = side / nc
-
-    def keys(x, z):
-        ix = np.minimum((x - x0) / a, nc - 1).astype(np.int64)
-        iz = np.minimum((z - z0) / a, nc - 1).astype(np.int64)
-        return morton(ix, iz)
-    ks, kt = keys(xs, zs), keys(xt, zt)
-    ps, pt = np.argsort(ks, kind="stable"), np.argsort(kt, kind="stable")
-    xs_, zs_, g_ = xs[ps], zs[ps], g[ps]
-    xt_, zt_ = xt[pt], zt[pt]
-    startS = np.searchsorted(ks[ps], np.arange(4 ** L + 1))
-    startT = np.searchsorted(kt[pt], np.arange(4 ** L + 1))
-
-    def rng(l, c):          # particle range of cell c at level l
-        sh = 2 * (L - l)
-        return startS[c << sh], startS[(c + 1) << sh]
-
-    def decode(c):
-        ix = iz = 0
-        for b in range(16):
-            ix |= ((c >> (2 * b)) & 1) << b
-            iz |= ((c >> (2 * b + 1)) & 1) << b
-        return ix, iz
-
-    # upward pass: proxies of every cell with more than P2 particles
-    qhat = {}
-    for l in range(L, 1, -1):
-        h = side / (1 << l) / 2
-        for c in range(4 ** l):
-            b, e = rng(l, c)
-            if e - b <= P2:
-                continue
-            ix, iz = decode(c)
-            cx, cz = x0 + (2 * ix + 1) * h, z0 + (2 * iz + 1) * h
-            if l == L:
-                xi, ze, gg = (xs_[b:e] - cx) / h, (zs_[b:e] - cz) / h, g_[b:e]
-            else:
-                xi, ze, gg = [], [], []
-                for ch in range(4):
-                    cc = 4 * c + ch
-                    cb, ce = rng(l + 1, cc)
-                    ox, oz = (ch & 1) * 2 - 1, (ch >> 1) * 2 - 1
-                    if (l + 1, cc) in qhat:
-                        S1, S2 = np.meshgrid(s, s, indexing="ij")
-                        xi.append(((S1 + ox) * 0.5).ravel()); ze.append(((S2 + oz) * 0.5).ravel()); gg.append(qhat[(l + 1, cc)])
-                    elif ce > cb:
-                        xi.append((xs_[cb:ce] - cx) / h); ze.append((zs_[cb:ce] - cz) / h); gg.append(g_[cb:ce])
-                xi, ze, gg = np.concatenate(xi), np.concatenate(ze), np.concatenate(gg)
-            Lx, Lz = basis(s, wb, xi), basis(s, wb, ze)
-            qhat[(l, c)] = np.einsum("j,ja,jb->ab", gg, Lx, Lz).ravel()
-
-    u, w = np.zeros(len(xt)), np.zeros(len(xt))
-    pairs = 0
-    S1, S2 = np.meshgrid(s, s, indexing="ij")
-    for c in np.nonzero(startT[1:] > startT[:-1])[0]:
-        tb, te = startT[c], startT[c + 1]
-        ix, iz = decode(int(c))
-        sx, sz, sg = [], [], []
-        for dz_ in (-1, 0, 1):
-            for dx_ in (-1, 0, 1):
-                jx, jz = ix + dx_, iz + dz_
-                if 0 <= jx < nc and 0 <= jz < nc:
-                    b, e = rng(L, int(morton(np.array(jx), np.array(jz))))
-                    sx.append(xs_[b:e]); sz.append(zs_[b:e]); sg.append(g_[b:e])
-        for l in range(2, L + 1):
-            cxl, czl = ix >> (L - l), iz >> (L - l)
-            px, pz = cxl >> 1, czl >> 1
-            h = side / (1 << l) / 2
-            for pdz in (-1, 0, 1):
-                for pdx in (-1, 0, 1):
-                    qx, qz = px + pdx, pz + pdz
-                    if not (0 <= qx < (1 << (l - 1)) and 0 <= qz < (1 << (l - 1))):
-                        continue
-                    for ch in range(4):
-                        jx, jz = 2 * qx + (ch & 1), 2 * qz + (ch >> 1)
-                        if max(abs(jx - cxl), abs(jz - czl)) <= 1:
-                            continue
-                        cc = int(morton(np.array(jx), np.array(jz)))
-                        b, e = rng(l, cc)
-                        if e == b:
-                            continue
-                        if (l, cc) in qhat:
-                            sx.append((x0 + (2 * jx + 1) * h + h * S1).ravel()); sz.append((z0 + (2 * jz + 1) * h + h * S2).ravel())
-                            sg.append(qhat[(l, cc)])
-                        else:
-                            sx.append(xs_[b:e]); sz.append(zs_[b:e]); sg.append(g_[b:e])
-        sx, sz, sg = np.concatenate(sx), np.concatenate(sz), np.concatenate(sg)
-        pairs += (te - tb) * len(sx)
-        uu, ww = direct(xt_[tb:te], zt_[tb:te], sx, sz, sg, vc4)
-        u[pt[tb:te]], w[pt[tb:te]] = uu, ww
-    return u, w, dict(L=L, pairs=pairs, proxy_cells=len(qhat))
+    """The model's velocity at order p on this script's scale, that of direct(..., g, ...): circulations without the
+    1 / (2 pi).  Returns u, w and dict(L, pairs, proxy_cells = number of cells with proxies over all levels)."""
+    u, w, info = tree_model.tree_velocity(g, xs, zs, xt, zt, vc4, order=p, leaf=leaf, L=L)
+    return (2.0 * math.pi) * u, (2.0 * math.pi) * w, dict(L=info["L"], pairs=info["pairs"],
+                                                          proxy_cells=sum(info["proxy_cells"].values()))
 
 
 if __name__ == "__main__":

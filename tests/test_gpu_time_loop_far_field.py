@@ -1,6 +1,6 @@
-"""GPU tests of the far-field convection in the device time loop (LUDVM(..., far_field_order=18), fast mode).  The clouds
+"""GPU tests of the far-field convection in the device time loop (LUDVM(..., far_field_order=p), fast mode).  The clouds
 are at least the library's all-pairs / far-field crossover (SIM_FAR_FIELD_MIN_WAKE), so every step takes the far-field
-step; far_field_info confirms it."""
+step, except in the test of a run that crosses it; far_field_info confirms it."""
 import ctypes
 
 import numpy as np
@@ -133,3 +133,67 @@ def test_enable_far_field_state_checks():
     assert L.ludvm_sim_enable_far_field(s._sim, 0) == E_STATE
     s.close()
     e.close()
+
+
+def _sum_abs_terms(g, x, z, vc4):
+    """sum_j |Gamma_j| |K_ij| over the cloud at each of its points, |K| = r / (2 pi sqrt(r^4 + vc^4)), on the GPU."""
+    import torch
+    t = lambda v: torch.tensor(np.ascontiguousarray(v), dtype=torch.float64, device="cuda")
+    tx, tz, tg = t(x), t(z), t(np.abs(g))
+    out = np.empty(len(x))
+    for r in range(0, len(x), 2048):
+        r2 = (tx[r:r + 2048, None] - tx[None, :]) ** 2 + (tz[r:r + 2048, None] - tz[None, :]) ** 2
+        out[r:r + 2048] = (tg[None, :] * torch.sqrt(r2) / (2 * np.pi * torch.sqrt(r2 * r2 + vc4))).sum(1).cpu().numpy()
+    return out
+
+
+@pytest.mark.parametrize("order", [5, 20, 24])
+def test_one_far_field_step_matches_the_model(order):
+    """A one-step loop at orders other than 18.  Step 1 convects FREE alone through the tree and everything else in it
+    is the all-pairs run's arithmetic on the same state, so (FREE_ff[1] - FREE_ap[1]) / dt is the tree's velocity minus
+    the all-pairs velocity: it must equal oracle/tree_model.py's minus the exact all-pairs sum, to the tree's rounding
+    (test_gpu_tree_orders.TOL of sum |terms|) plus the rounding of the positions."""
+    from ludvm_b200 import LUDVM, ops
+    from oracle import tree_model
+    from test_gpu_tree_orders import TOL
+    kw = dict(KW, tf=KW["dt"], **gust(NF), verbose=False, mode="fast")
+    a = LUDVM(**kw)
+    f = LUDVM(**kw, far_field_order=order)
+    info = f.far_field_info
+    assert info["far_field_steps"] == 1 and info["fallback_steps"] == 0 and info["order"] == order, info
+    g = np.asarray(kw["circulation_freevort"], dtype=np.float64)
+    x0, z0 = a.path["FREE"][0]
+    assert biteq(f.path["FREE"][0], a.path["FREE"][0])
+    vc4 = a.v_core ** 4
+    um, wm, st = tree_model.tree_velocity(g, x0, z0, x0, z0, vc4, order=order)
+    assert st["L"] == info["leaf_level"]
+    ua, wa = ops.induced_velocity(g, x0, z0, x0, z0, a.v_core, mode="exact")
+    d = (f.path["FREE"][1] - a.path["FREE"][1]) / a.dt
+    den = _sum_abs_terms(g, x0, z0, vc4)
+    pos = 4 * np.spacing(np.abs(a.path["FREE"][1])) / a.dt
+    err = np.abs(d - np.stack([um - ua, wm - wa]))
+    assert np.all(err <= TOL * den + pos), float(np.max((err - pos) / den))
+
+
+def test_far_field_from_the_step_whose_wake_crosses_the_threshold():
+    """nfree = 65526: the wake bounds of steps 0-2 (65530, 65532, 65534) are below SIM_FAR_FIELD_MIN_WAKE, steps 3-5 take
+    the far field.  The first three steps are the run without the option bit for bit, and graph chunks of 2 or 7 steps,
+    which ludvm_sim_run cuts at the first far-field step, change nothing."""
+    from ludvm_b200 import LUDVM
+    kw = dict(KW, **gust(65526), verbose=False, mode="fast")
+    a = LUDVM(**kw)
+    f = LUDVM(**kw, far_field_order=20)
+    assert f.nt == 7
+    assert f.far_field_info["far_field_steps"] == 3 and f.far_field_info["fallback_steps"] == 0, f.far_field_info
+    for k in ("L", "D", "M", "LESP", "LEV_shed", "fourier"):
+        assert biteq(getattr(f, k)[:4], getattr(a, k)[:4]), k
+    for k in ("FREE", "TEV", "LEV"):
+        assert biteq(f.path[k][:4], a.path[k][:4]), k
+    assert not biteq(f.path["FREE"][4], a.path["FREE"][4])
+    for K in (2, 7):
+        c = LUDVM(**kw, far_field_order=20, steps_per_graph=K)
+        assert c.far_field_info == f.far_field_info
+        for k in ("L", "D", "M", "LESP", "LEV_shed", "fourier"):
+            assert biteq(getattr(c, k), getattr(f, k)), (K, k)
+        for k in ("FREE", "TEV", "LEV"):
+            assert biteq(c.path[k], f.path[k]), (K, k)
