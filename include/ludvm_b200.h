@@ -221,7 +221,7 @@ int ludvm_sim_create(ludvm_ctx *ctx, const ludvm_sim_params *p, const ludvm_sim_
 int ludvm_sim_run(ludvm_sim *sim, long nsteps);
 /* Steps completed so far (synchronises). */
 int ludvm_sim_steps_done(ludvm_sim *sim, long *out);
-/* Diagnostic twin of ludvm_sim_run (method Faure): advances `nsteps` steps launching the step's kernels one by one
+/* Diagnostic twin of ludvm_sim_run (either method): advances `nsteps` steps launching the step's kernels one by one
  * with CUDA events around each.  ms_out[0..3] = summed milliseconds of wake-on-foil, solve, convection partials,
  * finish; ms_out[4] = their total.  Synchronises. */
 int ludvm_sim_profile_steps(ludvm_sim *sim, long nsteps, double *ms_out);

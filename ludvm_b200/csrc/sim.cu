@@ -29,8 +29,9 @@
 //                    old wake's self-convection through the treecode (tree.cu), enqueued step by step from the host.
 //   * CTA path    -- k_sim_cta: one persistent CTA runs ALL steps of one case with __syncthreads() between phases;
 //                    cases are pulled from an atomic counter.  Used for batched parameter sweeps (config 4: 4096
-//                    independent cases, no collective) and for method='Ramesh', whose Newton loops have a
-//                    data-dependent trip count.
+//                    independent cases, no collective).
+// Both methods take the coop and graph paths.  method='Ramesh' differs only in the solve (its Newton loops run on the
+// solve CTA, grid_downwash) and, in exact mode, in phase 1, which evaluates the step's Newton wake instead of the old one.
 // The once-per-step scalar reductions live in block_reduce.cuh.  -DLUDVM_TRACE adds clock64 phase traces (scripts/
 // solve_trace.py); it is off in the shipped library.
 #include <algorithm>
@@ -45,7 +46,6 @@ namespace ludvm {
 #define SIM_DMAX 11          // at most 2^11 tree nodes per row are evaluated by separate warps
 #define SOLVE_THREADS 256
 #define CTA_THREADS 256
-#define RAMESH_THREADS 1024
 #define PI_D 3.141592653589793
 #define SIM_TILED_MIN_WAKE 2048   // fast mode: wakes at least this large use the tiled convection kernel (measured: 8192 -> 5.48 s,
                                   // 4096 -> 5.31 s, 2048 -> 5.30 s, 1024 -> 5.29 s for the 20 000-step dt = 2e-3 run)
@@ -143,6 +143,23 @@ __host__ __device__ __forceinline__ int wof_fold(int mode, int n, int P, int tar
     if (single && mode != LUDVM_EXACT_F64) return 1;
     return mode == LUDVM_EXACT_F64 ? min(sim_depth(n, P, target_warps), SIM_WOF_MAX_DEPTH)
                                    : min(sim_chunks(n, P, target_warps), 1 << SIM_WOF_MAX_DEPTH);
+}
+
+// Node of numpy's pairwise tree over n elements, cut at depth d (pw_node's numbering), that holds logical element e.
+__device__ __forceinline__ int pw_node_of(int n, int d, int e)
+{
+    int b = 0;
+    for (int l = d - 1; l >= 0; l--) {
+        const int n2 = pw_left(n);
+        if (e >= n2) {
+            b |= 1 << l;
+            e -= n2;
+            n -= n2;
+        } else {
+            n = n2;
+        }
+    }
+    return b;
 }
 
 struct Step {
@@ -430,8 +447,65 @@ __device__ __noinline__ void cta_downwash(const SimDev &S, const StepTables &t, 
     __syncthreads();
 }
 
+// The same downwash on the grid drivers, whose phase 1 ran grid-wide before the solve; the wake is not summed again.
+// Between the Newton evaluations of a step only two elements of the wake change: logical itev (the TEV) and itev+1+ilev
+// (the LEV slot), in circulation, plus the LEV position set once before the 2-D loop.
+//   exact: phase 1 left the tree-node partials of the Newton wake TEV[:itev+1] ++ LEV[:ilev+1] ++ FREE (same cut and
+//          [node][P] layout as here).  The <= 2 nodes holding those elements are evaluated again over their slots, then
+//          folded.  A node's partial is a pure function of its range, so this is the full evaluation bit for bit.
+//   fast:  m.T1 / m.T2 hold the folded sums of the old wake TEV[:itev] ++ LEV[:ilev] ++ FREE (Faure's phase 1); the two
+//          new vortices' terms are added at each gamma point, in k_conv_new's order.
+__device__ __noinline__ void grid_downwash(const SimDev &S, const StepTables &t, const Step &st, const Kin &k,
+                                           const SolveSmem &m)
+{
+    __syncthreads();  // circulation guesses written by thread 0 are visible
+    const int P = S.P, itev = st.itev, lev = S.nv + st.ilev;
+    if (S.mode == LUDVM_EXACT_F64) {
+        const SrcView W = wake_view(S, itev + 1, st.ilev + 1);
+        const TgtGamma T{k.xa, k.za};
+        const int d = wof_fold(S.mode, W.n, P, S.target_warps);
+        const int b0 = pw_node_of(W.n, d, itev), b1 = pw_node_of(W.n, d, itev + 1 + st.ilev);
+        const int ng = (P + 3) >> 2, ntask = (b0 == b1 ? 1 : 2) * ng;
+        const Pool pl = block_pool();
+        const bool safe = range_safe(S);
+        for (int q = pl.wid; q < ntask; q += pl.nwarps) {
+            const long task = q < ng ? (long)b0 * ng + q : (long)b1 * ng + (q - ng);
+            if (safe) exact_rows_warp_task<1, false>(W, T, P, d, task, pl.lane, S.pa_u, S.pa_w);
+            else exact_rows_warp_task<1, true>(W, T, P, d, task, pl.lane, S.pa_u, S.pa_w);
+        }
+        fold_wake_on_foil(S, W.n, m);
+    } else {
+        const double xt = S.wx[itev], zt = S.wz[itev], gt = S.wg[itev] * LUDVM_INV_TWO_PI;
+        const double xl = S.wx[lev], zl = S.wz[lev], gl = S.wg[lev] * LUDVM_INV_TWO_PI;
+        for (int j = threadIdx.x; j < P; j += blockDim.x) {
+            double u = m.T1[j], w = m.T2[j];
+            pair_fast(k.xa[j], k.za[j], xt, zt, gt, S.vc4, u, w);
+            pair_fast(k.xa[j], k.za[j], xl, zl, gl, S.vc4, u, w);
+            m.u1[j] = u;
+            m.w1[j] = w;
+        }
+    }
+    for (int j = threadIdx.x; j < P; j += blockDim.x) {
+        double w = downwash_at(S, t, k, m.u1, m.w1, j);
+        m.W[j] = w;
+        m.Wu[j] = w / S.Uinf;
+    }
+    __syncthreads();
+}
+
+// Downwash of the Newton wake TEV[:itev+1] ++ LEV[:ilev+1] ++ FREE into W, Wu.
+template <bool GRID>
+__device__ __forceinline__ void newton_downwash(const SimDev &S, const StepTables &t, const Step &st, const Kin &k,
+                                                const SolveSmem &m)
+{
+    if (GRID) grid_downwash(S, t, st, k, m);
+    else cta_downwash(S, t, st, k, st.itev + 1, st.ilev + 1, m);
+}
+
 // Kelvin residual of the Newton loops (LUDVM.py:697-699, :825-827).  Leaves A0 in sc[20], A1 in sc[21], the bound
-// circulation in sc[24]; returns the residual on every thread.
+// circulation in sc[24]; returns the residual on every thread.  One copy per GRID (phase_solve): the sweep driver's copy
+// sees its descriptor in shared memory only, and keeps the code it had before the grid drivers called it.
+template <bool GRID>
 __device__ __noinline__ double cta_kelvin_f(const SimDev &S, const StepTables &t, const Step &st, const SolveSmem &m)
 {
     block_fourier(S, t, m, 0, 2, m.sc + 20);
@@ -452,7 +526,9 @@ __device__ __noinline__ double cta_kelvin_f(const SimDev &S, const StepTables &t
 // through another barrier.
 // ---------------------------------------------------------------------------------------------------
 // `tab` = shared memory of the StepTables (staged here when stage_now, else already resident), `sm` = scratch.
-template <int METHOD>
+// GRID (Ramesh): phase 1 ran grid-wide before this solve, so the Newton evaluations use grid_downwash; the one-CTA sweep
+// driver keeps cta_downwash.
+template <int METHOD, bool GRID = false>
 __device__ void phase_solve(const SimDev &S, const Step &st, double *tab, double *sm, const double *pre_sums,
                             bool stage_now)
 {
@@ -556,15 +632,22 @@ __device__ void phase_solve(const SimDev &S, const Step &st, double *tab, double
         }
         if (stage_now) tables_wait();
         __syncthreads();
+        if (GRID && S.mode != LUDVM_EXACT_F64) {   // the old wake's sums at the gamma points, fixed for the step
+            fold_wake_on_foil(S, itev + ilev + S.nfree, m);
+            for (int j = tid; j < P; j += nth) {
+                T1[j] = m.u1[j];
+                T2[j] = m.w1[j];
+            }
+        }
         int niter = 1;
         while (fabs(sc[26]) > S.maxerror && niter < S.maxiter) {
             double shed = sc[27];
             if (tid == 0) S.wg[itev] = shed;
-            cta_downwash(S, t, st, k, itev + 1, ilev + 1, m);
-            double f = cta_kelvin_f(S, t, st, m);
+            newton_downwash<GRID>(S, t, st, k, m);
+            double f = cta_kelvin_f<GRID>(S, t, st, m);
             if (tid == 0) S.wg[itev] = shed + S.epsilon;
-            cta_downwash(S, t, st, k, itev + 1, ilev + 1, m);
-            double fdelta = cta_kelvin_f(S, t, st, m);
+            newton_downwash<GRID>(S, t, st, k, m);
+            double fdelta = cta_kelvin_f<GRID>(S, t, st, m);
             if (tid == 0) {
                 double fprime = (fdelta - f) / S.epsilon;
                 sc[27] = shed - f / fprime;
@@ -574,7 +657,7 @@ __device__ void phase_solve(const SimDev &S, const Step &st, double *tab, double
             __syncthreads();
             niter++;
         }
-        cta_downwash(S, t, st, k, itev + 1, ilev + 1, m);
+        newton_downwash<GRID>(S, t, st, k, m);
         block_fourier(S, t, m, 0, Nc, A);
         for (int n = tid; n < Nc; n += nth) F[Nc + n] = (A[n] - Fprev[n]) / dt;
         if (tid == 0) {
@@ -644,17 +727,17 @@ __device__ void phase_solve(const SimDev &S, const Step &st, double *tab, double
             while ((fabs(sc[26]) > S.maxerror || fabs(sc[27]) > S.maxerror) && niter < S.maxiter) {
                 double tg = sc[28], lg = sc[29];
                 if (tid == 0) { S.wg[itev] = tg; S.wg[nv + ilev] = lg; }
-                cta_downwash(S, t, st, k, itev + 1, ilev + 1, m);
-                double f1 = cta_kelvin_f(S, t, st, m);
+                newton_downwash<GRID>(S, t, st, k, m);
+                double f1 = cta_kelvin_f<GRID>(S, t, st, m);
                 double cbound = sc[24], f2 = sc[15] - sc[20];
                 __syncthreads();
                 if (tid == 0) { S.wg[itev] = tg + S.epsilon; S.wg[nv + ilev] = lg; }
-                cta_downwash(S, t, st, k, itev + 1, ilev + 1, m);
-                double f1dT = cta_kelvin_f(S, t, st, m), f2dT = sc[15] - sc[20];
+                newton_downwash<GRID>(S, t, st, k, m);
+                double f1dT = cta_kelvin_f<GRID>(S, t, st, m), f2dT = sc[15] - sc[20];
                 __syncthreads();
                 if (tid == 0) { S.wg[itev] = tg; S.wg[nv + ilev] = lg + S.epsilon; }
-                cta_downwash(S, t, st, k, itev + 1, ilev + 1, m);
-                double f1dL = cta_kelvin_f(S, t, st, m), f2dL = sc[15] - sc[20];
+                newton_downwash<GRID>(S, t, st, k, m);
+                double f1dL = cta_kelvin_f<GRID>(S, t, st, m), f2dL = sc[15] - sc[20];
                 __syncthreads();
                 if (tid == 0) {
                     double eps = S.epsilon, x0, x1;
@@ -670,7 +753,7 @@ __device__ void phase_solve(const SimDev &S, const Step &st, double *tab, double
                 __syncthreads();
                 niter++;
             }
-            cta_downwash(S, t, st, k, itev + 1, ilev + 1, m);
+            newton_downwash<GRID>(S, t, st, k, m);
             block_fourier(S, t, m, 0, Nc, A);  // LUDVM.py:902-909
             if (tid == 0) {
                 sc[10] = S.wg[itev];
@@ -738,7 +821,7 @@ __device__ __forceinline__ void phase_gamma_cumsum(const SimDev &S, const Step &
 // again here with the same expression; row itev - 1 is complete.  Called after the loads, where little else is live
 // (inside the loads' loop, or out of line, it cost the kernels around it spills); on the graph path it is a kernel of its
 // own after k_finish / k_finish_ov (k_pressure), which keep their register allocation.  In the one-CTA driver
-// (single-simulation Ramesh and the DP sweep instantiations) it runs before that CTA's own phase_gamma_cumsum, so a
+// (the DP sweep instantiations) it runs before that CTA's own phase_gamma_cumsum, so a
 // compact sweep case, whose one Gamma row every step overwrites (af_stride = 0), still holds row itev - 1 in it here:
 // each thread reads Gprev[j] before the same thread (same j mapping) writes that element in phase_gamma_cumsum.
 __device__ __forceinline__ void pressure_row(const SimDev &S, const Step &st)
@@ -924,6 +1007,15 @@ __device__ __forceinline__ void phase_finish_update(const SimDev &S, const Step 
 // ---------------------------------------------------------------------------------------------------
 // graph path: four kernels per step
 // ---------------------------------------------------------------------------------------------------
+// Ramesh in exact mode: the partials of the step's Newton wake TEV[:itev+1] ++ LEV[:ilev+1] ++ FREE, whatever the two new
+// slots hold now (grid_downwash evaluates their nodes again); fast mode and Faure: the old wake TEV[:itev] ++ LEV[:ilev] ++ FREE.
+template <int METHOD>
+__device__ __forceinline__ int wof_extra(const SimDev &S)
+{
+    return (METHOD == LUDVM_METHOD_RAMESH && S.mode == LUDVM_EXACT_F64) ? 1 : 0;
+}
+
+template <int METHOD>
 __global__ void __launch_bounds__(256) k_wake_on_foil(SimDev S, int s)
 {
     Step st;
@@ -941,9 +1033,11 @@ __global__ void __launch_bounds__(256) k_wake_on_foil(SimDev S, int s)
     Pool pl = grid_pool();
     pl.nwarps -= blockDim.x >> 5;
     pl.nth -= blockDim.x;
-    phase_wake_on_foil(S, st, st.itev, st.ilev, pl);
+    phase_wake_on_foil(S, st, st.itev + wof_extra<METHOD>(S), st.ilev + wof_extra<METHOD>(S), pl);
 }
+template __global__ void k_wake_on_foil<LUDVM_METHOD_FAURE>(SimDev, int);   // emission order: see method_kernels
 
+template <int METHOD>
 __global__ void __launch_bounds__(SOLVE_THREADS) k_solve(SimDev S, int s)
 {
     extern __shared__ double sm[];
@@ -951,10 +1045,12 @@ __global__ void __launch_bounds__(SOLVE_THREADS) k_solve(SimDev S, int s)
     TRACE(20);
     if (!step_begin(S, s, st)) return;
     TRACE(21);
-    phase_solve<LUDVM_METHOD_FAURE>(S, st, sm, sm + TABLE_SMEM_DOUBLES(S.P, S.Nc, S.sinn_smem), S.pre_sums, true);
+    phase_solve<METHOD, METHOD == LUDVM_METHOD_RAMESH>(S, st, sm, sm + TABLE_SMEM_DOUBLES(S.P, S.Nc, S.sinn_smem),
+                                                       S.pre_sums, true);
     __syncthreads();
     TRACE(22);
 }
+template __global__ void k_solve<LUDVM_METHOD_FAURE>(SimDev, int);
 
 __global__ void __launch_bounds__(256) k_conv_partials(SimDev S, int s)
 {
@@ -1053,13 +1149,16 @@ struct TiledGeom {
     }
 };
 
+template <int METHOD>
 __global__ void __launch_bounds__(SOLVE_THREADS, 4) k_solve_small(SimDev S, int s)
 {
     extern __shared__ double sm[];
     Step st;
     if (!step_begin(S, s, st)) return;
-    phase_solve<LUDVM_METHOD_FAURE>(S, st, sm, sm + TABLE_SMEM_DOUBLES(S.P, S.Nc, S.sinn_smem), S.pre_sums, true);
+    phase_solve<METHOD, METHOD == LUDVM_METHOD_RAMESH>(S, st, sm, sm + TABLE_SMEM_DOUBLES(S.P, S.Nc, S.sinn_smem),
+                                                       S.pre_sums, true);
 }
+template __global__ void k_solve_small<LUDVM_METHOD_FAURE>(SimDev, int);
 
 template <int R>
 __global__ void __launch_bounds__(FT_THREADS, 2) k_conv_old_tiled(SimDev S, int s, int slots)
@@ -1339,7 +1438,7 @@ __device__ __forceinline__ void persist_barrier(unsigned long long *bar, unsigne
 // 256 threads per CTA on both paths: 512 threads halve the O(N^2) phases' rounds but cap the kernel at 128 registers and
 // slow the solve by ~3 us: README case 30.4 / 25.7 us per step (exact / fast) against 28.7 / 24.0 with 256
 // (profiles/r02s_coop_probe_1.txt).
-template <bool CLUSTER>
+template <bool CLUSTER, int METHOD>
 __global__ void __launch_bounds__(256, 1) k_sim_persist(SimDev S, int nsteps, unsigned long long *bar)
 {
     extern __shared__ double sm[];
@@ -1380,12 +1479,12 @@ __global__ void __launch_bounds__(256, 1) k_sim_persist(SimDev S, int nsteps, un
             Pool pl = grid_pool();
             pl.nwarps -= blockDim.x >> 5;
             pl.nth -= blockDim.x;
-            phase_wake_on_foil(S, st, st.itev, st.ilev, pl);
+            phase_wake_on_foil(S, st, st.itev + wof_extra<METHOD>(S), st.ilev + wof_extra<METHOD>(S), pl);
         }
         COOP_T(0);
         persist_barrier<CLUSTER>(bar, epoch, S.counters);
         COOP_T(1);
-        if (blockIdx.x == 0) phase_solve<LUDVM_METHOD_FAURE>(S, st, tab, scr, S.pre_sums, false);
+        if (blockIdx.x == 0) phase_solve<METHOD, METHOD == LUDVM_METHOD_RAMESH>(S, st, tab, scr, S.pre_sums, false);
         else if (i > first) deferred_tail(i - 1);
         COOP_T(2);
         persist_barrier<CLUSTER>(bar, epoch, S.counters);
@@ -1807,8 +1906,7 @@ struct ludvm_sim {
     ludvm_sim_params p{};
     SimDev d{};
     std::vector<void *> allocs;
-    SimDev *d_case = nullptr;  // device copy of `d` (CTA path)
-    int *d_next = nullptr;
+    SimDev *d_case = nullptr;  // device copy of `d` (k_case_init)
     long steps_enqueued = 0;
     int K = 50;
     std::map<int, cudaGraphExec_t> graphs;  // (bracket, length) -> instantiated graph
@@ -1897,6 +1995,15 @@ struct StepPlan {
     dim3 gte;
 };
 
+// The kernels of one method's step (the rest of the step does not depend on the method).
+struct MethodKernels {
+    void (*wake_on_foil)(SimDev, int);
+    void (*solve)(SimDev, int);
+    void (*solve_small)(SimDev, int);
+    const void *persist_coop, *persist_cluster;   // k_sim_persist<false / true, METHOD>
+};
+static const MethodKernels &method_kernels(int method);
+
 typedef void (*conv_old_fn)(SimDev, int, int);
 static conv_old_fn conv_old_kernel(int R)
 {
@@ -1964,12 +2071,10 @@ static StepPlan plan_step(const ludvm_sim *s, int bracket)
 static void enqueue_step_kernel(const ludvm_sim *s, const StepPlan &pl, int which, int k, cudaStream_t cs)
 {
     const SimDev &D = s->d;
+    const MethodKernels &mk = method_kernels(D.method);
     switch (which) {
-    case 0: k_wake_on_foil<<<pl.g1, 256, 0, cs>>>(D, k); break;
-    case 1:
-        if (pl.ov) k_solve_small<<<1, SOLVE_THREADS, s->solve_smem, cs>>>(D, k);
-        else k_solve<<<1, SOLVE_THREADS, s->solve_smem, cs>>>(D, k);
-        break;
+    case 0: mk.wake_on_foil<<<pl.g1, 256, 0, cs>>>(D, k); break;
+    case 1: (pl.ov ? mk.solve_small : mk.solve)<<<1, SOLVE_THREADS, s->solve_smem, cs>>>(D, k); break;
     case 2:
         if (pl.tiled_exact) k_conv_partials_exact_tiled<<<pl.gte, ET_THREADS, 0, cs>>>(D, k);
         else if (!pl.tiled) k_conv_partials<<<pl.g3, 256, 0, cs>>>(D, k);
@@ -2106,15 +2211,16 @@ static int set_smem_limits(size_t solve_smem, size_t finish_smem)
 {
     if (solve_smem > SOLVE_SMEM_LIMIT + 4096) return set_error(LUDVM_E_UNSUPPORTED, "Npoints too large for the solve kernel");
     if (solve_smem > 48 * 1024) {
-        CUDA_TRY(cudaFuncSetAttribute(k_solve, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
-        CUDA_TRY(cudaFuncSetAttribute(k_solve_small, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
+        for (int method : {LUDVM_METHOD_FAURE, LUDVM_METHOD_RAMESH}) {
+            CUDA_TRY(cudaFuncSetAttribute(method_kernels(method).solve, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
+            CUDA_TRY(cudaFuncSetAttribute(method_kernels(method).solve_small, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
+        }
         CUDA_TRY(cudaFuncSetAttribute(k_sim_cta<CTA_THREADS, LUDVM_METHOD_FAURE, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
         CUDA_TRY(cudaFuncSetAttribute(k_sim_cta<128, LUDVM_METHOD_FAURE, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
         CUDA_TRY(cudaFuncSetAttribute(k_sim_cta<CTA_THREADS, LUDVM_METHOD_RAMESH, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
         CUDA_TRY(cudaFuncSetAttribute(k_sim_cta<CTA_THREADS, LUDVM_METHOD_FAURE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
         CUDA_TRY(cudaFuncSetAttribute(k_sim_cta<128, LUDVM_METHOD_FAURE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
         CUDA_TRY(cudaFuncSetAttribute(k_sim_cta<CTA_THREADS, LUDVM_METHOD_RAMESH, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
-        CUDA_TRY(cudaFuncSetAttribute(k_sim_cta<RAMESH_THREADS, LUDVM_METHOD_RAMESH, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)solve_smem));
     }
     if (finish_smem > 48 * 1024)
         CUDA_TRY(cudaFuncSetAttribute(k_finish, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)finish_smem));
@@ -2138,14 +2244,13 @@ LUDVM_API int ludvm_sim_create(ludvm_ctx *ctx, const ludvm_sim_params *p, const 
 #define CU(x) do { cudaError_t e__ = (x); if (e__ != cudaSuccess) { ludvm_sim_destroy(s); return set_error(LUDVM_E_CUDA, "%s failed: %s", #x, cudaGetErrorString(e__)); } } while (0)
     DevTables dt{};
     TRY(upload_tables(ctx, s->allocs, *p, *t, &dt));
-    const bool cta = p->method == LUDVM_METHOD_RAMESH;  // Newton loops: the whole step runs in one CTA
     // exact mode splits the summation tree deeper: its large-wake convection kernel runs one 128-thread CTA per
     // (128 rows, tree node) and wants several waves of 4 CTAs/SM (the split depth never changes a result).  Measured on
     // the 20 000-step dt = 2e-3 run in exact mode: 96 x SMs 16.9 s, 192 x 15.1 s, 384 x 14.4 s.
-    const int target = cta ? 2 * (RAMESH_THREADS / 32) : ctx->sm_count * (p->mode == LUDVM_EXACT_F64 ? 384 : 48);
+    const int target = ctx->sm_count * (p->mode == LUDVM_EXACT_F64 ? 384 : 48);
     // shared-memory staging area of the block-wide folds / integrals: all Nc Fourier integrands, or 64 partials of
     // every (row, component), in one batch
-    const int sum_nodes = clamp_sum_nodes(p->P, p->Nc, std::max<long>(cta ? 1024 : 4096, std::max<long>(p->Nc * p->P, cta ? 0 : 2 * p->P * 65)));
+    const int sum_nodes = clamp_sum_nodes(p->P, p->Nc, std::max<long>(4096, std::max<long>(p->Nc * p->P, 2 * p->P * 65)));
     Arena measure;
     layout_case(s->d, *p, dt, measure, target, sum_nodes, false);
     void *base;
@@ -2155,9 +2260,8 @@ LUDVM_API int ludvm_sim_create(ludvm_ctx *ctx, const ludvm_sim_params *p, const 
     real.base = (char *)base;
     layout_case(s->d, *p, dt, real, target, sum_nodes, false);
     void *dc;
-    TRY(dev_malloc(ctx, s->allocs, sizeof(SimDev) + 1024, &dc));
+    TRY(dev_malloc(ctx, s->allocs, sizeof(SimDev), &dc));
     s->d_case = (SimDev *)dc;
-    s->d_next = (int *)((char *)dc + ((sizeof(SimDev) + 255) & ~(size_t)255));
     {
         void *db;
         TRY(dev_malloc(ctx, s->allocs, COOP_BAR_WORDS * sizeof(unsigned long long), &db));
@@ -2172,14 +2276,15 @@ LUDVM_API int ludvm_sim_create(ludvm_ctx *ctx, const ludvm_sim_params *p, const 
     {   // cooperative path: needs cooperative-launch support and one resident CTA per SM
         int coop = 0, per_sm = 0;
         cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, ctx->device);
-        if (coop && !cta && cudaFuncSetAttribute(k_sim_persist<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s->solve_smem) == cudaSuccess &&
-            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sim_persist<false>, 256, s->solve_smem) == cudaSuccess && per_sm >= 1)
+        const void *kcoop = method_kernels(p->method).persist_coop;
+        if (coop && cudaFuncSetAttribute(kcoop, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s->solve_smem) == cudaSuccess &&
+            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kcoop, 256, s->solve_smem) == cudaSuccess && per_sm >= 1)
             s->coop_grid = ctx->sm_count;
         cudaGetLastError();
         // cluster path: one thread-block cluster of SIM_CLUSTER_CTAS CTAs (16 needs the non-portable opt-in), if the
         // device can co-schedule it with this much shared memory per CTA
-        if (!cta && !getenv("LUDVM_NO_CLUSTER")) {
-            const void *kern = (const void *)k_sim_persist<true>;
+        if (!getenv("LUDVM_NO_CLUSTER")) {
+            const void *kern = method_kernels(p->method).persist_cluster;
             if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s->solve_smem) == cudaSuccess &&
                 cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess) {
                 cudaLaunchConfig_t cfg = {};
@@ -2214,9 +2319,7 @@ LUDVM_API int ludvm_sim_enable_pressure(ludvm_sim *s)
     int rc = dev_malloc(s->ctx, s->allocs, bytes, &p);
     if (rc) return rc;
     CUDA_TRY(cudaMemsetAsync(p, 0, bytes, s->ctx->stream));   // row 0 and rows of steps not run stay zero
-    s->d.dp = (double *)p;
-    // the one-CTA driver reads the device copy of the descriptor; the other drivers take `d` by value at launch
-    CUDA_TRY(cudaMemcpyAsync(s->d_case, &s->d, sizeof(SimDev), cudaMemcpyHostToDevice, s->ctx->stream));
+    s->d.dp = (double *)p;   // every driver takes `d` by value at launch
     CUDA_TRY(cudaStreamSynchronize(s->ctx->stream));
     return LUDVM_OK;
 }
@@ -2228,7 +2331,7 @@ LUDVM_API int ludvm_sim_enable_far_field(ludvm_sim *s, int order)
     if (s->p.mode == LUDVM_EXACT_F64)
         return set_error(LUDVM_E_UNSUPPORTED, "the far field is an approximation; exact mode keeps numpy's sums bit for bit");
     if (s->p.method == LUDVM_METHOD_RAMESH)
-        return set_error(LUDVM_E_UNSUPPORTED, "method='Ramesh' runs on the one-CTA driver, which has no far-field step");
+        return set_error(LUDVM_E_UNSUPPORTED, "the far-field step is built for method Faure; method='Ramesh' convects by all pairs");
     if (s->p.P > 256)
         return set_error(LUDVM_E_UNSUPPORTED, "P = %ld: the far-field step builds on the overlapped step, which needs P <= 256",
                          (long)s->p.P);
@@ -2262,14 +2365,6 @@ LUDVM_API int ludvm_sim_run(ludvm_sim *s, long nsteps)
     long total = s->p.nt - 1;
     long todo = std::min(nsteps, total - s->steps_enqueued);
     if (todo <= 0) return LUDVM_OK;
-    if (s->p.method == LUDVM_METHOD_RAMESH) {  // CTA path
-        CUDA_TRY(cudaMemsetAsync(s->d_next, 0, sizeof(int), s->ctx->stream));
-        k_sim_cta<RAMESH_THREADS, LUDVM_METHOD_RAMESH, true><<<1, RAMESH_THREADS, s->solve_smem, s->ctx->stream>>>(s->d_case, 1, s->d_next, (int)todo);
-        CUDA_TRY(cudaGetLastError());
-        s->ctx->launches++;
-        s->steps_enqueued += todo;
-        return LUDVM_OK;
-    }
     // smallest wakes: ONE thread-block cluster with the hardware cluster barrier between the phases
     if (s->cluster_ctas >= 4) {
         const long last_small = (SIM_CLUSTER_MAX_WAKE - 2 - (long)s->p.nfree) / 2;
@@ -2286,7 +2381,10 @@ LUDVM_API int ludvm_sim_run(ludvm_sim *s, long nsteps)
             at[0].id = cudaLaunchAttributeClusterDimension;
             at[0].val.clusterDim.x = s->cluster_ctas; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
             cfg.attrs = at; cfg.numAttrs = 1;
-            CUDA_TRY(cudaLaunchKernelEx(&cfg, k_sim_persist<true>, dc, (int)k, (unsigned long long *)nullptr));
+            unsigned long long *nobar = nullptr;
+            int ki = (int)k;
+            void *args[] = {&dc, &ki, &nobar};
+            CUDA_TRY(cudaLaunchKernelExC(&cfg, method_kernels(s->p.method).persist_cluster, args));
             s->ctx->launches++;
             s->steps_enqueued += k;
             todo -= k;
@@ -2305,7 +2403,7 @@ LUDVM_API int ludvm_sim_run(ludvm_sim *s, long nsteps)
             unsigned long long *bar = s->d_bar;
             void *args[] = {&dc, &ki, &bar};
             CUDA_TRY(cudaMemsetAsync(s->d_bar, 0, COOP_BAR_WORDS * sizeof(unsigned long long), s->ctx->stream));
-            CUDA_TRY(cudaLaunchCooperativeKernel((const void *)k_sim_persist<false>, dim3(s->coop_grid), dim3(256), args, s->solve_smem, s->ctx->stream));
+            CUDA_TRY(cudaLaunchCooperativeKernel(method_kernels(s->p.method).persist_coop, dim3(s->coop_grid), dim3(256), args, s->solve_smem, s->ctx->stream));
             s->ctx->launches++;
             s->steps_enqueued += k;
             todo -= k;
@@ -2348,8 +2446,6 @@ LUDVM_API int ludvm_sim_run(ludvm_sim *s, long nsteps)
 LUDVM_API int ludvm_sim_profile_steps(ludvm_sim *s, long nsteps, double *ms_out)
 {
     ARG_CHECK(s != nullptr && nsteps >= 0 && ms_out != nullptr);
-    if (s->p.method == LUDVM_METHOD_RAMESH)
-        return set_error(LUDVM_E_UNSUPPORTED, "method='Ramesh' runs as one persistent CTA; there are no phases to time");
     if (s->ff_order)
         return set_error(LUDVM_E_UNSUPPORTED, "the far-field step is not one of the graph path's phases; time ludvm_sim_run");
     DeviceGuard g(s->ctx->device);
@@ -2623,3 +2719,22 @@ LUDVM_API int ludvm_sweep_run_pressure(ludvm_ctx *ctx, long ncases, const ludvm_
     ARG_CHECK(dp != nullptr);
     return sweep_run(ctx, ncases, params, tables, out, out_doubles_per_case, dp, dp_doubles_per_case);
 }
+
+namespace ludvm {
+
+// Defined last: the translation unit's device code is emitted in the order its kernels are first referenced, and that
+// order feeds the device compiler's optimisation order.  With every Ramesh instantiation referenced here, after all Faure
+// kernels (k_wake_on_foil / k_solve / k_solve_small<Faure> are instantiated explicitly at their definitions), the Faure
+// kernels compile to the same SASS as before Ramesh had single-simulation drivers.
+static const MethodKernels &method_kernels(int method)
+{
+    static const MethodKernels faure{k_wake_on_foil<LUDVM_METHOD_FAURE>, k_solve<LUDVM_METHOD_FAURE>,
+                                     k_solve_small<LUDVM_METHOD_FAURE>, (const void *)k_sim_persist<false, LUDVM_METHOD_FAURE>,
+                                     (const void *)k_sim_persist<true, LUDVM_METHOD_FAURE>};
+    static const MethodKernels ramesh{k_wake_on_foil<LUDVM_METHOD_RAMESH>, k_solve<LUDVM_METHOD_RAMESH>,
+                                      k_solve_small<LUDVM_METHOD_RAMESH>, (const void *)k_sim_persist<false, LUDVM_METHOD_RAMESH>,
+                                      (const void *)k_sim_persist<true, LUDVM_METHOD_RAMESH>};
+    return method == LUDVM_METHOD_RAMESH ? ramesh : faure;
+}
+
+}  // namespace ludvm

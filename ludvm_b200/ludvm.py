@@ -100,7 +100,7 @@ class LUDVM:
             if mode == 'exact':
                 raise ValueError("far_field_order needs mode='fast': exact mode reproduces numpy's sums bit for bit")
             if method == 'Ramesh':
-                raise ValueError("far_field_order is not available for method='Ramesh' (one-CTA driver)")
+                raise ValueError("far_field_order is available for method='Faure' only (the far-field step is built on Faure's solve)")
             if Npoints > 257:
                 raise ValueError("far_field_order supports Npoints <= 257 (the overlapped step needs at most 256 panels)")
             if isinstance(far_field_order, bool) or int(far_field_order) != far_field_order or not 2 <= far_field_order <= 24:
